@@ -1,7 +1,8 @@
 #!/usr/bin/env python3
 """bench.py -- headline benchmark of the equity hot path (BASELINE.json: "showdown evals/s ...; get_equity calls/s").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W]          # the driver's line: cfg3 headline + every other config
+    python bench.py [--gpus N] [--steps K] [--warmup W]          # the default line: cfg3 headline + every other config
+    python bench.py --dump-outputs DIR ...      # also write the counters of the headline's last timed step to DIR/*.npy
     python bench.py --workload cfg1|cfg2|cfg3|cfg4|cfg5|ranges [--deal uniform|reference]    # one workload alone
     python bench.py --impl reference ...        # the reference's own C++ calculator on the host cores (oracle/_ref)
     torchrun --nproc-per-node N bench.py --gpus N ...   (one rank per GPU)
@@ -325,7 +326,7 @@ def run_exact(args, wl, cx, steps=None):
     torch.cuda.synchronize()
     assert int((w + t + l).sum().item()) == matchups
     cx.barrier()
-    steps = min(args.steps, 50) if steps is None else steps
+    steps = args.steps if steps is None else steps
     ev = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
     sampler = ClockSampler(cx.local_rank)
     sampler.start()
@@ -452,7 +453,7 @@ def run_ranges(args, wl, cx, steps=None):
     import torch
     import neuron_poker_b200 as npk
     dev = cx.dev
-    steps = min(args.steps, 20) if steps is None else steps
+    steps = args.steps if steps is None else steps
     hole_h, board_h, npl_h = make_queries(wl, cx.world, cx.rank)
     hole, board, npl = (torch.as_tensor(x).to(dev) for x in (hole_h, board_h, npl_h))
     Q, T, P = len(hole_h), wl["trials"], wl["players"]
@@ -633,6 +634,7 @@ def run_mc(args, wl, cx, deal, steps, warmup, peak=None, peak_detail=None, e2e=T
     clocks = sampler.stop()
     cx.barrier()
     dev_ms = cx.max_over_ranks(sum(s.elapsed_time(e) for s, e in zip(starts, ends)))
+    last = res.cpu().numpy()          # [2, Q] wins / ties of the last timed step, read before the e2e leg reuses the job's buffers
     check_eq = float((res[0] + res[1]).double().mean().item() / T)
     evals_per_step = Q * T * P * (1 if by_trial else world)      # whole job, all ranks
     value = evals_per_step * steps / (dev_ms * 1e-3)
@@ -705,7 +707,7 @@ def run_mc(args, wl, cx, deal, steps, warmup, peak=None, peak_detail=None, e2e=T
                                 "api": "neuron_poker_b200.equity_counts_batch(block=False) -> npk_equity_host_submit / "
                                        "npk_equity_host_wait, two batches in flight; blocking_value = one blocking "
                                        "npk_equity_host call per step"})
-    return line, (hole_h, board_h, npl_h)
+    return line, (hole_h, board_h, npl_h), last
 
 
 def run_strong(args, cx, deal="uniform", steps=10):
@@ -715,9 +717,9 @@ def run_strong(args, cx, deal="uniform", steps=10):
     import torch
     import neuron_poker_b200 as npk
     wl = workload("cfg4")
-    sharded, _ = run_mc(args, wl, cx, deal, steps, 3, e2e=False, flush=False)
+    sharded, _, _ = run_mc(args, wl, cx, deal, steps, 3, e2e=False, flush=False)
     one = Ctx(0, 1, cx.local_rank, cx.dev, cx.L)                # the same job, whole trial range, this GPU alone
-    alone, _ = run_mc(args, wl, one, deal, max(3, steps // 2), 2, e2e=False, flush=False)
+    alone, _, _ = run_mc(args, wl, one, deal, max(3, steps // 2), 2, e2e=False, flush=False)
     t1 = cx.max_over_ranks(alone["ms_per_step"])
     hole_h, board_h, npl_h = make_queries(wl, 1, 0)
     hole, board, npl = (torch.as_tensor(x).to(cx.dev) for x in (hole_h, board_h, npl_h))
@@ -791,6 +793,15 @@ def run_sustained(args, cx, deal="uniform", seconds=3.0):
                     "of queries and 131 KB of tables per CTA)"}
 
 
+def dump_outputs(directory, last):
+    """What get_equity_batch handed back in the headline's last timed step: wins [Q] and ties [Q] of every query, as
+    float64 (exact: the counts are far below 2**53).  The queries and the step's seed follow from the arguments alone."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, row in zip(("wins", "ties"), last):
+        np.save(os.path.join(directory, name + ".npy"), row.astype(np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -802,7 +813,12 @@ def main():
     ap.add_argument("--deal-ranges", dest="deal_ranges", default="reference", choices=["uniform", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="cfg3 headline only (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write wins.npy and ties.npy (float64, one entry per query of rank 0) of the headline's last timed "
+                         "step to DIR, to compare two builds output for output")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.workload not in ("all", "cfg3")):
+        ap.error("--dump-outputs writes the counters of the cfg3 headline: use it with --workload all or cfg3")
     everything = args.workload == "all"
     wl = workload("cfg3" if everything else args.workload)
     rank = int(os.environ.get("RANK", "0"))
@@ -841,11 +857,13 @@ def main():
     if args.workload == "cfg1":
         return finish({"metric": "get_equity_latency", "config": {"workload": wl["name"]}, **run_latency(args, wl, cx, with_cpu)})
     if args.workload == "cfg4":
-        line = run_strong(args, cx, args.deal, steps=min(args.steps, 50))
+        line = run_strong(args, cx, args.deal, steps=args.steps)
         return finish(line)
 
     peak, peak_detail = int_issue_peak(L)
-    line, (hole_h, board_h, npl_h) = run_mc(args, wl, cx, args.deal, args.steps, max(3, args.warmup), peak, peak_detail)
+    line, (hole_h, board_h, npl_h), last = run_mc(args, wl, cx, args.deal, args.steps, max(3, args.warmup), peak, peak_detail)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
     try:
         with open(os.path.join(ROOT, "profiles", "ncu_traffic.json")) as f:
             t_rec = json.load(f).get(line["roofline"]["kernel"])
@@ -875,7 +893,7 @@ def main():
         return {k: rec[k] for k in keep if k in rec}
 
     extras["cfg2"] = brief(run_exact(args, workload("cfg2"), cx, steps=10))
-    ref3, _ = run_mc(args, workload("cfg3"), cx, "reference", 20, 3, peak, peak_detail, e2e=False)
+    ref3, _, _ = run_mc(args, workload("cfg3"), cx, "reference", 20, 3, peak, peak_detail, e2e=False)
     extras["cfg3_reference_dealer"] = brief(ref3)
     extras["cfg4"] = brief(run_strong(args, cx, "uniform", steps=20))
     extras["cfg4_reference_dealer"] = brief(run_strong(args, cx, "reference", steps=10))
