@@ -3,7 +3,6 @@
 
 #include <cstdio>
 #include <cstring>
-#include <cstdlib>
 #include <atomic>
 #include <mutex>
 #include <string>
@@ -36,8 +35,6 @@ bool g_tables_ready = false;
 constexpr int kMaxDevices = 64;
 DeviceState g_dev[kMaxDevices];
 
-// host-staging state of npk_equity_host: one per CALLING THREAD (its own stream, pinned buffers and one-query scratch), so
-// the host entry point is re-entrant -- two host threads never share a stream, a counter or a result block
 // One resident server per device and process: a second one could not get the SMs the first one holds and its requests would
 // starve.  Owner = address of the owning thread's staging block, 0 = none.
 std::atomic<uintptr_t> g_resident_owner[kMaxDevices];
@@ -87,6 +84,7 @@ struct HostStage {
     unsigned int oneshot_parity = 0;              // accumulator the next launched one-query call uses
     bool res_dirty = false;                       // a server has used the state block since the last launched call
     void stop_resident();
+    void release_resident_slot();
     void release()
     {
         if (device < 0) return;
@@ -94,10 +92,7 @@ struct HostStage {
         if (cudaGetDevice(&cur) != cudaSuccess) { device = -1; return; }     // runtime already torn down
         cudaSetDevice(device);
         stop_resident();
-        if (res_enabled && device < kMaxDevices) {
-            uintptr_t mine = reinterpret_cast<uintptr_t>(this);
-            g_resident_owner[device].compare_exchange_strong(mine, 0);
-        }
+        release_resident_slot();
         cudaFree(res_state); cudaFreeHost(res_mb);
         for (HostSlot& s : slot) {
             if (s.stream) cudaStreamSynchronize(s.stream);
@@ -130,33 +125,13 @@ void HostStage::stop_resident()
     res_running = false;
 }
 
-// give the device's resident slot back (the thread stops serving its calls through a server)
-static void release_resident_slot(HostStage& st)
+// give the device's resident slot back if this thread holds it (the thread stops serving its calls through a server)
+void HostStage::release_resident_slot()
 {
-    if (st.device >= 0 && st.device < kMaxDevices) {
-        uintptr_t mine = reinterpret_cast<uintptr_t>(&st);
-        g_resident_owner[st.device].compare_exchange_strong(mine, 0);
+    if (device >= 0 && device < kMaxDevices) {
+        uintptr_t mine = reinterpret_cast<uintptr_t>(this);
+        g_resident_owner[device].compare_exchange_strong(mine, 0);
     }
-}
-
-// Tuning aids, read from the environment ONCE (a getenv per launch costs as much as the launch of a 30 us call).
-struct Tuning {
-    long long chunk = 0;        // NPK_CHUNK: trials per work item
-    int warps = 0;              // NPK_WARPS: warps per CTA of the Monte-Carlo kernels
-    bool no_single_path = false;// NPK_NO_SINGLE_PATH: one-query host calls through the general path
-    bool no_oneshot = false;    // NPK_NO_ONESHOT: launched one-query calls through the shape's own kernel (per-warp hand-over)
-    Tuning()
-    {
-        if (const char* e = getenv("NPK_CHUNK")) chunk = atoll(e);
-        if (const char* e = getenv("NPK_WARPS")) warps = atoi(e);
-        no_single_path = getenv("NPK_NO_SINGLE_PATH") != nullptr;
-        no_oneshot = getenv("NPK_NO_ONESHOT") != nullptr;
-    }
-};
-const Tuning& tuning()
-{
-    static const Tuning t;
-    return t;
 }
 
 int fail(int code, const std::string& msg)
@@ -205,23 +180,8 @@ __device__ __forceinline__ int classify_query(const uint8_t* hole, const uint8_t
                                               long long q)
 {
     const int np = n_players[q];
-    unsigned long long mask = 0;
-    int known = 0, bad = 0;
-    bool ended = false;
-    for (int i = 0; i < 2; i++) {
-        const int c = hole[2 * q + i];
-        if (c >= 52) bad = 1; else { bad |= (int)(mask >> c & 1ull); mask |= 1ull << c; }
-    }
-    for (int i = 0; i < 5; i++) {
-        const int c = board[5 * q + i];
-        if (c == 0xFF) { ended = true; continue; }
-        if (ended || c >= 52) { bad = 1; continue; }
-        bad |= (int)(mask >> c & 1ull);
-        mask |= 1ull << c;
-        known++;
-    }
-    if (np < 1 || np > 10) bad = 1;
-    return bad ? -1 : (np - 1) * 6 + known;
+    const int known = npk::validate_query(hole + 2 * q, board + 5 * q, np);
+    return known < 0 ? -1 : (np - 1) * 6 + known;
 }
 
 // Count the queries of every shape -- per block in shared memory, then one global atomic per shape and block (65,536
@@ -312,7 +272,6 @@ long long plan_items(npk::EquityParams& p, long long queries, long long trials, 
 {
     const long long warps = (long long)sm_count * 16;
     long long c = (queries * trials) / (8 * warps);
-    if (tuning().chunk > 0) c = tuning().chunk;
     c = (c + lanes_worth - 1) / lanes_worth * lanes_worth;      // a warp iteration covers 64 trials (a pair per lane)
     if (c < lanes_worth) c = lanes_worth;
     if (c > 2048) c = 2048;
@@ -329,6 +288,53 @@ int grid_for(const DeviceState& ds, long long items, int warps_per_cta)
     if (ctas < 1) ctas = 1;
     if (ctas > ds.sm_count) ctas = ds.sm_count;
     return (int)ctas;
+}
+
+int check_deal_mode(int deal_mode)
+{
+    if (deal_mode == NPK_DEAL_UNIFORM || deal_mode == NPK_DEAL_REFERENCE) return NPK_OK;
+    return fail(NPK_ERR_INVALID_ARGUMENT, "deal_mode must be NPK_DEAL_UNIFORM or NPK_DEAL_REFERENCE");
+}
+
+// First checks of the batched Monte-Carlo entry points: the current device and the sizes.  Returns NPK_OK, an error code,
+// or kEmptyBatch when there is nothing to compute (Q or trials is 0; the pointers are not looked at then).
+constexpr int kEmptyBatch = 1;
+int batch_start(DeviceState** ds, int64_t Q, int64_t trials, int64_t trial_offset)
+{
+    int rc = current_state(ds);
+    if (rc) return rc;
+    if (Q < 0 || trials < 0 || trial_offset < 0) return fail(NPK_ERR_INVALID_ARGUMENT, "negative size");
+    if (Q == 0 || trials == 0) return kEmptyBatch;
+    if (Q > 0x7fffffffLL) return fail(NPK_ERR_INVALID_ARGUMENT, "at most 2^31-1 queries per call");
+    return NPK_OK;
+}
+
+// Zero the workspace header (work counters, shape counts, invalid / abort words) before a batch's kernels.
+int clear_workspace(uint8_t* ws, cudaStream_t s)
+{
+    const cudaError_t e = cudaMemsetAsync(ws, 0, kWsIndex, s);
+    return e == cudaSuccess ? NPK_OK : cuda_fail(e, "cudaMemsetAsync(workspace)");
+}
+
+// The fields of a Monte-Carlo launch that every entry point fills alike, and the plan of its work items: returns the items
+// per query.  Only the reference's dealer and the range kernels count `passes`; the uniform dealer never reads it.
+long long fill_params(npk::EquityParams& p, const DeviceState& ds, const uint8_t* hole, const uint8_t* board,
+                      const uint8_t* n_players, int64_t Q, int64_t trials, int64_t trial_offset, int64_t query_offset,
+                      uint64_t seed, int deal_mode, uint64_t* wins, uint64_t* ties, uint64_t* win_types, uint64_t* passes,
+                      uint32_t* abort_flag, int lanes_worth = 64)
+{
+    p = npk::EquityParams{};
+    p.tables = ds.t;
+    p.hole = hole; p.board = board; p.n_players = n_players;
+    p.nq = Q; p.trials = trials; p.trial_offset = trial_offset; p.query_offset = (uint32_t)query_offset;
+    p.seed_lo = (uint32_t)seed; p.seed_hi = (uint32_t)(seed >> 32);
+    p.reference_dealer = deal_mode == NPK_DEAL_REFERENCE ? 1u : 0u;
+    p.wins = reinterpret_cast<unsigned long long*>(wins);
+    p.ties = reinterpret_cast<unsigned long long*>(ties);
+    p.win_types = reinterpret_cast<unsigned long long*>(win_types);
+    p.passes = reinterpret_cast<unsigned long long*>(passes);
+    p.abort_flag = abort_flag;
+    return plan_items(p, Q, trials, ds.sm_count, lanes_worth);
 }
 
 }  // namespace
@@ -492,40 +498,28 @@ int npk_equity_batch(const uint8_t* hole, const uint8_t* board, const uint8_t* n
                      void* workspace, void* stream)
 {
     DeviceState* ds;
-    int rc = current_state(&ds);
-    if (rc) return rc;
-    if (Q < 0 || trials < 0 || trial_offset < 0) return fail(NPK_ERR_INVALID_ARGUMENT, "negative size");
-    if (Q == 0 || trials == 0) return NPK_OK;
-    if (Q > 0x7fffffffLL) return fail(NPK_ERR_INVALID_ARGUMENT, "at most 2^31-1 queries per call");
+    int rc = batch_start(&ds, Q, trials, trial_offset);
+    if (rc) return rc == kEmptyBatch ? NPK_OK : rc;
     if (!hole || !board || !n_players || !wins_strict || !ties || !workspace)
         return fail(NPK_ERR_INVALID_ARGUMENT, "null pointer");
-    if (deal_mode != NPK_DEAL_UNIFORM && deal_mode != NPK_DEAL_REFERENCE)
-        return fail(NPK_ERR_INVALID_ARGUMENT, "deal_mode must be NPK_DEAL_UNIFORM or NPK_DEAL_REFERENCE");
+    if ((rc = check_deal_mode(deal_mode))) return rc;
     const bool uniform_shape = uniform_players >= 0 && uniform_known >= 0;
     if (uniform_shape && (uniform_players < 1 || uniform_players > 10 || uniform_known > 5))
         return fail(NPK_ERR_INVALID_CARDS, "players must be 1..10 and known board cards 0..5");
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     uint8_t* ws = static_cast<uint8_t*>(workspace);
-    cudaError_t e = cudaMemsetAsync(ws, 0, kWsIndex, s);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(workspace)");
+    if ((rc = clear_workspace(ws, s))) return rc;
 
-    npk::EquityParams p{};
-    p.tables = ds->t;
-    p.hole = hole; p.board = board; p.n_players = n_players;
-    p.trials = trials; p.trial_offset = trial_offset; p.query_offset = (uint32_t)query_offset;
-    p.seed_lo = (uint32_t)seed; p.seed_hi = (uint32_t)(seed >> 32);
-    const long long chunks = plan_items(p, Q, trials, ds->sm_count);
-    p.wins = reinterpret_cast<unsigned long long*>(wins_strict);
-    p.ties = reinterpret_cast<unsigned long long*>(ties);
-    p.win_types = reinterpret_cast<unsigned long long*>(win_types);
-    p.passes = deal_mode == NPK_DEAL_REFERENCE ? reinterpret_cast<unsigned long long*>(passes) : nullptr;
-    p.reference_dealer = deal_mode == NPK_DEAL_REFERENCE ? 1u : 0u;
-    p.abort_flag = reinterpret_cast<uint32_t*>(ws + kWsAbort);      // + 15 diagnostic words, all inside the header
+    npk::EquityParams p;
+    const long long chunks = fill_params(p, *ds, hole, board, n_players, Q, trials, trial_offset, query_offset, seed, deal_mode,
+                                         wins_strict, ties, win_types, passes,
+                                         reinterpret_cast<uint32_t*>(ws + kWsAbort));   // + 15 diagnostic words, all inside the header
     const bool validate = (flags & NPK_FLAG_VALIDATE) != 0;
+    cudaError_t e;
 
     if (uniform_shape && !validate) {
-        p.qindex = nullptr; p.nq = Q; p.work_counter = reinterpret_cast<unsigned long long*>(ws + kWsCounters);
-        e = npk::launch_equity_uniform(uniform_players - 1, 5 - uniform_known, p, Q * chunks, ds->sm_count, tuning().warps, s);
+        p.work_counter = reinterpret_cast<unsigned long long*>(ws + kWsCounters);
+        e = npk::launch_equity_uniform(uniform_players - 1, 5 - uniform_known, p, Q * chunks, ds->sm_count, s);
         return e == cudaSuccess ? NPK_OK : cuda_fail(e, "equity_uniform_kernel launch");
     }
     if (uniform_shape) {
@@ -541,8 +535,8 @@ int npk_equity_batch(const uint8_t* hole, const uint8_t* board, const uint8_t* n
                                    " (card id >= 52, duplicate cards, gap in the board, or players outside 1..10)");
         if (host[(uniform_players - 1) * 6 + uniform_known] != (uint32_t)Q)
             return fail(NPK_ERR_INVALID_ARGUMENT, "queries do not all have the declared uniform shape");
-        p.qindex = nullptr; p.nq = Q; p.work_counter = reinterpret_cast<unsigned long long*>(ws + kWsCounters) + 1;
-        e = npk::launch_equity_uniform(uniform_players - 1, 5 - uniform_known, p, Q * chunks, ds->sm_count, tuning().warps, s);
+        p.work_counter = reinterpret_cast<unsigned long long*>(ws + kWsCounters) + 1;
+        e = npk::launch_equity_uniform(uniform_players - 1, 5 - uniform_known, p, Q * chunks, ds->sm_count, s);
         return e == cudaSuccess ? NPK_OK : cuda_fail(e, "equity_uniform_kernel launch");
     }
     rc = enqueue_mixed(ds, p, hole, board, n_players, Q, ~0ull, ws, s);
@@ -563,33 +557,19 @@ int npk_equity_batch_async(const uint8_t* hole, const uint8_t* board, const uint
                            void* stream)
 {
     DeviceState* ds;
-    int rc = current_state(&ds);
-    if (rc) return rc;
-    if (Q < 0 || trials < 0 || trial_offset < 0) return fail(NPK_ERR_INVALID_ARGUMENT, "negative size");
-    if (Q == 0 || trials == 0) return NPK_OK;
-    if (Q > 0x7fffffffLL) return fail(NPK_ERR_INVALID_ARGUMENT, "at most 2^31-1 queries per call");
+    int rc = batch_start(&ds, Q, trials, trial_offset);
+    if (rc) return rc == kEmptyBatch ? NPK_OK : rc;
     if (!hole || !board || !n_players || !wins_strict || !ties || !workspace)
         return fail(NPK_ERR_INVALID_ARGUMENT, "null pointer");
-    if (deal_mode != NPK_DEAL_UNIFORM && deal_mode != NPK_DEAL_REFERENCE)
-        return fail(NPK_ERR_INVALID_ARGUMENT, "deal_mode must be NPK_DEAL_UNIFORM or NPK_DEAL_REFERENCE");
+    if ((rc = check_deal_mode(deal_mode))) return rc;
     shape_mask &= (1ull << kGroups) - 1ull;
     if (!shape_mask) return fail(NPK_ERR_INVALID_ARGUMENT, "empty shape mask");
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     uint8_t* ws = static_cast<uint8_t*>(workspace);
-    cudaError_t e = cudaMemsetAsync(ws, 0, kWsIndex, s);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(workspace)");
-    npk::EquityParams p{};
-    p.tables = ds->t;
-    p.hole = hole; p.board = board; p.n_players = n_players;
-    p.trials = trials; p.trial_offset = trial_offset; p.query_offset = (uint32_t)query_offset;
-    p.seed_lo = (uint32_t)seed; p.seed_hi = (uint32_t)(seed >> 32);
-    plan_items(p, Q, trials, ds->sm_count);
-    p.wins = reinterpret_cast<unsigned long long*>(wins_strict);
-    p.ties = reinterpret_cast<unsigned long long*>(ties);
-    p.win_types = reinterpret_cast<unsigned long long*>(win_types);
-    p.passes = deal_mode == NPK_DEAL_REFERENCE ? reinterpret_cast<unsigned long long*>(passes) : nullptr;
-    p.reference_dealer = deal_mode == NPK_DEAL_REFERENCE ? 1u : 0u;
-    p.abort_flag = reinterpret_cast<uint32_t*>(ws + kWsAbort);
+    if ((rc = clear_workspace(ws, s))) return rc;
+    npk::EquityParams p;
+    fill_params(p, *ds, hole, board, n_players, Q, trials, trial_offset, query_offset, seed, deal_mode, wins_strict, ties,
+                win_types, passes, reinterpret_cast<uint32_t*>(ws + kWsAbort));
     return enqueue_mixed(ds, p, hole, board, n_players, Q, shape_mask, ws, s);
 }
 
@@ -612,24 +592,32 @@ int npk_equity_batch_status(const void* workspace, void* stream, uint32_t* inval
 }
 
 namespace {
-// validation of one host query (what npk_equity_host does per query); returns the number of known board cards or -1
-int validate_one(const uint8_t* hole, const uint8_t* board, int players)
+// The query of a one-query call as the one-query kernels read it (ResidentMailbox::ReqA, serve_request in npk_mixed.cu):
+// x = hole[0] | hole[1] << 8 | board[0] << 16 | board[1] << 24, y = board[2..4] | players << 24 | reference dealer << 31.
+uint2 pack_query(const uint8_t* hole, const uint8_t* board, int players, int deal_mode)
 {
-    unsigned long long mask = 0;
-    int known = 0;
-    bool ended = false, bad = players < 1 || players > 10;
-    for (int i = 0; i < 2 && !bad; i++) {
-        const int c = hole[i];
-        if (c >= 52 || (mask >> c & 1ull)) bad = true; else mask |= 1ull << c;
+    return make_uint2((unsigned int)hole[0] | (unsigned int)hole[1] << 8 | (unsigned int)board[0] << 16 |
+                          (unsigned int)board[1] << 24,
+                      (unsigned int)board[2] | (unsigned int)board[3] << 8 | (unsigned int)board[4] << 16 |
+                          (unsigned int)players << 24 | (deal_mode == NPK_DEAL_REFERENCE ? 1u << 31 : 0u));
+}
+
+// Wait for a launched one-query kernel: spin on the sequence word it writes to mapped host memory last, and after a few
+// hundred ms ask the driver.
+int await_result(const volatile unsigned long long* seq_word, unsigned long long seq, cudaStream_t s)
+{
+    for (long spins = 0; spins < 4000000 && *seq_word != seq; spins++) {
+#if defined(__x86_64__) || defined(__i386__)
+        __builtin_ia32_pause();
+#endif
     }
-    for (int i = 0; i < 5 && !bad; i++) {
-        const int c = board[i];
-        if (c == 0xFF) { ended = true; continue; }
-        if (ended || c >= 52 || (mask >> c & 1ull)) { bad = true; break; }
-        mask |= 1ull << c;
-        known++;
+    if (*seq_word != seq) {
+        const cudaError_t e = cudaStreamSynchronize(s);
+        if (e != cudaSuccess) return cuda_fail(e, "equity kernel");
+        if (*seq_word != seq) return fail(NPK_ERR_CUDA, "the one-query kernel finished without publishing its result");
     }
-    return bad ? -1 : known;
+    std::atomic_thread_fence(std::memory_order_acquire);
+    return NPK_OK;
 }
 
 // (Re)start this thread's resident server on its stream.  `completed` = sequence number of the last request whose result has
@@ -664,26 +652,18 @@ int resident_launch(DeviceState* ds, HostStage& st)
 
 // One query through the resident server: post the request in the mailbox, spin on the result.  No CUDA call on this path
 // unless the server has left in the meantime (idle limit) and is started again.
-int resident_query(DeviceState* ds, HostStage& st, const uint8_t* hole, const uint8_t* board, int players, int64_t trials,
-                   uint64_t seed, int deal_mode, uint64_t* wins_strict, uint64_t* ties)
+int resident_query(DeviceState* ds, HostStage& st, uint2 query, int64_t trials, uint64_t seed, uint64_t* wins_strict,
+                   uint64_t* ties)
 {
-    if (validate_one(hole, board, players) < 0)
-        return fail(NPK_ERR_INVALID_CARDS, "query 0: card id >= 52, duplicate cards, gap in the board, or players outside 1..10");
-    wins_strict[0] = 0; ties[0] = 0;
-    if (trials == 0) return NPK_OK;
     if (!st.res_mb) { int rc = resident_launch(ds, st); if (rc) return rc; }
     volatile npk::ResidentMailbox* mb = st.res_mb;
     unsigned int seq = ++st.res_seq;
     if (seq == 0) seq = ++st.res_seq;
-    const unsigned int packed_lo = (unsigned int)hole[0] | (unsigned int)hole[1] << 8 | (unsigned int)board[0] << 16 |
-                                   (unsigned int)board[1] << 24;
-    const unsigned int packed_hi = (unsigned int)board[2] | (unsigned int)board[3] << 8 | (unsigned int)board[4] << 16 |
-                                   (unsigned int)players << 24 | (deal_mode == NPK_DEAL_REFERENCE ? 1u << 31 : 0u);
     // the halves that carry the sequence number go last (x86 keeps the order of stores): a record the device reads is
     // either complete or still shows the old number
     volatile unsigned long long* ra = reinterpret_cast<volatile unsigned long long*>(&st.res_mb->a);
     volatile unsigned long long* rb = reinterpret_cast<volatile unsigned long long*>(&st.res_mb->b);
-    ra[1] = (unsigned long long)packed_lo | (unsigned long long)packed_hi << 32;
+    ra[1] = (unsigned long long)query.x | (unsigned long long)query.y << 32;
     rb[1] = (unsigned long long)(uint32_t)(seed >> 32);                                   // seed_hi, stop = 0
     std::atomic_thread_fence(std::memory_order_release);
     rb[0] = (unsigned long long)seq | (unsigned long long)(uint32_t)seed << 32;
@@ -722,26 +702,28 @@ int resident_query(DeviceState* ds, HostStage& st, const uint8_t* hole, const ui
 //   * resident mode on: post the query in the mailbox of this thread's persistent server (resident_query above);
 //   * wins and ties only (what get_equity needs): ONE launch of equity_oneshot_kernel, query in the kernel parameters, one packed
 //     atomic per CTA, one 16-byte store (csrc/npk_mixed.cu);
-//   * win types / passes wanted (or NPK_NO_ONESHOT): one launch of the shape's own kernel; the counters stay in device memory
-//     between calls, the last warp of the grid hands them over and zeroes them (finish_single_call, csrc/npk_mc.cuh).
+//   * win types / passes wanted, or 2^28 trials and more: one launch of the shape's own kernel; the counters stay in device
+//     memory between calls, the last warp of the grid hands them over and zeroes them (finish_single_call, csrc/npk_mc.cuh).
 int single_query(DeviceState* ds, HostStage& st, const uint8_t* hole, const uint8_t* board, int players, int64_t trials,
                  uint64_t seed, int deal_mode, uint64_t* wins_strict, uint64_t* ties, uint64_t* win_types, uint64_t* passes)
 {
     cudaError_t e;
-    if (deal_mode != NPK_DEAL_UNIFORM && deal_mode != NPK_DEAL_REFERENCE)
-        return fail(NPK_ERR_INVALID_ARGUMENT, "deal_mode must be NPK_DEAL_UNIFORM or NPK_DEAL_REFERENCE");
+    int rc = check_deal_mode(deal_mode);
+    if (rc) return rc;
     if (trials < 0) return fail(NPK_ERR_INVALID_ARGUMENT, "negative size");
-    if (st.res_enabled && !win_types && !passes && trials < npk::kResidentMaxTrials)
-        return resident_query(ds, st, hole, board, players, trials, seed, deal_mode, wins_strict, ties);
-    st.stop_resident();                            // this path launches on the stream the server would be holding
-    const int known = validate_one(hole, board, players);
+    const int known = npk::validate_query(hole, board, players);
     if (known < 0) return fail(NPK_ERR_INVALID_CARDS, "query 0: card id >= 52, duplicate cards, gap in the board, or players outside 1..10");
-    if (!win_types && !passes && trials < npk::kResidentMaxTrials && !tuning().no_oneshot) {
+    wins_strict[0] = 0; ties[0] = 0;
+    if (win_types) std::memset(win_types, 0, 72);
+    if (passes) passes[0] = 0;
+    if (trials == 0) return NPK_OK;
+    const uint2 query = pack_query(hole, board, players, deal_mode);
+    const bool counts_only = !win_types && !passes && trials < npk::kResidentMaxTrials;   // the packed hand-over's limit
+    if (st.res_enabled && counts_only) return resident_query(ds, st, query, trials, seed, wins_strict, ties);
+    st.stop_resident();                            // the launches below use the stream the server would be holding
+    if (counts_only) {
         // the common call: a kernel launched for this request, handing over like the resident server (npk_mixed.cu)
-        wins_strict[0] = 0; ties[0] = 0;
-        if (trials == 0) return NPK_OK;
-        int rc = resident_buffers(st);
-        if (rc) return rc;
+        if ((rc = resident_buffers(st))) return rc;
         if (st.res_dirty) {
             if ((e = cudaMemsetAsync(st.res_state, 0, sizeof(npk::ResidentState), st.stream)) != cudaSuccess) return cuda_fail(e, "memset");
             st.oneshot_parity = 0;
@@ -749,28 +731,13 @@ int single_query(DeviceState* ds, HostStage& st, const uint8_t* hole, const uint
         }
         unsigned int seq = ++st.res_seq;
         if (seq == 0) seq = ++st.res_seq;
-        const uint4 a = make_uint4(0u, (unsigned int)trials,
-                                   (unsigned int)hole[0] | (unsigned int)hole[1] << 8 | (unsigned int)board[0] << 16 |
-                                       (unsigned int)board[1] << 24,
-                                   (unsigned int)board[2] | (unsigned int)board[3] << 8 | (unsigned int)board[4] << 16 |
-                                       (unsigned int)players << 24 | (deal_mode == NPK_DEAL_REFERENCE ? 1u << 31 : 0u));
-        const uint4 b = make_uint4(0u, (unsigned int)seed, (unsigned int)(seed >> 32), seq);
-        e = npk::launch_equity_oneshot(ds->t, st.res_state, st.res_mb_dev, a, b, st.oneshot_parity, ds->sm_count, st.stream);
+        e = npk::launch_equity_oneshot(ds->t, st.res_state, st.res_mb_dev, make_uint4(0u, (unsigned int)trials, query.x, query.y),
+                                       make_uint4(0u, (unsigned int)seed, (unsigned int)(seed >> 32), seq), st.oneshot_parity,
+                                       ds->sm_count, st.stream);
         if (e != cudaSuccess) return cuda_fail(e, "equity kernel launch");
         st.oneshot_parity ^= 1u;
         volatile npk::ResidentMailbox* mb = st.res_mb;
-        bool arrived = false;
-        for (long spins = 0; spins < 4000000; spins++) {          // a few hundred ms at most, then ask the driver
-            if ((unsigned int)mb->done.seq == seq) { arrived = true; break; }
-#if defined(__x86_64__) || defined(__i386__)
-            __builtin_ia32_pause();
-#endif
-        }
-        if (!arrived) {
-            if ((e = cudaStreamSynchronize(st.stream)) != cudaSuccess) return cuda_fail(e, "equity kernel");
-            if ((unsigned int)mb->done.seq != seq) return fail(NPK_ERR_CUDA, "the one-query kernel finished without publishing its result");
-        }
-        std::atomic_thread_fence(std::memory_order_acquire);
+        if ((rc = await_result(&mb->done.seq, seq, st.stream))) return rc;
         wins_strict[0] = mb->done.wins; ties[0] = mb->done.ties;
         return NPK_OK;
     }
@@ -785,45 +752,21 @@ int single_query(DeviceState* ds, HostStage& st, const uint8_t* hole, const uint
         if ((e = cudaMemcpy(st.single, &init, sizeof init, cudaMemcpyHostToDevice)) != cudaSuccess) return cuda_fail(e, "cudaMemcpy");
         st.single_seq = 0;
     }
-    wins_strict[0] = 0; ties[0] = 0;
-    if (win_types) std::memset(win_types, 0, 72);
-    if (passes) passes[0] = 0;
-    if (trials == 0) return NPK_OK;
-    npk::EquityParams p{};
-    p.tables = ds->t;
-    p.hole = nullptr; p.board = nullptr; p.n_players = nullptr; p.qindex = nullptr;
-    p.inline_query = (uint64_t)hole[0] | (uint64_t)hole[1] << 8;
-    for (int i = 0; i < 5; i++) p.inline_query |= (uint64_t)board[i] << (16 + 8 * i);
-    p.nq = 1; p.trials = trials; p.trial_offset = 0; p.query_offset = 0;
-    p.seed_lo = (uint32_t)seed; p.seed_hi = (uint32_t)(seed >> 32);
-    const long long chunks = plan_items(p, 1, trials, ds->sm_count);
-    p.reference_dealer = deal_mode == NPK_DEAL_REFERENCE ? 1u : 0u;
+    npk::EquityParams p;
+    const long long chunks = fill_params(p, *ds, nullptr, nullptr, nullptr, 1, trials, 0, 0, seed, deal_mode,
+                                         reinterpret_cast<uint64_t*>(&st.single->wins),
+                                         reinterpret_cast<uint64_t*>(&st.single->ties),
+                                         win_types ? reinterpret_cast<uint64_t*>(st.single->win_types) : nullptr,
+                                         passes ? reinterpret_cast<uint64_t*>(&st.single->passes) : nullptr,
+                                         st.single->abort_flag);
+    p.inline_query = (uint64_t)query.x | (uint64_t)(query.y & 0xFFFFFFu) << 32;
     p.single = st.single;
     p.single_seq = ++st.single_seq;
-    const bool quick = !win_types && !passes && trials < (1ll << 32);
-    p.single_quick = quick ? 1u : 0u;
     p.work_counter = &st.single->work_counter;
-    p.wins = &st.single->wins; p.ties = &st.single->ties;
-    p.win_types = win_types ? st.single->win_types : nullptr;
-    p.passes = (passes && deal_mode == NPK_DEAL_REFERENCE) ? &st.single->passes : nullptr;
-    p.abort_flag = st.single->abort_flag;
-    e = npk::launch_equity_uniform(players - 1, 5 - known, p, chunks, ds->sm_count, tuning().warps, st.stream);
+    e = npk::launch_equity_uniform(players - 1, 5 - known, p, chunks, ds->sm_count, st.stream);
     if (e != cudaSuccess) return cuda_fail(e, "equity kernel launch");
     const volatile npk::SingleResult* r = st.single_host;
-    const volatile unsigned long long* flag = quick ? &r->quick.seq : &r->seq;
-    bool arrived = false;
-    for (long spins = 0; spins < 4000000; spins++) {              // a few hundred ms at most, then ask the driver
-        if (*flag == p.single_seq) { arrived = true; break; }
-#if defined(__x86_64__) || defined(__i386__)
-        __builtin_ia32_pause();
-#endif
-    }
-    if (!arrived) {
-        if ((e = cudaStreamSynchronize(st.stream)) != cudaSuccess) return cuda_fail(e, "equity kernel");
-        if (*flag != p.single_seq) return fail(NPK_ERR_CUDA, "the one-query kernel finished without publishing its result");
-    }
-    std::atomic_thread_fence(std::memory_order_acquire);
-    if (quick) { wins_strict[0] = r->quick.wins; ties[0] = r->quick.ties; return NPK_OK; }
+    if ((rc = await_result(&r->seq, p.single_seq, st.stream))) return rc;
     wins_strict[0] = r->wins; ties[0] = r->ties;
     if (win_types) for (int i = 0; i < 9; i++) win_types[i] = r->win_types[i];
     if (passes) passes[0] = r->passes;
@@ -867,7 +810,7 @@ int host_submit(DeviceState* ds, HostStage& st, const uint8_t* hole, const uint8
     for (int i = 0; i < 5; i++) uk += board[i] != 0xFF;
     bool uniform = true;
     for (int64_t q = 0; q < Q; q++) {
-        const int known = validate_one(hole + 2 * q, board + 5 * q, n_players[q]);
+        const int known = npk::validate_query(hole + 2 * q, board + 5 * q, n_players[q]);
         if (known < 0) return fail(NPK_ERR_INVALID_CARDS, "query " + std::to_string(q) +
                                    ": card id >= 52, duplicate cards, gap in the board, or players outside 1..10");
         if (n_players[q] != up || known != uk) uniform = false;
@@ -941,7 +884,7 @@ int npk_equity_host(const uint8_t* hole, const uint8_t* board, const uint8_t* n_
     if (!hole || !board || !n_players || !wins_strict || !ties) return fail(NPK_ERR_INVALID_ARGUMENT, "null pointer");
     HostStage* st;
     if ((rc = thread_stage(&st))) return rc;
-    if (Q == 1 && !tuning().no_single_path)
+    if (Q == 1)
         return single_query(ds, *st, hole, board, n_players[0], trials, seed, deal_mode, wins_strict, ties, win_types, passes);
     int64_t ticket = -1;
     rc = host_submit(ds, *st, hole, board, n_players, Q, trials, seed, deal_mode, (win_types ? 1u : 0u) | (passes ? 2u : 0u),
@@ -988,12 +931,7 @@ int npk_equity_one(uint64_t packed, int players, int64_t trials, uint64_t seed, 
     for (int i = 0; i < 7; i++) q[i] = (uint8_t)(packed >> (8 * i));
     HostStage* stp;
     if ((rc = thread_stage(&stp))) return rc;
-    HostStage& st = *stp;
-    const uint8_t np = (uint8_t)(players < 0 || players > 255 ? 255 : players);
-    if (tuning().no_single_path)
-        return npk_equity_host(q, q + 2, &np, 1, trials, seed, deal_mode, out, out + 1, (want & 1u) ? out + 2 : nullptr,
-                               (want & 2u) ? out + 11 : nullptr);
-    return single_query(ds, st, q, q + 2, players, trials, seed, deal_mode, out, out + 1, (want & 1u) ? out + 2 : nullptr,
+    return single_query(ds, *stp, q, q + 2, players, trials, seed, deal_mode, out, out + 1, (want & 1u) ? out + 2 : nullptr,
                         (want & 2u) ? out + 11 : nullptr);
 }
 
@@ -1031,7 +969,7 @@ int npk_resident_stop(void)
     if ((rc = thread_stage(&st))) return rc;
     st->res_enabled = false;
     st->stop_resident();
-    release_resident_slot(*st);
+    st->release_resident_slot();
     return NPK_OK;
 }
 
@@ -1148,27 +1086,21 @@ int npk_equity_batch_sharded(void* group, const uint8_t* hole, const uint8_t* bo
     if (Q <= 0 || 2 * Q > g->stride) return fail(NPK_ERR_INVALID_ARGUMENT, "Q must be 1..max_words/2 of the peer group");
     if (trials_total < 0) return fail(NPK_ERR_INVALID_ARGUMENT, "negative size");
     if (players < 1 || players > 10 || known < 0 || known > 5) return fail(NPK_ERR_INVALID_CARDS, "players must be 1..10 and known board cards 0..5");
-    if (deal_mode != NPK_DEAL_UNIFORM && deal_mode != NPK_DEAL_REFERENCE)
-        return fail(NPK_ERR_INVALID_ARGUMENT, "deal_mode must be NPK_DEAL_UNIFORM or NPK_DEAL_REFERENCE");
+    if ((rc = check_deal_mode(deal_mode))) return rc;
     // this rank's trial range: the same split as neuron_poker_b200.dist.trial_shard
     const int64_t base = trials_total / g->world, extra = trials_total % g->world;
     const int64_t begin = g->rank * base + std::min<int64_t>(g->rank, extra);
     const int64_t count = base + (g->rank < extra ? 1 : 0);
-    npk::EquityParams p{};
-    p.tables = ds->t;
-    p.hole = hole; p.board = board; p.n_players = n_players;
-    p.nq = Q; p.trials = count; p.trial_offset = begin; p.query_offset = (uint32_t)query_offset;
-    p.seed_lo = (uint32_t)seed; p.seed_hi = (uint32_t)(seed >> 32);
-    const long long chunks = plan_items(p, Q, count, ds->sm_count);
-    p.reference_dealer = deal_mode == NPK_DEAL_REFERENCE ? 1u : 0u;
-    p.wins = g->acc; p.ties = g->acc + Q;
-    p.abort_flag = g->abort_flag;
+    npk::EquityParams p;
+    const long long chunks = fill_params(p, *ds, hole, board, n_players, Q, count, begin, query_offset, seed, deal_mode,
+                                         reinterpret_cast<uint64_t*>(g->acc), reinterpret_cast<uint64_t*>(g->acc + Q), nullptr,
+                                         nullptr, g->abort_flag);
     p.peer = g->call; p.peer_epoch = ++g->epoch; p.peer_totals = reinterpret_cast<unsigned long long*>(totals);
     p.peer_words = (uint32_t)(2 * Q);
     p.work_counter = &g->call->work_counter;
     // a rank without trials (more ranks than trials) still takes part in the exchange: one item-less CTA
     cudaError_t e = npk::launch_equity_uniform(players - 1, 5 - known, p, std::max<long long>(Q * chunks, 1), ds->sm_count,
-                                               tuning().warps, static_cast<cudaStream_t>(stream));
+                                               static_cast<cudaStream_t>(stream));
     return e == cudaSuccess ? NPK_OK : cuda_fail(e, "equity kernel launch (sharded)");
 }
 
@@ -1181,21 +1113,8 @@ __global__ void validate_ranges_kernel(const uint8_t* hole, const uint8_t* board
     uint32_t* invalid = reinterpret_cast<uint32_t*>(ws + kWsInvalid);
     for (long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x; q < Q; q += (long long)gridDim.x * blockDim.x) {
         const int np = n_players[q];
-        unsigned long long mask = 0;
-        int bad = np < 1 || np > 10;
-        bool ended = false;
-        if (hole)
-            for (int i = 0; i < 2; i++) {
-                const int c = hole[2 * q + i];
-                if (c >= 52) bad = 1; else { bad |= (int)(mask >> c & 1ull); mask |= 1ull << c; }
-            }
-        for (int i = 0; i < 5; i++) {
-            const int c = board[5 * q + i];
-            if (c == 0xFF) { ended = true; continue; }
-            if (ended || c >= 52) { bad = 1; continue; }
-            bad |= (int)(mask >> c & 1ull);
-            mask |= 1ull << c;
-        }
+        unsigned long long mask;
+        int bad = npk::validate_query(hole ? hole + 2 * q : nullptr, board + 5 * q, np, &mask) < 0;
         if (ghost) {
             // the reference pops ghost cards from the deck first (montecarlo_python.py:206-208): a board card equal to
             // a ghost card then fails list.index (ValueError); a hero card equal to one is silently kept (:154-161)
@@ -1235,11 +1154,8 @@ int npk_equity_ranges_known_batch(const uint8_t* hole, const uint8_t* board, con
                                   void* workspace, void* stream)
 {
     DeviceState* ds;
-    int rc = current_state(&ds);
-    if (rc) return rc;
-    if (Q < 0 || trials < 0 || trial_offset < 0) return fail(NPK_ERR_INVALID_ARGUMENT, "negative size");
-    if (Q == 0 || trials == 0) return NPK_OK;
-    if (Q > 0x7fffffffLL) return fail(NPK_ERR_INVALID_ARGUMENT, "at most 2^31-1 queries per call");
+    int rc = batch_start(&ds, Q, trials, trial_offset);
+    if (rc) return rc == kEmptyBatch ? NPK_OK : rc;
     if ((!hole && !hero_allowed) || !board || !n_players || !wins_strict || !ties || !workspace || !opp_allowed)
         return fail(NPK_ERR_INVALID_ARGUMENT, "null pointer");
     if (n_known < 0 || n_known > 9 || (n_known > 0 && !known_opp))
@@ -1247,8 +1163,7 @@ int npk_equity_ranges_known_batch(const uint8_t* hole, const uint8_t* board, con
     if (n_known > 0 && hero_allowed)
         return fail(NPK_ERR_INVALID_ARGUMENT, "a hero range together with known opponent hands is not supported (the reference "
                                               "draws the hero before it removes the known hands, montecarlo_python.py:132-163)");
-    if (deal_mode != NPK_DEAL_UNIFORM && deal_mode != NPK_DEAL_REFERENCE)
-        return fail(NPK_ERR_INVALID_ARGUMENT, "deal_mode must be NPK_DEAL_UNIFORM or NPK_DEAL_REFERENCE");
+    if ((rc = check_deal_mode(deal_mode))) return rc;
     const uint64_t top = (1ull << (169 - 128)) - 1ull;
     if (!(opp_allowed[0] | opp_allowed[1] | (opp_allowed[2] & top)))
         return fail(NPK_ERR_RANGE, "the opponent range is empty (the reference would never finish a draw)");
@@ -1256,23 +1171,15 @@ int npk_equity_ranges_known_batch(const uint8_t* hole, const uint8_t* board, con
         return fail(NPK_ERR_RANGE, "the hero range is empty (the reference would never finish a draw)");
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     uint8_t* ws = static_cast<uint8_t*>(workspace);
-    cudaError_t e = cudaMemsetAsync(ws, 0, kWsIndex, s);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(workspace)");
+    if ((rc = clear_workspace(ws, s))) return rc;
 
-    npk::EquityParams p{};
-    p.tables = ds->t;
-    p.hole = hero_allowed ? nullptr : hole; p.board = board; p.n_players = n_players; p.ghost = ghost;
+    npk::EquityParams p;
+    const long long chunks = fill_params(p, *ds, hero_allowed ? nullptr : hole, board, n_players, Q, trials, trial_offset,
+                                         query_offset, seed, deal_mode, wins_strict, ties, win_types, passes,
+                                         reinterpret_cast<uint32_t*>(ws + kWsAbort), 32);
+    p.ghost = ghost;
     p.known_opp = n_known > 0 ? known_opp : nullptr; p.n_known = (uint32_t)n_known;
-    p.trials = trials; p.trial_offset = trial_offset; p.query_offset = (uint32_t)query_offset;
-    p.seed_lo = (uint32_t)seed; p.seed_hi = (uint32_t)(seed >> 32);
-    const long long chunks = plan_items(p, Q, trials, ds->sm_count, 32);
-    p.wins = reinterpret_cast<unsigned long long*>(wins_strict);
-    p.ties = reinterpret_cast<unsigned long long*>(ties);
-    p.win_types = reinterpret_cast<unsigned long long*>(win_types);
-    p.passes = reinterpret_cast<unsigned long long*>(passes);
-    p.qindex = nullptr; p.nq = Q;
     p.work_counter = reinterpret_cast<unsigned long long*>(ws + kWsCounters);
-    p.abort_flag = reinterpret_cast<uint32_t*>(ws + kWsAbort);
     for (int i = 0; i < 3; i++) {
         const uint64_t o = i == 2 ? opp_allowed[i] & top : opp_allowed[i];
         const uint64_t h = hero_allowed ? (i == 2 ? hero_allowed[i] & top : hero_allowed[i]) : 0;
@@ -1282,6 +1189,7 @@ int npk_equity_ranges_known_batch(const uint8_t* hole, const uint8_t* board, con
     p.hero_range = hero_allowed ? 1u : 0u;
 
     const bool validate = (flags & NPK_FLAG_VALIDATE) != 0;
+    cudaError_t e;
     if (validate) {
         const int cg = (int)std::min<long long>((Q + 255) / 256, 4 * ds->sm_count);
         validate_ranges_kernel<<<cg, 256, 0, s>>>(p.hole, board, n_players, ghost, p.known_opp, n_known, Q, ws);

@@ -54,6 +54,31 @@ struct SmemTables {
 
 constexpr uint32_t kDescBytes = 256;   // the 52 card descriptors follow the flush table in the device blob, padded
 
+// What a valid equity query is, on the host and on the device: card ids < 52, no card twice, the board's empty slots (0xFF)
+// only at its end, and 1..10 players.  `hole` may be null (a hero drawn from a range).  Returns the number of known board
+// cards, or -1; `mask` (if given) receives the cards seen, one bit per id.
+__host__ __device__ __forceinline__ int validate_query(const uint8_t* hole, const uint8_t* board, int players,
+                                                       unsigned long long* mask = nullptr)
+{
+    unsigned long long m = 0;
+    int known = 0;
+    bool bad = players < 1 || players > 10, ended = false;
+    for (int i = 0; hole && i < 2; i++) {
+        const int c = hole[i];
+        if (c >= 52) bad = true; else { bad |= (m >> c & 1ull) != 0; m |= 1ull << c; }
+    }
+    for (int i = 0; i < 5; i++) {
+        const int c = board[i];
+        if (c == 0xFF) { ended = true; continue; }
+        if (ended || c >= 52) { bad = true; continue; }
+        bad |= (m >> c & 1ull) != 0;
+        m |= 1ull << c;
+        known++;
+    }
+    if (mask) *mask = m;
+    return bad ? -1 : known;
+}
+
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
 // ---- mbarrier + 1-D bulk copy (cp.async.bulk -> UBLKCP) -------------------------------------------------------------

@@ -21,46 +21,35 @@
 
 namespace npk {
 
-template <int NOPP, int NB>
-__global__ void __launch_bounds__(kEquityMaxThreads, 1) equity_uniform_kernel(const EquityParams p)
+// One kernel per shape and dealer: the warps pull the (query, trial range) items of queries 0..nq-1.  A rank of a sharded job
+// without trials runs one CTA without items, which still takes part in the peer exchange.
+template <int NOPP, int NB, int REF>
+__device__ __forceinline__ void shape_kernel_body(const EquityParams& p)
 {
-    constexpr int N = 45 + NB;             // unseen cards
-    // sync-free mixed batches: the size of this shape's group and the start of its query list live in device memory
-    const long long nq = p.group ? (long long)p.group[0] : p.nq;
-    if (nq == 0) return;                                   // nothing of this shape in the batch: leave before staging
-    const int32_t* qindex = p.group ? p.qindex + p.group[64] : p.qindex;
     extern __shared__ __align__(128) uint8_t smem[];
-    const WarpCtx cx = warp_context(p, smem, 64 + N * 32);
+    const WarpCtx cx = warp_context(p, smem, 64 + (45 + NB) * 32);
     const int lane = cx.lane;
-    const long long n_items = nq * p.chunks;
+    const long long n_items = p.nq * p.chunks;
     for (long long item = next_item(p.work_counter, lane); item < n_items; item = next_item(p.work_counter, lane)) {
-        long long qslot, t_begin, t_end;
-        item_range(p, item, qslot, t_begin, t_end);
-        uniform_item<NOPP, NB>(p, cx, qindex ? qindex[qslot] : qslot, t_begin, t_end);
+        long long q, t_begin, t_end;
+        item_range(p, item, q, t_begin, t_end);
+        if (REF) refdeal_item<NOPP, NB>(p, cx, q, t_begin, t_end);
+        else uniform_item<NOPP, NB>(p, cx, q, t_begin, t_end);
     }
     finish_single_call(p, lane);
     if (p.peer) finish_peer(p.peer, p.peer_epoch, p.peer_totals, p.peer_words, lane);
 }
 
 template <int NOPP, int NB>
+__global__ void __launch_bounds__(kEquityMaxThreads, 1) equity_uniform_kernel(const EquityParams p)
+{
+    shape_kernel_body<NOPP, NB, 0>(p);
+}
+
+template <int NOPP, int NB>
 __global__ void __launch_bounds__(kEquityMaxThreads, 1) equity_refdeal_kernel(const EquityParams p)
 {
-    constexpr int N = 45 + NB;             // unseen cards
-    // sync-free mixed batches: the size of this shape's group and the start of its query list live in device memory
-    const long long nq = p.group ? (long long)p.group[0] : p.nq;
-    if (nq == 0) return;                                   // nothing of this shape in the batch: leave before staging
-    const int32_t* qindex = p.group ? p.qindex + p.group[64] : p.qindex;
-    extern __shared__ __align__(128) uint8_t smem[];
-    const WarpCtx cx = warp_context(p, smem, 64 + N * 32);
-    const int lane = cx.lane;
-    const long long n_items = nq * p.chunks;
-    for (long long item = next_item(p.work_counter, lane); item < n_items; item = next_item(p.work_counter, lane)) {
-        long long qslot, t_begin, t_end;
-        item_range(p, item, qslot, t_begin, t_end);
-        refdeal_item<NOPP, NB>(p, cx, qindex ? qindex[qslot] : qslot, t_begin, t_end);
-    }
-    finish_single_call(p, lane);
-    if (p.peer) finish_peer(p.peer, p.peer_epoch, p.peer_totals, p.peer_words, lane);
+    shape_kernel_body<NOPP, NB, 1>(p);
 }
 
 // =====================================================================================================================
@@ -94,9 +83,8 @@ __global__ void __launch_bounds__(kRefThreads, 1) equity_ranges_kernel(const Equ
     const long long n_items = p.nq * p.chunks;
 
     for (long long item = next_item(p.work_counter, lane); item < n_items; item = next_item(p.work_counter, lane)) {
-        long long qslot, t_begin, t_end;
-        item_range(p, item, qslot, t_begin, t_end);
-        const long long q = p.qindex ? p.qindex[qslot] : qslot;
+        long long q, t_begin, t_end;
+        item_range(p, item, q, t_begin, t_end);
         int known = 0;
         for (int i = 0; i < 5; i++) known += p.board[5 * q + i] != 0xFF;
         // opponents dealt at random; the others' cards are known (montecarlo_python.py:132-163: removed from the deck like the
@@ -614,27 +602,22 @@ cudaError_t launch_int_peak(int variant, uint32_t* out, int iters, int grid, cud
 // ---------------------------------------------------------------------------------------------------------------------
 // Shared memory decides the CTA shape: tables + one private deck per warp.  As many warps as fit (at most 16) run on
 // each SM; the deck of N = 45..50 cards costs 128 B per card per warp.
-static int uniform_warps(const DeviceTables& t, int nb, int forced)
+static int uniform_warps(const DeviceTables& t, int nb)
 {
     const size_t fixed = 128 + (size_t)t.value_bytes + t.rowoff_bytes + t.flush_bytes + kDescBytes;
     const size_t per_warp = (size_t)(64 + (45 + nb) * 32) * 4;
     int w = (int)((kMaxDynamicSmem - fixed) / per_warp);
     if (w > kEquityMaxThreads / 32) w = kEquityMaxThreads / 32;
-    if (forced > 0 && forced < w) w = forced;
     return w < 1 ? 1 : w;
 }
 
 constexpr int kMaxDevicesForAttr = 64;
 
 template <int NOPP, int NB>
-static cudaError_t launch_uniform_t(const EquityParams& p, long long items, int sm_count, int forced_warps, cudaStream_t s)
+static cudaError_t launch_uniform_t(const EquityParams& p, long long items, int sm_count, cudaStream_t s)
 {
-#ifdef NPK_UNIFORM_LEHMER
-    auto k = equity_refdeal_kernel<NOPP, NB>;      // experiment build: every deal mode through the Lehmer path
-#else
     auto k = p.reference_dealer ? equity_refdeal_kernel<NOPP, NB> : equity_uniform_kernel<NOPP, NB>;
-#endif
-    const int warps = uniform_warps(p.tables, NB, forced_warps);
+    const int warps = uniform_warps(p.tables, NB);
     const size_t smem = 128 + (size_t)p.tables.value_bytes + p.tables.rowoff_bytes + p.tables.flush_bytes + kDescBytes +
                         (size_t)warps * (64 + (45 + NB) * 32) * 4;
     // the opt-in is per kernel and per device: ask the driver once, not on every launch of a 20 us call
@@ -655,33 +638,32 @@ static cudaError_t launch_uniform_t(const EquityParams& p, long long items, int 
 }
 
 template <int NB>
-static cudaError_t launch_uniform_nb(int nopp, const EquityParams& p, long long items, int sm_count, int fw, cudaStream_t s)
+static cudaError_t launch_uniform_nb(int nopp, const EquityParams& p, long long items, int sm_count, cudaStream_t s)
 {
     switch (nopp) {
-        case 0: return launch_uniform_t<0, NB>(p, items, sm_count, fw, s);
-        case 1: return launch_uniform_t<1, NB>(p, items, sm_count, fw, s);
-        case 2: return launch_uniform_t<2, NB>(p, items, sm_count, fw, s);
-        case 3: return launch_uniform_t<3, NB>(p, items, sm_count, fw, s);
-        case 4: return launch_uniform_t<4, NB>(p, items, sm_count, fw, s);
-        case 5: return launch_uniform_t<5, NB>(p, items, sm_count, fw, s);
-        case 6: return launch_uniform_t<6, NB>(p, items, sm_count, fw, s);
-        case 7: return launch_uniform_t<7, NB>(p, items, sm_count, fw, s);
-        case 8: return launch_uniform_t<8, NB>(p, items, sm_count, fw, s);
-        case 9: return launch_uniform_t<9, NB>(p, items, sm_count, fw, s);
+        case 0: return launch_uniform_t<0, NB>(p, items, sm_count, s);
+        case 1: return launch_uniform_t<1, NB>(p, items, sm_count, s);
+        case 2: return launch_uniform_t<2, NB>(p, items, sm_count, s);
+        case 3: return launch_uniform_t<3, NB>(p, items, sm_count, s);
+        case 4: return launch_uniform_t<4, NB>(p, items, sm_count, s);
+        case 5: return launch_uniform_t<5, NB>(p, items, sm_count, s);
+        case 6: return launch_uniform_t<6, NB>(p, items, sm_count, s);
+        case 7: return launch_uniform_t<7, NB>(p, items, sm_count, s);
+        case 8: return launch_uniform_t<8, NB>(p, items, sm_count, s);
+        case 9: return launch_uniform_t<9, NB>(p, items, sm_count, s);
         default: return cudaErrorInvalidValue;
     }
 }
 
-cudaError_t launch_equity_uniform(int nopp, int nb, const EquityParams& p, long long items, int sm_count, int forced_warps,
-                                  cudaStream_t s)
+cudaError_t launch_equity_uniform(int nopp, int nb, const EquityParams& p, long long items, int sm_count, cudaStream_t s)
 {
     switch (nb) {
-        case 0: return launch_uniform_nb<0>(nopp, p, items, sm_count, forced_warps, s);
-        case 1: return launch_uniform_nb<1>(nopp, p, items, sm_count, forced_warps, s);
-        case 2: return launch_uniform_nb<2>(nopp, p, items, sm_count, forced_warps, s);
-        case 3: return launch_uniform_nb<3>(nopp, p, items, sm_count, forced_warps, s);
-        case 4: return launch_uniform_nb<4>(nopp, p, items, sm_count, forced_warps, s);
-        case 5: return launch_uniform_nb<5>(nopp, p, items, sm_count, forced_warps, s);
+        case 0: return launch_uniform_nb<0>(nopp, p, items, sm_count, s);
+        case 1: return launch_uniform_nb<1>(nopp, p, items, sm_count, s);
+        case 2: return launch_uniform_nb<2>(nopp, p, items, sm_count, s);
+        case 3: return launch_uniform_nb<3>(nopp, p, items, sm_count, s);
+        case 4: return launch_uniform_nb<4>(nopp, p, items, sm_count, s);
+        case 5: return launch_uniform_nb<5>(nopp, p, items, sm_count, s);
         default: return cudaErrorInvalidValue;
     }
 }

@@ -20,10 +20,6 @@ constexpr int kRank7Threads = 1024;    // rank7 is latency-bound at one CTA per 
 struct SingleResult {             // in mapped host memory
     unsigned long long wins, ties, win_types[9], passes;
     unsigned long long seq;       // number of the call these values belong to: written last, the host spins on it
-    unsigned long long pad_[3];
-    // the common case (wins and ties only, fewer than 2^32 trials): ONE 16-byte store carries counters and sequence number,
-    // so the hand-over needs no system-wide fence between data and flag
-    struct __align__(16) Quick { unsigned int wins, ties; unsigned long long seq; } quick;
 };
 struct SingleCall {               // in device memory
     unsigned long long wins, ties, win_types[9], passes;
@@ -82,11 +78,10 @@ struct EquityParams {
     const uint8_t* hole;          // [Q,2] card ids
     const uint8_t* board;         // [Q,5] card ids, 0xFF = not dealt yet (known cards first)
     const uint8_t* n_players;     // [Q]
-    const int32_t* qindex;        // [nq] query ids handled by this launch, or null = 0..nq-1
-    const uint32_t* group;        // device {count, offset} of this launch's shape group (sync-free mixed batches), or null:
-                                  // then nq = group[0] and qindex starts at qindex + group[64].  The all-shapes kernel
-                                  // (npk_mixed.cu) reads all 60 groups: counts group[0..59], offsets group[64..123]
-    long long nq;
+    const int32_t* qindex;        // all-shapes kernel only (npk_mixed.cu): query ids sorted by shape
+    const uint32_t* group;        // all-shapes kernel only: queries per shape group[0..59], their first qindex slot
+                                  // group[64..123]
+    long long nq;                 // queries 0..nq-1 of the per-shape and range kernels
     long long trials;             // trials per query in this launch
     long long trial_offset;       // first trial number (sharding a query over launches / GPUs)
     uint32_t query_offset;        // added to the query number in the Philox counter (sharding queries over GPUs)
@@ -102,7 +97,6 @@ struct EquityParams {
     uint64_t inline_query;        // hole[2] | board[5] << 16 (bytes), used when `hole` is null
     SingleCall* single;           // device scratch + mapped host result block, or null
     unsigned long long single_seq;
-    uint32_t single_quick;        // 1: publish through SingleResult::quick
     // ---- trial-sharded job: reduce the counters over the ranks inside the kernel ----
     PeerCall* peer;               // or null
     unsigned long long peer_epoch;
@@ -133,8 +127,7 @@ struct EnumParams {
 };
 
 size_t aux_smem(const DeviceTables& t);
-cudaError_t launch_equity_uniform(int nopp, int nb, const EquityParams& p, long long items, int sm_count, int forced_warps,
-                                  cudaStream_t s);
+cudaError_t launch_equity_uniform(int nopp, int nb, const EquityParams& p, long long items, int sm_count, cudaStream_t s);
 cudaError_t launch_equity_mixed(const EquityParams& p, int sm_count, cudaStream_t s);
 cudaError_t launch_equity_resident(const DeviceTables& t, ResidentState* st, ResidentMailbox* mb, unsigned long long launch_id,
                                    unsigned int last_seq, long long idle_cycles, int ctas, cudaStream_t s);

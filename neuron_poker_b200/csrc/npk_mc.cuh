@@ -79,15 +79,6 @@ __device__ __forceinline__ void finish_single_call(const EquityParams& p, int la
         v = atomicExch(src + lane, 0ull);                             // read and reset for the next call
     }
     if (lane == 0) { sc->work_counter = 0; sc->ticket = 0; }
-    if (p.single_quick) {
-        const unsigned long long t = __shfl_sync(0xffffffffu, v, 1);
-        if (lane == 0) {
-            const uint4 q = make_uint4((unsigned int)v, (unsigned int)t, (unsigned int)p.single_seq, (unsigned int)(p.single_seq >> 32));
-            asm volatile("st.global.v4.u32 [%0], {%1, %2, %3, %4};" ::"l"(&sc->host->quick), "r"(q.x), "r"(q.y), "r"(q.z), "r"(q.w)
-                         : "memory");                                                                     // one 16-byte store
-        }
-        return;
-    }
     if (lane < 12) (&sc->host->wins)[lane] = v;
     __threadfence_system();
     __syncwarp();
@@ -418,41 +409,11 @@ __device__ __forceinline__ int select_bit(uint64_t m, int k)
     return base;
 }
 
-// NPK_IMAD_LEVEL (experiment, kept for the record): multipliers read from constant memory stop ptxas from strength-reducing
-// the multiply-adds below into LEA / SHF / IADD3 (alu pipe) and keep them on the fma pipe (IMAD).  Measured on B200, cfg3
-// with the reference's dealer: level 0 (ptxas decides: SHF + IMAD.IADD) 380 G evals/s, level 1 (pack / unpack / shift as
-// IMAD) 352 G, level 2 (the add of the bump as IMAD too) 349 G -- ptxas balances the two pipes better than a fixed rule.
-#ifndef NPK_IMAD_LEVEL
-#define NPK_IMAD_LEVEL 0
-#endif
-static __constant__ uint32_t c_mul[12] = {1u, 256u, 65536u, 1u << 24, 1u << 25, 128u, 1u << 31, 1u << 23, 1u << 15, 0u, 0u, 0u};
-
-__device__ __forceinline__ uint32_t imad_lo(uint32_t a, uint32_t b, uint32_t c)
-{
-    uint32_t r;
-    asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(r) : "r"(a), "r"(b), "r"(c));
-    return r;
-}
-__device__ __forceinline__ uint32_t imad_hi(uint32_t a, uint32_t b, uint32_t c)
-{
-    uint32_t r;
-    asm("mad.hi.u32 %0, %1, %2, %3;" : "=r"(r) : "r"(a), "r"(b), "r"(c));
-    return r;
-}
-
 // x4 + (((x4 + c) & h) >> 7): the byte-wise "bump" of the Lehmer sweep
 __device__ __forceinline__ uint32_t bump4(uint32_t x4, uint32_t c, uint32_t h)
 {
-#if NPK_IMAD_LEVEL >= 2
-    const uint32_t t = imad_lo(x4, c_mul[0], c) & h;
-#else
     const uint32_t t = (x4 + c) & h;
-#endif
-#if NPK_IMAD_LEVEL >= 1
-    return imad_hi(t, c_mul[4], x4);
-#else
     return x4 + (t >> 7);
-#endif
 }
 
 // Decode D pop indices (raw[k] < 64, pop k taken from the list shortened by pops 0..k-1) into canonical slots, packed
@@ -466,13 +427,7 @@ __device__ __forceinline__ void lehmer_decode(const uint32_t (&raw)[D > 0 ? D : 
         uint32_t v = raw[4 * g];
 #pragma unroll
         for (int b = 1; b < 4; b++)
-            if (4 * g + b < D) {
-#if NPK_IMAD_LEVEL >= 1
-                v = imad_lo(raw[4 * g + b], c_mul[b], v);
-#else
-                v += raw[4 * g + b] << (8 * b);
-#endif
-            }
+            if (4 * g + b < D) v += raw[4 * g + b] << (8 * b);
         x4[g] = v;
     }
 #pragma unroll
@@ -493,11 +448,7 @@ __device__ __forceinline__ void lehmer_decode(const uint32_t (&raw)[D > 0 ? D : 
 __device__ __forceinline__ uint32_t slot_addr(uint32_t x4, int b, uint32_t base)
 {
     const uint32_t f = x4 & (0xFFu << (8 * b));
-#if NPK_IMAD_LEVEL >= 1
-    return b == 0 ? imad_lo(f, c_mul[5], base) : imad_hi(f, c_mul[5 + b], base);
-#else
     return b == 0 ? base + f * 128u : base + (f >> (8 * b - 7));
-#endif
 }
 
 template <int NOPP, int NB>
@@ -507,11 +458,7 @@ __device__ __forceinline__ void refdeal_item(const EquityParams& p, const WarpCt
     constexpr int KNOWN = 5 - NB;
     constexpr int N = 50 - KNOWN;          // unseen cards
     constexpr int D = 2 * NOPP + NB;       // cards dealt per trial
-#ifdef NPK_UNIFORM_LEHMER       // experiment: UNIFORM index law (every pop uniform over the remaining list) through the same path
-    constexpr int NWR = (D + 1) / 2;
-#else
     constexpr int NWR = NOPP + (NB + 1) / 2;       // Philox words per trial
-#endif
     constexpr int NBLK2 = (2 * NWR + 3) / 4;       // Philox blocks per trial PAIR
     constexpr int G = (D + 3) / 4;
     static_assert(D <= N, "not enough cards");
@@ -552,17 +499,6 @@ __device__ __forceinline__ void refdeal_item(const EquityParams& p, const WarpCt
 #pragma unroll
         for (int u = 0; u < 2; u++) {
             uint32_t raw[D > 0 ? D : 1];
-#ifdef NPK_UNIFORM_LEHMER
-            {
-                uint32_t remw = 0;
-#pragma unroll
-                for (int k = 0; k < D; k++) {
-                    const uint32_t x = (k & 1) ? remw : w[u * NWR + (k >> 1)];
-                    raw[k] = __umulhi(x, (uint32_t)(N - k));
-                    remw = x * (uint32_t)(N - k);
-                }
-            }
-#else
 #pragma unroll
             for (int o = 0; o < NOPP; o++) {
                 const uint32_t m = (uint32_t)(N - 2 * o - 1);              // n - 1
@@ -579,7 +515,6 @@ __device__ __forceinline__ void refdeal_item(const EquityParams& p, const WarpCt
                 raw[2 * NOPP + c] = __umulhi(x, m);
                 rem = x * m;
             }
-#endif
             uint32_t x4[G > 0 ? G : 1];
             lehmer_decode<D>(raw, x4);
 #pragma unroll

@@ -89,9 +89,8 @@ __global__ void __launch_bounds__(kRefThreads, 1) equity_ranges_fast_kernel(cons
 
     const long long n_items = p.nq * p.chunks;
     for (long long item = next_item(p.work_counter, lane); item < n_items; item = next_item(p.work_counter, lane)) {
-        long long qslot, t_begin, t_end;
-        item_range(p, item, qslot, t_begin, t_end);
-        const long long q = p.qindex ? p.qindex[qslot] : qslot;
+        long long q, t_begin, t_end;
+        item_range(p, item, q, t_begin, t_end);
         int known = 0;
         for (int i = 0; i < 5; i++) known += p.board[5 * q + i] != 0xFF;
         const int nknown = (int)p.n_known;                    // opponents whose cards are known (montecarlo_python.py:132-163)

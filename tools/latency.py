@@ -1,4 +1,4 @@
-"""Latency of one blocking get_equity call (10,000 runs, 6 players, flop), with and without the one-query fast path."""
+"""Latency of one blocking get_equity call (10,000 runs, 6 players, flop), launched per call and through the resident server."""
 import sys, os, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import neuron_poker_b200 as npk
@@ -8,7 +8,7 @@ for mode, fn in (("reference", lambda: npk.get_equity({"AS", "KS"}, {"2C", "7D",
     t0 = time.perf_counter(); n = 2000
     vals = [fn() for _ in range(n)]
     dt = time.perf_counter() - t0
-    print(mode, "%.1f us/call  %.0f calls/s  mean equity %.4f" % (1e6 * dt / n, n / dt, sum(vals) / n), "single path" if not os.environ.get("NPK_NO_SINGLE_PATH") else "general path", flush=True)
+    print(mode, "%.1f us/call  %.0f calls/s  mean equity %.4f" % (1e6 * dt / n, n / dt, sum(vals) / n), flush=True)
 # the same calls with the resident server (no kernel launch per call)
 import ctypes
 for sms in (0, 64, 16):
