@@ -17,6 +17,8 @@
  *   npk_rank7_batch     _calc_score ordering                      tools/hand_evaluator.py:27-119
  *   npk_showdown_batch  get_winner / eval_best_hand               tools/hand_evaluator.py:9-24 (used by gym_env/env.py:576-593)
  *   npk_enum_batch      no counterpart (the reference only samples); exact enumeration used for bit-exact checks
+ *   npk_showdown_equity_batch  run_montecarlo with every hand in player_card_list known (:132-163, ghost cards :206-208),
+ *                       computed exactly (every board completion) and for every player, split pots included
  *
  * Cards are bytes: id = 4*rank + suit with ranks "23456789TJQKA" and suits "CDHS" -- the order of
  * MonteCarlo.create_card_deck (tools/montecarlo_python.py:114-119).  0xFF marks "no card" in board arrays.
@@ -259,6 +261,30 @@ int npk_enum_batch(const uint8_t* hole, const uint8_t* board, const uint8_t* n_p
  * best hands (hand_evaluator.py:23 stable sort), wtype [N] = its hand type 0..8, ranks [N,maxp] or NULL. */
 int npk_showdown_batch(const uint8_t* holes, const uint8_t* n_players, const uint8_t* board, int64_t N, int maxp,
                        int32_t* winner, uint8_t* wtype, uint16_t* ranks, uint32_t flags, void* stream);
+
+/*
+ * Exact showdown equity of KNOWN hands: for every spot, every completion of the board from the unseen cards is enumerated
+ * once and scored for every player.
+ *   holes [N,maxp,2]  the hands of players 0..n_players[s]-1 (maxp 1..10)   n_players [N]   board [N,5] 0xFF padding
+ *   dead  [N] or NULL  one bit per card id removed from the deck (the reference's ghost cards)
+ * The unseen cards U are the 52 minus hands, board and dead cards.  NPK_DEAL_UNIFORM enumerates every m-subset of U
+ * (m = missing board cards); NPK_DEAL_REFERENCE leaves the highest id of U out when m >= 1 -- the reference deals a board
+ * card with pop(randint(0, len-1)) from its id-ordered list (montecarlo_python.py:185-189) and so never deals the last one.
+ * Per completion, with best = the highest rank id and k = the number of players holding it, each of those k players gets
+ * win += (k == 1), tie += (k > 1), share += NPK_SHARE_UNIT / k.  Outputs (u64) are OVERWRITTEN; entries p >= n_players[s] are 0:
+ *   win, tie, share [N,maxp]   completions [N] = C(|U'|, m)     sum_p share = NPK_SHARE_UNIT * completions
+ *   split-pot equity = share / (NPK_SHARE_UNIT * completions); the reference's equity (ties count as wins) = (win + tie) / completions
+ * workspace: npk_showdown_equity_workspace_bytes(N) bytes, private to the call until it completes.  Asynchronous and free of host
+ * round trips (graph-capturable) unless NPK_FLAG_VALIDATE is set: NPK_ERR_INVALID_CARDS for an id >= 52, a card twice across
+ * hands, board and dead mask, a gap in the board or a dead bit >= 52; NPK_ERR_INVALID_ARGUMENT for n_players outside 1..maxp or
+ * fewer cards left than missing board cards.  Without the flag such a spot is memory-safe, and one with fewer cards left than
+ * missing gets completions = 0 and zero counters.
+ */
+#define NPK_SHARE_UNIT 2520   /* lcm(1..10): a pot split k ways gives each of the k players 2520 / k */
+int64_t npk_showdown_equity_workspace_bytes(int64_t N);
+int npk_showdown_equity_batch(const uint8_t* holes, const uint8_t* n_players, const uint8_t* board, const uint64_t* dead,
+                              int64_t N, int maxp, int deal_mode, uint32_t flags, uint64_t* win, uint64_t* tie, uint64_t* share,
+                              uint64_t* completions, void* workspace, void* stream);
 
 /* Integer-issue microbenchmark on the current device (the roofline denominator of the Monte-Carlo kernel):
  * variant 0 = LOP3 chains (alu pipe), 1 = IMAD chains (fma pipe), 2 = both interleaved.  Reports executed

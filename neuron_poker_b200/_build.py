@@ -9,7 +9,8 @@ import subprocess
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libnpk.so")
-SOURCES = ["npk_capi.cu", "npk_kernels.cu", "npk_mixed.cu", "npk_ranges.cu", "npk_holdem.cu", "npk_tables.cpp"]
+SOURCES = ["npk_capi.cu", "npk_kernels.cu", "npk_mixed.cu", "npk_ranges.cu", "npk_holdem.cu", "npk_showdown_equity.cu",
+           "npk_tables.cpp"]
 HEADERS = ["npk_kernels.h", "npk_device.cuh", "npk_mc.cuh", "npk_tables.h", "npk_holdem_launch.h",
            os.path.join("..", "..", "include", "npk.h"), os.path.join("..", "..", "include", "npk_holdem.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

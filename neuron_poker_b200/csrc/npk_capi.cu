@@ -1275,8 +1275,11 @@ int npk_equity_ranges_known_host(const uint8_t* hole, const uint8_t* board, cons
 // ---- validation of the evaluator entry points (NPK_FLAG_VALIDATE) -----------------------------------------------------------
 // rows of `len` card ids: every id < 52 and no id twice.  enum_mode: the row is hole[2] + board[5] (0xFF padding allowed
 // at the end of the board only) and the shape must be one enum_kernel implements.
+// mode 2 (npk_showdown_equity_batch): the same board rule, the optional dead mask of the row takes part in the duplicate test
+// (a bit >= 52 is an invalid card), and the cards left to deal from -- one fewer in REFERENCE mode -- must cover the board.
 __global__ void check_rows_kernel(const uint8_t* a, int len_a, const uint8_t* b, int len_b, const uint8_t* n_players,
-                                  int maxp, int enum_mode, long long n, uint32_t* bad /*[2]: cards, shape*/)
+                                  int maxp, int enum_mode, long long n, uint32_t* bad /*[2]: cards, shape*/,
+                                  const uint64_t* dead, int deal_mode)
 {
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
         unsigned long long mask = 0;
@@ -1300,8 +1303,17 @@ __global__ void check_rows_kernel(const uint8_t* a, int len_a, const uint8_t* b,
             mask |= 1ull << c;
             known++;
         }
+        if (dead) {
+            const unsigned long long d = dead[i];
+            wrong |= (d >> 52) != 0 || (d & mask) != 0;
+            mask |= d;
+        }
         if (wrong) atomicAdd(&bad[0], 1u);
-        if (enum_mode) {
+        if (enum_mode == 2) {
+            const int missing = 5 - known;
+            const int left = 52 - __popcll(mask & ((1ull << 52) - 1ull)) - (deal_mode == NPK_DEAL_REFERENCE && missing > 0 ? 1 : 0);
+            if (left < missing) atomicAdd(&bad[1], 1u);
+        } else if (enum_mode) {
             const int np = n_players[i];
             if (!(np == 2 || (np == 3 && known == 5))) atomicAdd(&bad[1], 1u);
         }
@@ -1310,14 +1322,15 @@ __global__ void check_rows_kernel(const uint8_t* a, int len_a, const uint8_t* b,
 
 namespace {
 int check_rows(DeviceState* ds, const uint8_t* a, int len_a, const uint8_t* b, int len_b, const uint8_t* n_players, int maxp,
-               int enum_mode, int64_t n, cudaStream_t s, const char* shape_msg)
+               int enum_mode, int64_t n, cudaStream_t s, const char* shape_msg, const uint64_t* dead = nullptr,
+               int deal_mode = NPK_DEAL_UNIFORM)
 {
     uint32_t* d_bad = nullptr;
     cudaError_t e = cudaMalloc(&d_bad, 8);
     if (e == cudaSuccess) e = cudaMemsetAsync(d_bad, 0, 8, s);
     if (e != cudaSuccess) { cudaFree(d_bad); return cuda_fail(e, "validation scratch"); }
     const int grid = (int)std::min<long long>((n + 255) / 256, 8 * ds->sm_count);
-    check_rows_kernel<<<grid, 256, 0, s>>>(a, len_a, b, len_b, n_players, maxp, enum_mode, n, d_bad);
+    check_rows_kernel<<<grid, 256, 0, s>>>(a, len_a, b, len_b, n_players, maxp, enum_mode, n, d_bad, dead, deal_mode);
     uint32_t bad[2] = {0, 0};
     e = cudaMemcpyAsync(bad, d_bad, 8, cudaMemcpyDeviceToHost, s);
     if (e == cudaSuccess) e = cudaStreamSynchronize(s);
@@ -1398,6 +1411,38 @@ int npk_showdown_batch(const uint8_t* holes, const uint8_t* n_players, const uin
     cudaError_t e = npk::launch_showdown(ds->t, holes, n_players, board, N, maxp, winner, wtype, ranks,
                                          grid_for(*ds, (N + 127) / 128, npk::kRank7Threads / 32), static_cast<cudaStream_t>(stream));
     return e == cudaSuccess ? NPK_OK : cuda_fail(e, "showdown_kernel launch");
+}
+
+int64_t npk_showdown_equity_workspace_bytes(int64_t N) { return npk::showdown_equity_workspace_bytes(N); }
+
+int npk_showdown_equity_batch(const uint8_t* holes, const uint8_t* n_players, const uint8_t* board, const uint64_t* dead,
+                              int64_t N, int maxp, int deal_mode, uint32_t flags, uint64_t* win, uint64_t* tie, uint64_t* share,
+                              uint64_t* completions, void* workspace, void* stream)
+{
+    DeviceState* ds;
+    int rc = batch_start(&ds, N, 1, 0);
+    if (rc) return rc == kEmptyBatch ? NPK_OK : rc;
+    if (maxp < 1 || maxp > 10) return fail(NPK_ERR_INVALID_ARGUMENT, "maxp must be 1..10");
+    if ((rc = check_deal_mode(deal_mode))) return rc;
+    if (!holes || !n_players || !board || !win || !tie || !share || !completions || !workspace)
+        return fail(NPK_ERR_INVALID_ARGUMENT, "null pointer");
+    const cudaStream_t s = static_cast<cudaStream_t>(stream);
+    if (flags & NPK_FLAG_VALIDATE) {
+        rc = check_rows(ds, holes, 2 * maxp, board, 5, n_players, maxp, 2, N, s,
+                        " spot(s) with n_players outside 1..maxp or fewer cards left than missing board cards", dead, deal_mode);
+        if (rc) return rc;
+    }
+    npk::ShowdownEquityParams p{};
+    p.tables = ds->t;
+    p.holes = holes; p.n_players = n_players; p.board = board; p.dead = dead;
+    p.n = N; p.maxp = maxp; p.reference = deal_mode == NPK_DEAL_REFERENCE; p.sm_count = ds->sm_count;
+    p.win = reinterpret_cast<unsigned long long*>(win);
+    p.tie = reinterpret_cast<unsigned long long*>(tie);
+    p.share = reinterpret_cast<unsigned long long*>(share);
+    p.completions = reinterpret_cast<unsigned long long*>(completions);
+    p.workspace = static_cast<uint8_t*>(workspace);
+    cudaError_t e = npk::launch_showdown_equity(p, s);
+    return e == cudaSuccess ? NPK_OK : cuda_fail(e, "showdown_equity_kernel launch");
 }
 
 // ---- vectorised HoldemTable (include/npk_holdem.h) ------------------------------------------------------------------------

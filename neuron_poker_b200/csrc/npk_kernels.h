@@ -126,7 +126,27 @@ struct EnumParams {
     unsigned long long* lose;
 };
 
+// exact showdown equity of known hands (npk_showdown_equity.cu)
+struct ShowdownEquityParams {
+    DeviceTables tables;
+    const uint8_t* holes;         // [n, maxp, 2]
+    const uint8_t* n_players;     // [n]
+    const uint8_t* board;         // [n, 5], 0xFF padding
+    const uint64_t* dead;         // [n] masks, or null
+    long long n;
+    int maxp;
+    int reference;                // 1: NPK_DEAL_REFERENCE (the highest unseen id is never dealt)
+    int sm_count;
+    unsigned long long* win;      // [n, maxp]
+    unsigned long long* tie;      // [n, maxp]
+    unsigned long long* share;    // [n, maxp]
+    unsigned long long* completions;   // [n]
+    uint8_t* workspace;           // showdown_equity_workspace_bytes(n)
+};
+
 size_t aux_smem(const DeviceTables& t);
+long long showdown_equity_workspace_bytes(long long n);
+cudaError_t launch_showdown_equity(const ShowdownEquityParams& p, cudaStream_t s);
 cudaError_t launch_equity_uniform(int nopp, int nb, const EquityParams& p, long long items, int sm_count, cudaStream_t s);
 cudaError_t launch_equity_mixed(const EquityParams& p, int sm_count, cudaStream_t s);
 cudaError_t launch_equity_resident(const DeviceTables& t, ResidentState* st, ResidentMailbox* mb, unsigned long long launch_id,

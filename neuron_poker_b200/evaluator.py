@@ -130,6 +130,84 @@ def enumerate_equity(hole, board, n_players=None, device=None, validate=None):
     return win, tie, lose
 
 
+SHARE_UNIT = 2520   # NPK_SHARE_UNIT: lcm(1..10), a pot split k ways gives each of the k players 2520 / k
+
+
+def _u8_tensor(x, dev):
+    torch = _torch()
+    if not isinstance(x, torch.Tensor):
+        x = torch.as_tensor(np.ascontiguousarray(x, dtype=np.uint8))
+    return x.to(dev).contiguous()
+
+
+def _dead_masks(dead, n, dev):
+    """[N, k] card ids with 0xFF padding -> [N] int64 masks, one bit per id (ids 52..254 map to bits the validation rejects)."""
+    torch = _torch()
+    ids = _u8_tensor(dead, dev).view(n, -1).to(torch.int64)
+    bits = torch.where(ids == 0xFF, torch.zeros_like(ids), torch.bitwise_left_shift(torch.ones_like(ids), ids.clamp(max=63)))
+    mask = torch.zeros(n, dtype=torch.int64, device=dev)
+    for j in range(bits.shape[1]):
+        mask |= bits[:, j]
+    return mask
+
+
+def showdown_equity_batch(holes, n_players, board, dead=None, deal_mode="uniform", device=None, validate=None):
+    """Exact showdown equity of known hands: every completion of each spot's board, scored for every player.
+    holes [N,maxp,2] (maxp 1..10), n_players [N], board [N,5] with 0xFF padding, dead [N,k] card ids removed from the deck
+    (0xFF padding) or None.  deal_mode "uniform" enumerates every board completion from the unseen cards; "reference" leaves out
+    the highest unseen id, which the reference's dealer never deals.  Returns a dict of int64 CUDA tensors: win, tie, share
+    [N,maxp] (share in units of 1/2520 pot per completion) and completions [N]; entries of players >= n_players are 0."""
+    from .equity import _DEAL
+    torch = _torch()
+    dev = _dev(device)
+    flags = _want_check(holes, validate)
+    holes, board, n_players = _u8_tensor(holes, dev), _u8_tensor(board, dev), _u8_tensor(n_players, dev)
+    N = holes.shape[0]
+    maxp = holes.shape[1] if holes.dim() == 3 else 0
+    if holes.dim() != 3 or holes.shape[2] != 2 or board.shape != (N, 5) or n_players.shape != (N,):
+        raise ValueError("expected holes [N,maxp,2], n_players [N] and board [N,5]")
+    masks = _dead_masks(dead, N, dev) if dead is not None and N else None
+    L = _lib.ensure_init(dev.index)
+    out = {k: torch.empty((N, maxp), dtype=torch.int64, device=dev) for k in ("win", "tie", "share")}
+    out["completions"] = torch.empty(N, dtype=torch.int64, device=dev)
+    ws = torch.empty(int(L.npk_showdown_equity_workspace_bytes(N)), dtype=torch.uint8, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(L.npk_showdown_equity_batch(holes.data_ptr(), n_players.data_ptr(), board.data_ptr(),
+                                               masks.data_ptr() if masks is not None else None, N, maxp, _DEAL[deal_mode],
+                                               flags, out["win"].data_ptr(), out["tie"].data_ptr(), out["share"].data_ptr(),
+                                               out["completions"].data_ptr(), ws.data_ptr(),
+                                               torch.cuda.current_stream(dev).cuda_stream))
+    return out
+
+
+def showdown_equity(hands, table_cards=(), dead_cards=(), deal_mode="uniform"):
+    """Exact equity of one spot whose hands are all known -- run_montecarlo with every entry of player_card_list known,
+    without sampling, for every player.  hands: two card strings per player (1..10 players, e.g. [{'AS','KS'}, {'QH','QD'}]),
+    table_cards: 0..5 card strings, dead_cards: cards removed from the deck (the reference's ghost cards).
+    Returns dict(equity = split-pot equity per player, win, tie = completions won alone / tied for best, completions).
+    Invalid or repeated cards raise ValueError, like get_equity."""
+    holes = [card_ids(h) for h in hands]
+    board, dead = card_ids(table_cards), card_ids(dead_cards)
+    if not 1 <= len(holes) <= 10:
+        raise ValueError("1..10 hands")
+    if any(len(h) != 2 for h in holes):
+        raise ValueError("every hand must hold exactly two cards")
+    if len(board) > 5:
+        raise ValueError("table_cards holds more than five cards")
+    if len(set(sum(holes, []) + board + dead)) != 2 * len(holes) + len(board) + len(dead):
+        raise ValueError("duplicate cards in hands / table_cards / dead_cards")
+    P = len(holes)
+    try:
+        out = showdown_equity_batch(np.array([holes], dtype=np.uint8), np.array([P], dtype=np.uint8),
+                                    np.array([board + [NO_CARD] * (5 - len(board))], dtype=np.uint8),
+                                    np.array([dead or [NO_CARD]], dtype=np.uint8), deal_mode=deal_mode, validate=True)
+    except _lib.NpkError as exc:
+        raise ValueError(str(exc)) from None
+    win, tie, share = (out[k][0].tolist() for k in ("win", "tie", "share"))
+    comp = int(out["completions"][0])
+    return {"equity": [x / (SHARE_UNIT * comp) for x in share], "win": win, "tie": tie, "completions": comp}
+
+
 def host_tables():
     """Host copies of the lookup tables built by libnpk (no GPU needed): dict of numpy arrays."""
     L = _lib.lib()

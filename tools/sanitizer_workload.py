@@ -108,6 +108,24 @@ for mode in ("reference", "uniform"):
                                       deal_mode=mode, known_opponents=kn, passes=mode == "reference"), 400, "known hands " + mode)
 print("ok known opponent hands", mc.equity, flush=True)
 
+# exact showdown equity of known hands: every player count and board size, dead cards, both dealers, garbage bytes
+se_h = np.full((40, 10, 2), 255, dtype=np.uint8); se_b = np.full((40, 5), 255, dtype=np.uint8)
+se_d = np.full((40, 2), 255, dtype=np.uint8); se_n = np.zeros(40, dtype=np.uint8)
+for i in range(40):
+    P, nb = 1 + i % 10, (3, 4, 5, 3)[i // 10]
+    c = rng.permutation(52)[:2 * P + nb + 2]
+    se_h[i, :P] = c[:2 * P].reshape(P, 2); se_b[i, :nb] = c[2 * P:2 * P + nb]; se_d[i] = c[2 * P + nb:]; se_n[i] = P
+for mode in ("uniform", "reference"):
+    o = npk.showdown_equity_batch(se_h, se_n, se_b, se_d, deal_mode=mode)
+    assert (o["share"].sum(dim=1) == 2520 * o["completions"]).all()
+npk.showdown_equity([["AS", "KS"], ["QH", "QD"], ["7C", "2D"]], ["2C"])
+npk.showdown_equity_batch(torch.randint(0, 256, (256, 10, 2), dtype=torch.uint8, device="cuda"),
+                          torch.randint(0, 256, (256,), dtype=torch.uint8, device="cuda"),
+                          torch.randint(0, 256, (256, 5), dtype=torch.uint8, device="cuda"),
+                          torch.randint(0, 256, (256, 3), dtype=torch.uint8, device="cuda"))
+torch.cuda.synchronize()
+print("ok showdown equity", flush=True)
+
 # vectorised HoldemTable: self-play with both dealers, observation vector, showdowns
 tb = HoldemTables(96, n_players=6, seed=3, autoplay=[1] * 6)
 tb.enable_observations()
