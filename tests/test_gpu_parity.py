@@ -239,23 +239,25 @@ def test_montecarlo_counts_equal_sampler_specification(torch_mod, mode):
 
 
 def test_every_kernel_instantiation_matches_specification(torch_mod):
-    """All 54 template instantiations of the uniform kernel (1..9 opponents x 0..5 known board cards) and the same
-    shapes through the reference-dealer kernel, each bit-exact against the specification.  (This is the test that caught
-    a ptxas miscompile of the last Fisher-Yates draw during bring-up.)"""
+    """All 60 template instantiations of the uniform kernel (0..9 opponents x 0..5 known board cards) and the same shapes
+    through the reference-dealer kernel, each launched on its own (uniform_shape) and bit-exact against the specification,
+    win types and passes included.  (This is the test that caught a ptxas miscompile of the last Fisher-Yates draw during
+    bring-up.)  The persistent mixed kernel runs the same shapes in test_montecarlo_counts_equal_sampler_specification and
+    test_mc_at_scale.py."""
     torch = torch_mod
     rng = np.random.default_rng(5)
-    hole, board, npl = [], [], []
-    for players in range(2, 11):
+    trials, seed = 40, 77
+    for players in range(1, 11):
         for known in range(6):
             c = rng.permutation(52)[:2 + known].tolist()
-            hole.append(c[:2]); board.append(pad_board(c[2:])); npl.append(players)
-    trials, seed = 40, 77
-    for mode in ("uniform", "reference"):
-        out = _run_batch(torch, hole, board, npl, trials, seed, mode)
-        for qi in range(len(hole)):
-            b = [c for c in board[qi] if c != NO]
-            m = sampler_model.run_model(oracle, mode, seed, qi, hole[qi], b, npl[qi], trials)
-            assert (int(out["wins"][qi]), int(out["ties"][qi])) == (m["wins"], m["ties"]), (mode, npl[qi], len(b))
+            for mode in ("uniform", "reference"):
+                out = _run_batch(torch, [c[:2]], [pad_board(c[2:])], [players], trials, seed, mode, uniform_shape=(players, known),
+                                 win_types=True, passes=(mode == "reference"))
+                m = sampler_model.run_model(oracle, mode, seed, 0, c[:2], c[2:], players, trials)
+                assert (int(out["wins"][0]), int(out["ties"][0])) == (m["wins"], m["ties"]), (mode, players, known)
+                assert out["win_types"][0].tolist() == m["win_types"], (mode, players, known)
+                if mode == "reference":
+                    assert int(out["passes"][0]) == m["passes"], (players, known)
 
 
 def test_partition_invariance(torch_mod):
