@@ -122,6 +122,38 @@ int npk_equity_batch_async(const uint8_t* hole, const uint8_t* board, const uint
 int npk_equity_batch_status(const void* workspace, void* stream, uint32_t* invalid, uint32_t* skipped);
 
 /*
+ * Monte-Carlo equity to a target PRECISION: every query runs until its standard error reaches `max_stderr`, checked at fixed
+ * checkpoints, or until max_trials.  The checkpoints are the same for every query of the call:
+ *     T_0 = min_trials,  T_{k+1} = min(2 T_k, max_trials),  up to max_trials       (1 <= min_trials <= max_trials)
+ * After checkpoint T_k a query still running stops when var <= max_stderr * max_stderr, computed in IEEE double in this order
+ * (every operation rounded to nearest, no fused multiply-add, so that a restatement in double arithmetic decides alike):
+ *     x = wins_strict + ties          (the reference's equity numerator: ties count as wins)
+ *     p = (x + 1) / (T_k + 2)         (add-one estimate: x = 0 or x = T_k does not give zero variance)
+ *     var = p * (1 - p) / T_k
+ * At max_trials every query stops.  The decision reads only the query's own counters, and trial t of query q is the same
+ * Philox stream as in npk_equity_batch (trial_offset 0), so the outputs of a query are EXACTLY the counters npk_equity_batch
+ * computes with trials = T_stop and the same seed and query_offset: they depend neither on the other queries of the batch nor
+ * on how it is split over calls or GPUs (query sharding through query_offset).
+ *   max_stderr  target standard error of the equity (wins_strict + ties) / trials; finite and > 0
+ *   shape_mask  as npk_equity_batch_async: queries of other shapes are left out
+ *   wins_strict, ties [Q], win_types [Q,9] or NULL, passes [Q] or NULL (REFERENCE mode): the counts of trials [0, T_stop)
+ *   trials      [Q] u64: T_stop of every query
+ * UNLIKE npk_equity_batch the call zeroes its outputs itself (the stopping rule reads them); invalid queries and queries outside
+ * shape_mask are left at 0 with trials = 0.  With NPK_FLAG_VALIDATE an invalid query is an error (NPK_ERR_INVALID_CARDS,
+ * reported after one small device->host read, before any trial runs).  Without it the call is asynchronous and free of host
+ * round trips (CUDA-graph capturable): it runs in rounds, one per checkpoint, launched back to back -- classification of the
+ * queries still active, the all-shapes kernel on trials [T_{k-1}, T_k), and a kernel that applies the rule, records trials of
+ * the queries it retires and plans the next round's work items from the number left.  NPK_ERR_INVALID_ARGUMENT for a
+ * max_stderr that is not finite or <= 0, min_trials < 1 or min_trials > max_trials is returned before the device is touched.
+ *   workspace   npk_equity_adaptive_workspace_bytes(Q) bytes of device memory, private to this call until it completes
+ */
+int64_t npk_equity_adaptive_workspace_bytes(int64_t Q);
+int npk_equity_batch_adaptive(const uint8_t* hole, const uint8_t* board, const uint8_t* n_players, int64_t Q,
+                              int64_t min_trials, int64_t max_trials, double max_stderr, uint64_t shape_mask, uint64_t seed,
+                              int64_t query_offset, int deal_mode, uint32_t flags, uint64_t* wins_strict, uint64_t* ties,
+                              uint64_t* win_types, uint64_t* passes, uint64_t* trials, void* workspace, void* stream);
+
+/*
  * Trial-sharded jobs (SURVEY 8e: one query spans several GPUs, e.g. 169 classes x 1,000,000 trials over 8 GPUs): the
  * count reduction is done by the Monte-Carlo kernel itself over NVLink-mapped peer memory; no NCCL call, no memset and no
  * pack kernel on the step path.  One process per GPU; the processes exchange 64-byte CUDA IPC handles once (any transport:

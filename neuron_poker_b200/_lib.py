@@ -49,6 +49,11 @@ def lib():
                 L.npk_equity_batch_async.argtypes = [u8, u8, u8, i64, i64, ctypes.c_uint64, ctypes.c_uint64, i64, i64, i32,
                                                      u64, u64, u64, u64, vp, vp]
                 L.npk_equity_batch_status.argtypes = [vp, vp, ctypes.POINTER(ctypes.c_uint32), ctypes.POINTER(ctypes.c_uint32)]
+                L.npk_equity_adaptive_workspace_bytes.argtypes = [i64]
+                L.npk_equity_adaptive_workspace_bytes.restype = i64
+                L.npk_equity_batch_adaptive.argtypes = [u8, u8, u8, i64, i64, i64, ctypes.c_double, ctypes.c_uint64,
+                                                        ctypes.c_uint64, i64, i32, ctypes.c_uint32, u64, u64, u64, u64, u64,
+                                                        vp, vp]
                 L.npk_equity_host.argtypes = [u8, u8, u8, i64, i64, ctypes.c_uint64, i32, u64, u64, u64, u64]
                 L.npk_equity_host_submit.argtypes = [u8, u8, u8, i64, i64, ctypes.c_uint64, i32, ctypes.c_uint32]
                 L.npk_equity_host_submit.restype = i64

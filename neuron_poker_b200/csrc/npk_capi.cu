@@ -1,6 +1,7 @@
 // npk_capi.cu -- the C ABI declared in include/npk.h: table upload, query classification, kernel launches.
 #include <cuda_runtime.h>
 
+#include <cmath>
 #include <cstdio>
 #include <cstring>
 #include <atomic>
@@ -187,8 +188,10 @@ __device__ __forceinline__ int classify_query(const uint8_t* hole, const uint8_t
 // Count the queries of every shape -- per block in shared memory, then one global atomic per shape and block (65,536
 // self-play queries fall into a dozen shapes: per-query global atomics on a dozen addresses took 35 us) -- and let the last
 // block to finish drop the shapes outside `shape_mask` and write the exclusive prefix of the counts behind them.
+// `active` [Q] or null: queries with active[q] == 0 (retired by an adaptive call) are left out altogether.
 __global__ void __launch_bounds__(256) classify_count_kernel(const uint8_t* hole, const uint8_t* board, const uint8_t* n_players,
-                                                             long long Q, uint8_t* ws, unsigned long long shape_mask)
+                                                             long long Q, uint8_t* ws, unsigned long long shape_mask,
+                                                             const uint8_t* active)
 {
     __shared__ uint32_t s_cnt[65];                         // [64] = invalid
     __shared__ bool last;
@@ -196,6 +199,7 @@ __global__ void __launch_bounds__(256) classify_count_kernel(const uint8_t* hole
     if (threadIdx.x < 65) s_cnt[threadIdx.x] = 0;
     __syncthreads();
     for (long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x; q < Q; q += (long long)gridDim.x * blockDim.x) {
+        if (active && !active[q]) continue;
         const int g = classify_query(hole, board, n_players, q);
         atomicAdd(&s_cnt[g < 0 ? 64 : g], 1u);
     }
@@ -223,7 +227,7 @@ __global__ void __launch_bounds__(256) classify_count_kernel(const uint8_t* hole
 // Sort the query numbers by shape: a block counts its own queries per shape, reserves one range per shape in qindex with a
 // single global atomic, and its threads take slots inside the range from shared-memory cursors.
 __global__ void __launch_bounds__(256) classify_fill_kernel(const uint8_t* hole, const uint8_t* board, const uint8_t* n_players,
-                                                            long long Q, uint8_t* ws)
+                                                            long long Q, uint8_t* ws, const uint8_t* active)
 {
     __shared__ uint32_t s_cnt[64], s_base[64];
     uint32_t* cursors = reinterpret_cast<uint32_t*>(ws + kWsCursors);
@@ -244,7 +248,7 @@ __global__ void __launch_bounds__(256) classify_fill_kernel(const uint8_t* hole,
         for (int k = 0; k < kPerThread; k++) {
             const long long q = base + (long long)k * blockDim.x + threadIdx.x;
             g[k] = -1;
-            if (q < q1) {
+            if (q < q1 && (!active || active[q])) {
                 g[k] = classify_query(hole, board, n_players, q);
                 if (g[k] >= 0 && counts[g[k]] == 0) g[k] = -1;          // a shape outside the caller's mask
                 if (g[k] >= 0) slot[k] = atomicAdd(&s_cnt[g[k]], 1u);
@@ -261,24 +265,103 @@ __global__ void __launch_bounds__(256) classify_fill_kernel(const uint8_t* hole,
     }
 }
 
-// Work items of a launch: (query, chunk of trials).  Items hold up to 2,048 trials (64 per lane: the per-item set-up --
-// query load, deck initialisation, reduction -- is then a few per cent of the work) but at least eight per warp; small jobs
-// are cut finer so that a single query still spreads over the whole chip (a lone get_equity call of 10,000 trials becomes 157
-// one-iteration items).  A finer-grained tail (the last eighth of every query in items an eighth of the size, handed out
-// last) was measured in round 2 and lost 1.5 % on cfg3: the warps left over in the last round of items run faster, because
-// the SM is throughput-bound, so the tail costs about 1 %, less than the extra item set-ups.
-// Returns the number of items per query.
+// ---- adaptive calls (npk_equity_batch_adaptive) -----------------------------------------------------------------------
+// Workspace: the header and qindex of npk_equity_workspace_bytes(Q) (reused by every round), then at adaptive_base(Q) a
+// 64-byte block of u32 words -- queries still active (a running sum), blocks done, invalid queries, the next round's
+// {chunk, chunks} -- and active [Q] bytes.  The running sum and the block count are reset by the block that consumes them.
+constexpr int kAdActive = 0, kAdBlocksDone = 1, kAdInvalid = 2, kAdPlan = 4, kAdHeaderBytes = 64;
+int64_t adaptive_base(int64_t Q) { return (npk_equity_workspace_bytes(Q) + 255) & ~int64_t(255); }
+
+// The stopping rule after checkpoint t: x = wins + ties, p = (x + 1) / (t + 2), var = p (1 - p) / t, stop if var <= bound
+// (= stderr * stderr).  IEEE double, rounded to nearest at every step and never contracted into an FMA, so that a host restatement
+// in double arithmetic takes the same decision at the boundary.
+__device__ __forceinline__ bool adaptive_stop(unsigned long long x, long long t, double bound)
+{
+    const double p = __ddiv_rn(__dadd_rn(__ull2double_rn(x), 1.0), __ll2double_rn(t + 2));
+    const double var = __ddiv_rn(__dmul_rn(p, __dsub_rn(1.0, p)), __ll2double_rn(t));
+    return var <= bound;
+}
+
+// Block sums of the queries still active (and of invalid ones) go to the workspace; the last block to finish plans the next
+// round's work items from the total and resets the sum for the next round.
+__device__ void adaptive_count(uint32_t n_active, uint32_t n_invalid, uint32_t* hdr, long long next_trials, int sm_count)
+{
+    __shared__ uint32_t s_n[2];
+    if (threadIdx.x == 0) { s_n[0] = 0; s_n[1] = 0; }
+    __syncthreads();
+    if (n_active) atomicAdd(&s_n[0], n_active);
+    if (n_invalid) atomicAdd(&s_n[1], n_invalid);
+    __syncthreads();
+    if (threadIdx.x != 0) return;
+    if (s_n[0]) atomicAdd(&hdr[kAdActive], s_n[0]);
+    if (s_n[1]) atomicAdd(&hdr[kAdInvalid], s_n[1]);
+    __threadfence();
+    if (atomicAdd(&hdr[kAdBlocksDone], 1u) != gridDim.x - 1) return;
+    __threadfence();
+    const uint32_t total = *reinterpret_cast<volatile uint32_t*>(&hdr[kAdActive]);
+    uint32_t chunk, chunks;
+    npk::item_plan(total, next_trials, sm_count, 64, chunk, chunks);
+    hdr[kAdPlan] = chunk; hdr[kAdPlan + 1] = chunks;
+    hdr[kAdActive] = 0; hdr[kAdBlocksDone] = 0;
+}
+
+// Zero the outputs (the stopping rule reads the counters, so the call owns them) and mark the valid queries of the caller's
+// shapes active; plan the first round.
+__global__ void __launch_bounds__(256) adaptive_init_kernel(const uint8_t* hole, const uint8_t* board, const uint8_t* n_players,
+                                                            long long Q, unsigned long long shape_mask,
+                                                            unsigned long long* wins, unsigned long long* ties,
+                                                            unsigned long long* win_types, unsigned long long* passes,
+                                                            unsigned long long* trials, uint8_t* active, uint32_t* hdr,
+                                                            long long first_trials, int sm_count)
+{
+    uint32_t n = 0, bad = 0;
+    for (long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x; q < Q; q += (long long)gridDim.x * blockDim.x) {
+        wins[q] = 0; ties[q] = 0; trials[q] = 0;
+        if (win_types)
+            for (int i = 0; i < 9; i++) win_types[9 * q + i] = 0;
+        if (passes) passes[q] = 0;
+        const int g = classify_query(hole, board, n_players, q);
+        const bool a = g >= 0 && (shape_mask >> g & 1ull);
+        active[q] = a ? 1 : 0;
+        n += a;
+        bad += g < 0;
+    }
+    adaptive_count(n, bad, hdr, first_trials, sm_count);
+}
+
+// After the round that ends at checkpoint t: retire every active query the rule stops (all of them in the final round),
+// recording trials = t, and plan the next round of `next_trials` trials for the queries left.  Grid: one thread per query.
+__global__ void __launch_bounds__(256) adaptive_retire_kernel(long long Q, const unsigned long long* wins,
+                                                              const unsigned long long* ties, unsigned long long* trials,
+                                                              uint8_t* active, uint32_t* hdr, long long t, double max_stderr,
+                                                              int final_round, long long next_trials, int sm_count)
+{
+    const double bound = __dmul_rn(max_stderr, max_stderr);
+    uint32_t n = 0;
+    const long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x;   // one query per thread: a grid-stride loop kept
+    if (q < Q && active[q]) {                                               // enough values live across the division's slow
+        if (final_round || adaptive_stop(wins[q] + ties[q], t, bound)) {    // path to spill
+            active[q] = 0;
+            trials[q] = (unsigned long long)t;
+        } else {
+            n = 1;
+        }
+    }
+    adaptive_count(n, 0, hdr, next_trials, sm_count);
+}
+
+// T_0 = min_trials, T_{k+1} = min(2 T_k, max_trials), up to max_trials.
+std::vector<long long> adaptive_checkpoints(long long min_trials, long long max_trials)
+{
+    std::vector<long long> t{min_trials};
+    while (t.back() < max_trials) t.push_back(t.back() > max_trials / 2 ? max_trials : 2 * t.back());
+    return t;
+}
+
+// Work items of a launch (npk::item_plan).  Returns the number of items per query.
 long long plan_items(npk::EquityParams& p, long long queries, long long trials, int sm_count, int lanes_worth = 64)
 {
-    const long long warps = (long long)sm_count * 16;
-    long long c = (queries * trials) / (8 * warps);
-    c = (c + lanes_worth - 1) / lanes_worth * lanes_worth;      // a warp iteration covers 64 trials (a pair per lane)
-    if (c < lanes_worth) c = lanes_worth;
-    if (c > 2048) c = 2048;
-    if (trials <= 0) { p.chunk = 1; p.chunks = 0; return 0; }
-    if (trials <= c) { p.chunk = (uint32_t)trials; p.chunks = 1; return 1; }
-    p.chunk = (uint32_t)c;
-    p.chunks = (uint32_t)((trials + c - 1) / c);
+    npk::item_plan(queries, trials, sm_count, lanes_worth, p.chunk, p.chunks);
     return p.chunks;
 }
 
@@ -477,12 +560,13 @@ int64_t npk_equity_workspace_bytes(int64_t Q) { return kWsIndex + 4 * (Q > 0 ? Q
 namespace {
 // Mixed batch: classify on the device (two small kernels), then ONE persistent kernel for all shapes (npk_mixed.cu).
 // Nothing is read back: asynchronous on `s`.
+// `active` [Q] or null: an adaptive call's round, which runs only the queries still active.
 int enqueue_mixed(DeviceState* ds, npk::EquityParams& p, const uint8_t* hole, const uint8_t* board, const uint8_t* n_players,
-                  int64_t Q, uint64_t shape_mask, uint8_t* ws, cudaStream_t s)
+                  int64_t Q, uint64_t shape_mask, uint8_t* ws, cudaStream_t s, const uint8_t* active = nullptr)
 {
     const int cg = (int)std::min<long long>((Q + 255) / 256, 4 * ds->sm_count);
-    classify_count_kernel<<<cg, 256, 0, s>>>(hole, board, n_players, Q, ws, shape_mask);
-    classify_fill_kernel<<<cg, 256, 0, s>>>(hole, board, n_players, Q, ws);
+    classify_count_kernel<<<cg, 256, 0, s>>>(hole, board, n_players, Q, ws, shape_mask, active);
+    classify_fill_kernel<<<cg, 256, 0, s>>>(hole, board, n_players, Q, ws, active);
     p.group = reinterpret_cast<const uint32_t*>(ws + kWsCounts);
     p.qindex = reinterpret_cast<const int32_t*>(ws + kWsIndex);
     p.nq = 0;
@@ -525,7 +609,7 @@ int npk_equity_batch(const uint8_t* hole, const uint8_t* board, const uint8_t* n
     if (uniform_shape) {
         // validated: classify first (one small device->host read), then the shape's own kernel
         const int cg = (int)std::min<long long>((Q + 255) / 256, 4 * ds->sm_count);
-        classify_count_kernel<<<cg, 256, 0, s>>>(hole, board, n_players, Q, ws, ~0ull);
+        classify_count_kernel<<<cg, 256, 0, s>>>(hole, board, n_players, Q, ws, ~0ull, nullptr);
         uint32_t host[64 + 64 + 1];
         e = cudaMemcpyAsync(host, ws + kWsCounts, 4 * 129, cudaMemcpyDeviceToHost, s);
         if (e == cudaSuccess) e = cudaStreamSynchronize(s);
@@ -588,6 +672,74 @@ int npk_equity_batch_status(const void* workspace, void* stream, uint32_t* inval
     if (e != cudaSuccess) return cuda_fail(e, "npk_equity_batch_status");
     if (invalid) *invalid = v[0];
     if (skipped) *skipped = v[1];
+    return NPK_OK;
+}
+
+int64_t npk_equity_adaptive_workspace_bytes(int64_t Q) { return adaptive_base(Q) + kAdHeaderBytes + (Q > 0 ? Q : 0); }
+
+int npk_equity_batch_adaptive(const uint8_t* hole, const uint8_t* board, const uint8_t* n_players, int64_t Q,
+                              int64_t min_trials, int64_t max_trials, double max_stderr, uint64_t shape_mask, uint64_t seed,
+                              int64_t query_offset, int deal_mode, uint32_t flags, uint64_t* wins_strict, uint64_t* ties,
+                              uint64_t* win_types, uint64_t* passes, uint64_t* trials, void* workspace, void* stream)
+{
+    // the arguments of the rule first: these errors need no device
+    if (!std::isfinite(max_stderr) || max_stderr <= 0.0)
+        return fail(NPK_ERR_INVALID_ARGUMENT, "stderr must be a finite number > 0");
+    if (min_trials < 1) return fail(NPK_ERR_INVALID_ARGUMENT, "min_trials must be >= 1");
+    if (min_trials > max_trials) return fail(NPK_ERR_INVALID_ARGUMENT, "min_trials must not exceed max_trials");
+    DeviceState* ds;
+    int rc = batch_start(&ds, Q, max_trials, 0);
+    if (rc) return rc == kEmptyBatch ? NPK_OK : rc;
+    if (!hole || !board || !n_players || !wins_strict || !ties || !trials || !workspace)
+        return fail(NPK_ERR_INVALID_ARGUMENT, "null pointer");
+    if ((rc = check_deal_mode(deal_mode))) return rc;
+    shape_mask &= (1ull << kGroups) - 1ull;
+    if (!shape_mask) return fail(NPK_ERR_INVALID_ARGUMENT, "empty shape mask");
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    uint8_t* ws = static_cast<uint8_t*>(workspace);
+    uint32_t* hdr = reinterpret_cast<uint32_t*>(ws + adaptive_base(Q));
+    uint8_t* active = ws + adaptive_base(Q) + kAdHeaderBytes;
+    auto* w = reinterpret_cast<unsigned long long*>(wins_strict);
+    auto* t = reinterpret_cast<unsigned long long*>(ties);
+    auto* n_trials = reinterpret_cast<unsigned long long*>(trials);
+    const std::vector<long long> cp = adaptive_checkpoints(min_trials, max_trials);
+    const int cg = (int)std::min<long long>((Q + 255) / 256, 4 * ds->sm_count);
+    const unsigned int retire_grid = (unsigned int)((Q + 255) / 256);
+
+    cudaError_t e = cudaMemsetAsync(hdr, 0, kAdHeaderBytes, s);
+    if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(workspace)");
+    adaptive_init_kernel<<<cg, 256, 0, s>>>(hole, board, n_players, Q, shape_mask, w, t,
+                                            reinterpret_cast<unsigned long long*>(win_types),
+                                            reinterpret_cast<unsigned long long*>(passes), n_trials, active, hdr, cp[0],
+                                            ds->sm_count);
+    if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "adaptive_init_kernel launch");
+    if (flags & NPK_FLAG_VALIDATE) {
+        uint32_t bad = 0;
+        e = cudaMemcpyAsync(&bad, hdr + kAdInvalid, 4, cudaMemcpyDeviceToHost, s);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+        if (e != cudaSuccess) return cuda_fail(e, "adaptive batch");
+        if (bad) return fail(NPK_ERR_INVALID_CARDS, std::to_string(bad) + " invalid quer" + (bad == 1 ? "y" : "ies") +
+                             " (card id >= 52, duplicate cards, gap in the board, or players outside 1..10); nothing has "
+                             "been computed");
+    }
+
+    // one round per checkpoint, back to back on the stream: the trials [T_{k-1}, T_k) of the queries still active, then the rule
+    npk::EquityParams p;
+    fill_params(p, *ds, hole, board, n_players, Q, cp[0], 0, query_offset, seed, deal_mode, wins_strict, ties, win_types,
+                passes, reinterpret_cast<uint32_t*>(ws + kWsAbort));
+    p.plan = hdr + kAdPlan;
+    long long done = 0;
+    for (size_t k = 0; k < cp.size(); k++) {
+        if ((rc = clear_workspace(ws, s))) return rc;
+        p.trials = cp[k] - done;
+        p.trial_offset = done;
+        if ((rc = enqueue_mixed(ds, p, hole, board, n_players, Q, ~0ull, ws, s, active))) return rc;
+        const bool final_round = k + 1 == cp.size();
+        adaptive_retire_kernel<<<retire_grid, 256, 0, s>>>(Q, w, t, n_trials, active, hdr, cp[k], max_stderr, final_round ? 1 : 0,
+                                                         final_round ? 0 : cp[k + 1] - cp[k], ds->sm_count);
+        if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "adaptive_retire_kernel launch");
+        done = cp[k];
+    }
     return NPK_OK;
 }
 

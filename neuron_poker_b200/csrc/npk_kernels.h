@@ -111,7 +111,32 @@ struct EquityParams {
                                   // player_card_list, montecarlo_python.py:132-163), or null
     uint32_t n_known;             // how many of the n_players - 1 opponents those are
     uint32_t* abort_flag;         // raised when one draw needs more than kMaxRangeAttempts attempts
+    // ---- adaptive calls (npk_equity_batch_adaptive): {chunk, chunks} of this round, written on the device by the kernel
+    // that retired the previous round's queries; the all-shapes kernel reads them instead of chunk / chunks when non-null
+    const uint32_t* plan;
 };
+
+// Work items of a Monte-Carlo launch: (query, chunk of trials).  Items hold up to 2,048 trials (64 per lane: the per-item
+// set-up -- query load, deck initialisation, reduction -- is then a few per cent of the work) but at least eight per warp;
+// small jobs are cut finer so that a single query still spreads over the whole chip (a lone get_equity call of 10,000 trials
+// becomes 157 one-iteration items).  A finer-grained tail (the last eighth of every query in items an eighth of the size,
+// handed out last) was measured in round 2 and lost 1.5 % on cfg3: the warps left over in the last round of items run faster,
+// because the SM is throughput-bound, so the tail costs about 1 %, less than the extra item set-ups.
+// The host plans a launch from its query count; an adaptive call's later rounds are planned on the device from the number of
+// queries still running.  The plan changes no result: a trial's outcome depends only on (seed, query, trial number).
+__host__ __device__ inline void item_plan(long long queries, long long trials, int sm_count, int lanes_worth, uint32_t& chunk,
+                                          uint32_t& chunks)
+{
+    const long long warps = (long long)sm_count * 16;
+    long long c = (queries * trials) / (8 * warps);
+    c = (c + lanes_worth - 1) / lanes_worth * lanes_worth;      // a warp iteration covers 64 trials (a pair per lane)
+    if (c < lanes_worth) c = lanes_worth;
+    if (c > 2048) c = 2048;
+    if (trials <= 0) { chunk = 1; chunks = 0; return; }
+    if (trials <= c) { chunk = (uint32_t)trials; chunks = 1; return; }
+    chunk = (uint32_t)c;
+    chunks = (uint32_t)((trials + c - 1) / c);
+}
 
 constexpr uint32_t kMaxRangeAttempts = 1u << 16;
 

@@ -44,7 +44,8 @@ __device__ __forceinline__ void dispatch_known(int known, const EquityParams* p,
     }
 }
 
-template <int REF>
+// PLAN = 1: the rounds of an adaptive call, whose work items are planned on the device (p.plan = {chunk, chunks}).
+template <int REF, int PLAN>
 __global__ void __launch_bounds__(kMixedThreads, 1) equity_mixed_kernel(const EquityParams p)
 {
     extern __shared__ __align__(128) uint8_t smem[];
@@ -52,7 +53,8 @@ __global__ void __launch_bounds__(kMixedThreads, 1) equity_mixed_kernel(const Eq
     const WarpCtx cx = warp_context(p, smem, 64 + 50 * 32);  // decks sized for the largest shape (preflop: 50 unseen cards)
     const int lane = cx.lane;
     const uint32_t* counts = p.group;                        // [64] queries per group, [64..128) first qindex slot per group
-    const long long per_query = p.chunks;
+    const uint32_t plan_chunk = PLAN ? p.plan[0] : 0u, plan_chunks = PLAN ? p.plan[1] : 0u;
+    const long long per_query = PLAN ? (long long)plan_chunks : (long long)p.chunks;
     if (threadIdx.x == 0) {
         long long acc = 0;
         for (int g = 0; g < kShapeGroups; g++) { s_first[g] = acc; acc += (long long)counts[g] * per_query; }
@@ -67,7 +69,14 @@ __global__ void __launch_bounds__(kMixedThreads, 1) equity_mixed_kernel(const Eq
         if (lane + 32 < kShapeGroups) before += item >= s_first[lane + 33];
         const int g = (int)__reduce_add_sync(0xffffffffu, before);
         long long qslot, t_begin, t_end;
-        item_range(p, item - s_first[g], qslot, t_begin, t_end);
+        if (PLAN) {
+            const long long rel = item - s_first[g];
+            qslot = rel / plan_chunks;
+            t_begin = (rel - qslot * plan_chunks) * plan_chunk;
+            t_end = min(p.trials, t_begin + (long long)plan_chunk);
+        } else {
+            item_range(p, item - s_first[g], qslot, t_begin, t_end);
+        }
         const long long q = p.qindex[counts[64 + g] + qslot];
         const int known = g % 6;
         switch (g / 6) {
@@ -278,7 +287,8 @@ cudaError_t launch_equity_oneshot(const DeviceTables& t, ResidentState* st, Resi
 
 cudaError_t launch_equity_mixed(const EquityParams& p, int sm_count, cudaStream_t s)
 {
-    auto k = p.reference_dealer ? equity_mixed_kernel<1> : equity_mixed_kernel<0>;
+    auto k = p.plan ? (p.reference_dealer ? equity_mixed_kernel<1, 1> : equity_mixed_kernel<0, 1>)
+                    : (p.reference_dealer ? equity_mixed_kernel<1, 0> : equity_mixed_kernel<0, 0>);
     const size_t fixed = 128 + (size_t)p.tables.value_bytes + p.tables.rowoff_bytes + p.tables.flush_bytes + kDescBytes;
     const size_t smem = fixed + (size_t)(kMixedThreads / 32) * (64 + 50 * 32) * 4;
     cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);

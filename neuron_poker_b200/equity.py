@@ -486,3 +486,60 @@ def get_equity_batch(hole, board, n_players, trials, seed_value=0, deal_mode="un
         ws.record_stream(torch.cuda.current_stream(dev))
     out["trials"] = int(trials)
     return out
+
+
+ALL_SHAPES = (1 << 60) - 1
+
+
+def adaptive_checkpoints(min_trials, max_trials):
+    """Checkpoints of get_equity_batch_adaptive: T_0 = min_trials, T_{k+1} = min(2 T_k, max_trials), up to max_trials."""
+    min_trials, max_trials = int(min_trials), int(max_trials)
+    if not 1 <= min_trials <= max_trials:
+        raise ValueError("need 1 <= min_trials <= max_trials, got %d, %d" % (min_trials, max_trials))
+    t = [min_trials]
+    while t[-1] < max_trials:
+        t.append(min(2 * t[-1], max_trials))
+    return t
+
+
+def adaptive_stops(wins_plus_ties, trials, stderr):
+    """The stopping rule of get_equity_batch_adaptive after checkpoint `trials`, in the device's order of double operations:
+    p = (x + 1) / (T + 2), var = p (1 - p) / T, stop when var <= stderr * stderr."""
+    p = (float(wins_plus_ties) + 1.0) / float(trials + 2)
+    return p * (1.0 - p) / float(trials) <= stderr * stderr
+
+
+def get_equity_batch_adaptive(hole, board, n_players, max_trials, stderr, min_trials=256, seed_value=0, deal_mode="uniform",
+                              query_offset=0, shapes=None, device=None, validate=True, win_types=False, passes=False):
+    """Monte-Carlo counts to a target precision (npk_equity_batch_adaptive, asynchronous on the current torch stream unless
+    validate=True): every query runs until the standard error of its equity (wins + ties) / trials is at most `stderr`,
+    checked at the checkpoints adaptive_checkpoints(min_trials, max_trials), or until max_trials.  The counters of a query
+    are exactly those of get_equity_batch(trials=T_stop) with the same seed and query_offset, whatever else is in the batch.
+    Returns the dict of get_equity_batch, except that `trials` is an int64 CUDA tensor [Q] holding every query's T_stop
+    (0 for a query outside `shapes`, or an invalid one when validate=False)."""
+    import torch
+    dev = _resolve_device(device)
+    hole = _as_cuda_u8(hole, dev, (2,))
+    board = _as_cuda_u8(board, dev, (5,))
+    n_players = _as_cuda_u8(n_players, dev, ())
+    Q = hole.shape[0]
+    L = _lib.ensure_init(dev.index)
+    with torch.cuda.device(dev):
+        out = {}
+        for name, shape, want in (("wins", (Q,), True), ("ties", (Q,), True), ("win_types", (Q, 9), win_types),
+                                  ("passes", (Q,), passes), ("trials", (Q,), True)):
+            if want:
+                out[name] = (torch.empty if Q else torch.zeros)(shape, dtype=torch.int64, device=dev)   # zeroed by the call
+        ws = torch.empty(int(L.npk_equity_adaptive_workspace_bytes(Q)), dtype=torch.uint8, device=dev)
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        _lib.check(L.npk_equity_batch_adaptive(hole.data_ptr(), board.data_ptr(), n_players.data_ptr(), Q, int(min_trials),
+                                               int(max_trials), ctypes.c_double(float(stderr)),
+                                               ctypes.c_uint64(ALL_SHAPES if shapes is None else int(shapes) & ALL_SHAPES),
+                                               ctypes.c_uint64(int(seed_value) & (2**64 - 1)), int(query_offset),
+                                               _DEAL[deal_mode], _lib.NPK_FLAG_VALIDATE if validate else 0,
+                                               out["wins"].data_ptr(), out["ties"].data_ptr(),
+                                               out["win_types"].data_ptr() if win_types else None,
+                                               out["passes"].data_ptr() if passes else None, out["trials"].data_ptr(),
+                                               ws.data_ptr(), stream))
+        ws.record_stream(torch.cuda.current_stream(dev))
+    return out

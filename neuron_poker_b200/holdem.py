@@ -209,15 +209,25 @@ class HoldemTables(object):
     # holdem_step (+ one memset of the workspace header and one torch zero_ of the [2,N] counters)
     launches_per_step = 6
 
-    def selfplay_step(self, agents, runs=1000, deal_mode="reference", restart_finished=True, sync_free=True):
+    def selfplay_step(self, agents, runs=1000, deal_mode="reference", restart_finished=True, sync_free=True, stderr=None):
         """One action on every table, entirely on the device: the equity query of every current player
         (env.py:262-264: 1,000 runs, all players alive), the Monte-Carlo kernel, the agents' decisions
         (agent_consider_equity / random) and the state machine.  Returns the actions taken (int8 CUDA tensor).
         The queries of a step mix player counts and streets: they are sorted by shape on the device and ONE persistent
         kernel handles all shapes (csrc/npk_mixed.cu); nothing is read back, so the step can be captured in a CUDA graph.
+        stderr: None runs `runs` trials for every query.  A number asks every equity to that standard error instead
+        (get_equity_batch_adaptive with max_trials = runs): a query stops at the first checkpoint that reaches it, and the
+        agents decide on equity = (wins + ties) / trials.
         (`sync_free` is accepted for compatibility: every mixed batch is free of host round trips now.)"""
-        from .equity import get_equity_batch
+        from .equity import get_equity_batch, get_equity_batch_adaptive
         hole, board, npl, _ = self.queries()
+        if stderr is not None:
+            out = get_equity_batch_adaptive(hole, board, npl, runs, stderr, min_trials=min(256, runs),
+                                            seed_value=(self.seed << 20) + self.decisions, deal_mode=deal_mode,
+                                            query_offset=self.table_offset, validate=False, device=self.device)
+            actions = self.decide(agents, equity=self.adaptive_equity(out))
+            self.step(actions, restart_finished=restart_finished)
+            return actions
         out = getattr(self, "_mc_out", None)
         if out is None:
             both = self.torch.zeros((2, self.n_tables), dtype=self.torch.int64, device=self.device)
@@ -229,6 +239,11 @@ class HoldemTables(object):
         actions = self.decide(agents, wins=out["wins"], ties=out["ties"], runs=runs)
         self.step(actions, restart_finished=restart_finished)
         return actions
+
+    @staticmethod
+    def adaptive_equity(out):
+        """(wins + ties) / trials of get_equity_batch_adaptive's counters, float64; 0 for a query that ran no trial."""
+        return (out["wins"] + out["ties"]).double() / out["trials"].clamp(min=1).double()
 
     # ---- observations ----
     def enable_observations(self):

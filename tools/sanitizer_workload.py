@@ -71,6 +71,13 @@ for mode in ("uniform", "reference"):
     check(npk.get_equity_batch(ho, bo, pl, 300, seed_value=4, deal_mode=mode), 300, mode + " mixed")
     check(npk.get_equity_batch(ho, bo, pl, 300, seed_value=4, deal_mode=mode,
                                shapes=npk.equity.shape_mask(range(2, 7))), 300, mode + " mixed sync-free")
+    # to a target precision: rounds of the all-shapes kernel on the queries still active, retired on the device
+    ad = npk.get_equity_batch_adaptive(ho, bo, pl, 700, 0.03, min_trials=64, seed_value=4, deal_mode=mode, win_types=True,
+                                       passes=mode == "reference")
+    torch.cuda.synchronize()
+    tr = ad["trials"].cpu().numpy()
+    assert ((tr >= 64) & (tr <= 700)).all() and ((ad["wins"] + ad["ties"]).cpu().numpy() <= tr).all(), mode + " adaptive"
+    print("ok", mode, "adaptive", flush=True)
     # host-buffer entry point: one-query fast path and the staged path
     for _ in range(3):
         c = npk.equity_counts({"AS", "KS"}, {"2C", "7D", "KH"}, 6, 1000, deal_mode=mode, win_types=True, passes=True)
@@ -131,7 +138,7 @@ tb = HoldemTables(96, n_players=6, seed=3, autoplay=[1] * 6)
 tb.enable_observations()
 agents = EquityAgents.equity_vs_random()
 for i in range(6 if QUICK else 25):
-    tb.selfplay_step(agents, runs=64, deal_mode="reference" if i & 1 else "uniform")
+    tb.selfplay_step(agents, runs=64, deal_mode="reference" if i & 1 else "uniform", stderr=0.05 if i % 3 == 2 else None)
     tb.observe()
 torch.cuda.synchronize()
 st = tb.state()
