@@ -263,6 +263,28 @@ int npk_equity_ranges_known_batch(const uint8_t* hole, const uint8_t* board, con
                                   int64_t trial_offset, int64_t query_offset, int deal_mode, uint32_t flags,
                                   uint64_t* wins_strict, uint64_t* ties, uint64_t* win_types, uint64_t* passes,
                                   void* workspace, void* stream);
+/*
+ * Monte-Carlo equity with ranges to a target PRECISION: npk_equity_batch_adaptive's contract (checkpoints T_0 = min_trials,
+ * doubling, capped at max_trials; a query stops after checkpoint T_k when var <= max_stderr^2 with p = (wins_strict + ties +
+ * 1) / (T_k + 2), var = p (1 - p) / T_k in round-to-nearest double without FMA; trials [Q] out) applied to
+ * npk_equity_ranges_known_batch.  Arguments as there, minus trials and trial_offset: the counters of a query are EXACTLY those
+ * npk_equity_ranges_known_batch computes with trials = T_stop, trial_offset = 0 and the same seed, query_offset, ranges,
+ * ghost cards, known hands and sampler (the generic kernel when passes is given, the pair-list sampler when it is NULL).
+ * The call zeroes its outputs; an invalid query is left at 0 with trials = 0, or with NPK_FLAG_VALIDATE is an error
+ * (NPK_ERR_INVALID_CARDS) reported after one small device->host read, before any trial runs.  Each round runs the range
+ * kernel on trials [T_{k-1}, T_k) of the queries still active, then a kernel that applies the rule, lists the queries left
+ * and plans the next round's work items on the device.  A draw that needs more than 65,536 attempts stops that round and
+ * every later one; with NPK_FLAG_VALIDATE it is reported as NPK_ERR_RANGE after the last round.  Without the flag the call is
+ * asynchronous and free of host round trips (CUDA-graph capturable).  The rule's argument errors (NPK_ERR_INVALID_ARGUMENT)
+ * are returned before the device is touched; the other argument errors are those of npk_equity_ranges_known_batch.
+ *   workspace   npk_equity_adaptive_workspace_bytes(Q) bytes of device memory, private to this call until it completes
+ */
+int npk_equity_ranges_batch_adaptive(const uint8_t* hole, const uint8_t* board, const uint8_t* n_players, const uint8_t* ghost,
+                                     const uint8_t* known_opp, int n_known, int64_t Q, int64_t min_trials, int64_t max_trials,
+                                     double max_stderr, const uint64_t* opp_allowed, const uint64_t* hero_allowed,
+                                     uint64_t seed, int64_t query_offset, int deal_mode, uint32_t flags,
+                                     uint64_t* wins_strict, uint64_t* ties, uint64_t* win_types, uint64_t* passes,
+                                     uint64_t* trials, void* workspace, void* stream);
 int npk_equity_ranges_known_host(const uint8_t* hole, const uint8_t* board, const uint8_t* n_players, const uint8_t* ghost,
                                  const uint8_t* known_opp, int n_known, int64_t Q, int64_t trials, const uint64_t* opp_allowed,
                                  const uint64_t* hero_allowed, uint64_t seed, int deal_mode, uint64_t* wins_strict,

@@ -66,6 +66,9 @@ def lib():
                                                      u64, u64]
                 L.npk_equity_ranges_known_batch.argtypes = [u8, u8, u8, u8, u8, i32, i64, i64, u64, u64, ctypes.c_uint64, i64, i64,
                                                             i32, ctypes.c_uint32, u64, u64, u64, u64, vp, vp]
+                L.npk_equity_ranges_batch_adaptive.argtypes = [u8, u8, u8, u8, u8, i32, i64, i64, i64, ctypes.c_double, u64,
+                                                               u64, ctypes.c_uint64, i64, i32, ctypes.c_uint32, u64, u64, u64,
+                                                               u64, u64, vp, vp]
                 L.npk_equity_ranges_known_host.argtypes = [u8, u8, u8, u8, u8, i32, i64, i64, u64, u64, ctypes.c_uint64, i32,
                                                            u64, u64, u64, u64]
                 L.npk_peer_create.argtypes = [i32, i32, i64, ctypes.POINTER(ctypes.c_void_p), vp]

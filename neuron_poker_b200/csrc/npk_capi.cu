@@ -265,11 +265,12 @@ __global__ void __launch_bounds__(256) classify_fill_kernel(const uint8_t* hole,
     }
 }
 
-// ---- adaptive calls (npk_equity_batch_adaptive) -----------------------------------------------------------------------
+// ---- adaptive calls (npk_equity_batch_adaptive, npk_equity_ranges_batch_adaptive) ----------------------------------------
 // Workspace: the header and qindex of npk_equity_workspace_bytes(Q) (reused by every round), then at adaptive_base(Q) a
-// 64-byte block of u32 words -- queries still active (a running sum), blocks done, invalid queries, the next round's
-// {chunk, chunks} -- and active [Q] bytes.  The running sum and the block count are reset by the block that consumes them.
-constexpr int kAdActive = 0, kAdBlocksDone = 1, kAdInvalid = 2, kAdPlan = 4, kAdHeaderBytes = 64;
+// 64-byte block of u32 words -- queries still active (a running sum), blocks done, invalid queries, the qindex cursor of the
+// range call, the next round's {chunk, chunks, queries} -- and active [Q] bytes.  The running sum, the cursor and the block
+// count are reset by the block that consumes them.
+constexpr int kAdActive = 0, kAdBlocksDone = 1, kAdInvalid = 2, kAdCursor = 3, kAdPlan = 4, kAdHeaderBytes = 64;
 int64_t adaptive_base(int64_t Q) { return (npk_equity_workspace_bytes(Q) + 255) & ~int64_t(255); }
 
 // The stopping rule after checkpoint t: x = wins + ties, p = (x + 1) / (t + 2), var = p (1 - p) / t, stop if var <= bound
@@ -283,8 +284,10 @@ __device__ __forceinline__ bool adaptive_stop(unsigned long long x, long long t,
 }
 
 // Block sums of the queries still active (and of invalid ones) go to the workspace; the last block to finish plans the next
-// round's work items from the total and resets the sum for the next round.
-__device__ void adaptive_count(uint32_t n_active, uint32_t n_invalid, uint32_t* hdr, long long next_trials, int sm_count)
+// round's work items from the total (items a multiple of `lanes_worth` trials, as the round's kernel iterates), publishes the
+// total next to the plan and resets the sum and the cursor for the next round.
+__device__ void adaptive_count(uint32_t n_active, uint32_t n_invalid, uint32_t* hdr, long long next_trials, int sm_count,
+                               int lanes_worth)
 {
     __shared__ uint32_t s_n[2];
     if (threadIdx.x == 0) { s_n[0] = 0; s_n[1] = 0; }
@@ -300,9 +303,22 @@ __device__ void adaptive_count(uint32_t n_active, uint32_t n_invalid, uint32_t* 
     __threadfence();
     const uint32_t total = *reinterpret_cast<volatile uint32_t*>(&hdr[kAdActive]);
     uint32_t chunk, chunks;
-    npk::item_plan(total, next_trials, sm_count, 64, chunk, chunks);
-    hdr[kAdPlan] = chunk; hdr[kAdPlan + 1] = chunks;
-    hdr[kAdActive] = 0; hdr[kAdBlocksDone] = 0;
+    npk::item_plan(total, next_trials, sm_count, lanes_worth, chunk, chunks);
+    hdr[kAdPlan] = chunk; hdr[kAdPlan + 1] = chunks; hdr[kAdPlan + 2] = total;
+    hdr[kAdActive] = 0; hdr[kAdBlocksDone] = 0; hdr[kAdCursor] = 0;
+}
+
+// Append the queries of the warp with `keep` to `list` at the cursor, one atomic per warp (the order does not matter: the
+// counters are integer atomics).  Every lane of the warp calls it.
+__device__ __forceinline__ void append_queries(uint32_t* cursor, int32_t* list, bool keep, long long q)
+{
+    const uint32_t votes = __ballot_sync(0xffffffffu, keep);
+    if (!votes) return;
+    const int lane = threadIdx.x & 31, leader = __ffs(votes) - 1;
+    uint32_t base = 0;
+    if (lane == leader) base = atomicAdd(cursor, (uint32_t)__popc(votes));
+    base = __shfl_sync(0xffffffffu, base, leader);
+    if (keep) list[base + __popc(votes & ((1u << lane) - 1u))] = (int32_t)q;
 }
 
 // Zero the outputs (the stopping rule reads the counters, so the call owns them) and mark the valid queries of the caller's
@@ -326,15 +342,17 @@ __global__ void __launch_bounds__(256) adaptive_init_kernel(const uint8_t* hole,
         n += a;
         bad += g < 0;
     }
-    adaptive_count(n, bad, hdr, first_trials, sm_count);
+    adaptive_count(n, bad, hdr, first_trials, sm_count, 64);
 }
 
 // After the round that ends at checkpoint t: retire every active query the rule stops (all of them in the final round),
 // recording trials = t, and plan the next round of `next_trials` trials for the queries left.  Grid: one thread per query.
+// `qindex` or null: the list of the queries left, which the range kernels read (the all-shapes kernel's rounds classify).
 __global__ void __launch_bounds__(256) adaptive_retire_kernel(long long Q, const unsigned long long* wins,
                                                               const unsigned long long* ties, unsigned long long* trials,
                                                               uint8_t* active, uint32_t* hdr, long long t, double max_stderr,
-                                                              int final_round, long long next_trials, int sm_count)
+                                                              int final_round, long long next_trials, int sm_count,
+                                                              int32_t* qindex, int lanes_worth)
 {
     const double bound = __dmul_rn(max_stderr, max_stderr);
     uint32_t n = 0;
@@ -347,7 +365,8 @@ __global__ void __launch_bounds__(256) adaptive_retire_kernel(long long Q, const
             n = 1;
         }
     }
-    adaptive_count(n, 0, hdr, next_trials, sm_count);
+    if (qindex) append_queries(hdr + kAdCursor, qindex, n != 0, q);
+    adaptive_count(n, 0, hdr, next_trials, sm_count, lanes_worth);
 }
 
 // T_0 = min_trials, T_{k+1} = min(2 T_k, max_trials), up to max_trials.
@@ -736,7 +755,7 @@ int npk_equity_batch_adaptive(const uint8_t* hole, const uint8_t* board, const u
         if ((rc = enqueue_mixed(ds, p, hole, board, n_players, Q, ~0ull, ws, s, active))) return rc;
         const bool final_round = k + 1 == cp.size();
         adaptive_retire_kernel<<<retire_grid, 256, 0, s>>>(Q, w, t, n_trials, active, hdr, cp[k], max_stderr, final_round ? 1 : 0,
-                                                         final_round ? 0 : cp[k + 1] - cp[k], ds->sm_count);
+                                                         final_round ? 0 : cp[k + 1] - cp[k], ds->sm_count, nullptr, 64);
         if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "adaptive_retire_kernel launch");
         done = cp[k];
     }
@@ -1259,33 +1278,123 @@ int npk_equity_batch_sharded(void* group, const uint8_t* hole, const uint8_t* bo
 }  // extern "C"
 
 // ---- ranges ------------------------------------------------------------------------------------------------------------
+namespace {
+// Is query q of a range call valid?  `hole` is null when the hero is drawn from a range.
+__device__ bool range_query_valid(const uint8_t* hole, const uint8_t* board, const uint8_t* n_players, const uint8_t* ghost,
+                                  const uint8_t* known_opp, int n_known, long long q)
+{
+    const int np = n_players[q];
+    unsigned long long mask;
+    int bad = npk::validate_query(hole ? hole + 2 * q : nullptr, board + 5 * q, np, &mask) < 0;
+    if (ghost) {
+        // the reference pops ghost cards from the deck first (montecarlo_python.py:206-208): a board card equal to
+        // a ghost card then fails list.index (ValueError); a hero card equal to one is silently kept (:154-161)
+        const int g0 = ghost[2 * q], g1 = ghost[2 * q + 1];
+        if ((g0 == 0xFF) != (g1 == 0xFF)) bad = 1;
+        else if (g0 != 0xFF) {
+            if (g0 >= 52 || g1 >= 52 || g0 == g1) bad = 1;
+            else { bad |= (int)((mask >> g0 | mask >> g1) & 1ull); mask |= (1ull << g0) | (1ull << g1); }
+        }
+    }
+    // opponents with known cards: valid ids, no card twice anywhere, and no more of them than opponents
+    if (n_known > np - 1) bad = 1;
+    for (int f = 0; f < 2 * n_known; f++) {
+        const int c = known_opp[2 * q * n_known + f];
+        if (c >= 52) bad = 1; else { bad |= (int)(mask >> c & 1ull); mask |= 1ull << c; }
+    }
+    return !bad;
+}
+
 __global__ void validate_ranges_kernel(const uint8_t* hole, const uint8_t* board, const uint8_t* n_players,
                                        const uint8_t* ghost, const uint8_t* known_opp, int n_known, long long Q, uint8_t* ws)
 {
     uint32_t* invalid = reinterpret_cast<uint32_t*>(ws + kWsInvalid);
-    for (long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x; q < Q; q += (long long)gridDim.x * blockDim.x) {
-        const int np = n_players[q];
-        unsigned long long mask;
-        int bad = npk::validate_query(hole ? hole + 2 * q : nullptr, board + 5 * q, np, &mask) < 0;
-        if (ghost) {
-            // the reference pops ghost cards from the deck first (montecarlo_python.py:206-208): a board card equal to
-            // a ghost card then fails list.index (ValueError); a hero card equal to one is silently kept (:154-161)
-            const int g0 = ghost[2 * q], g1 = ghost[2 * q + 1];
-            if ((g0 == 0xFF) != (g1 == 0xFF)) bad = 1;
-            else if (g0 != 0xFF) {
-                if (g0 >= 52 || g1 >= 52 || g0 == g1) bad = 1;
-                else { bad |= (int)((mask >> g0 | mask >> g1) & 1ull); mask |= (1ull << g0) | (1ull << g1); }
-            }
-        }
-        // opponents with known cards: valid ids, no card twice anywhere, and no more of them than opponents
-        if (n_known > np - 1) bad = 1;
-        for (int f = 0; f < 2 * n_known; f++) {
-            const int c = known_opp[2 * q * n_known + f];
-            if (c >= 52) bad = 1; else { bad |= (int)(mask >> c & 1ull); mask |= 1ull << c; }
-        }
-        if (bad) atomicAdd(invalid, 1u);
-    }
+    for (long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x; q < Q; q += (long long)gridDim.x * blockDim.x)
+        if (!range_query_valid(hole, board, n_players, ghost, known_opp, n_known, q)) atomicAdd(invalid, 1u);
 }
+
+// The adaptive range call's start: zero the outputs, mark the valid queries active, list them in qindex for the first round
+// and plan it.  Grid: one thread per query (append_queries wants whole warps).
+__global__ void __launch_bounds__(256) ranges_adaptive_init_kernel(const uint8_t* hole, const uint8_t* board,
+                                                                   const uint8_t* n_players, const uint8_t* ghost,
+                                                                   const uint8_t* known_opp, int n_known, long long Q,
+                                                                   unsigned long long* wins, unsigned long long* ties,
+                                                                   unsigned long long* win_types, unsigned long long* passes,
+                                                                   unsigned long long* trials, uint8_t* active, uint32_t* hdr,
+                                                                   int32_t* qindex, long long first_trials, int sm_count)
+{
+    const long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    bool a = false;
+    uint32_t bad = 0;
+    if (q < Q) {
+        wins[q] = 0; ties[q] = 0; trials[q] = 0;
+        if (win_types)
+            for (int i = 0; i < 9; i++) win_types[9 * q + i] = 0;
+        if (passes) passes[q] = 0;
+        a = range_query_valid(hole, board, n_players, ghost, known_opp, n_known, q);
+        active[q] = a ? 1 : 0;
+        bad = !a;
+    }
+    append_queries(hdr + kAdCursor, qindex, a, q);
+    adaptive_count(a ? 1u : 0u, bad, hdr, first_trials, sm_count, 32);
+}
+
+std::string ranges_invalid_message(uint32_t bad)
+{
+    return std::to_string(bad) + " invalid quer" + (bad == 1 ? "y" : "ies") +
+           " (card id >= 52, duplicate cards, gap in the board, ghost card on the board or in a hand, more known opponents "
+           "than opponents, or players outside 1..10)";
+}
+
+int ranges_aborted()
+{
+    return fail(NPK_ERR_RANGE, "a draw needed more than 65536 attempts: no remaining hand satisfies the range (the reference "
+                               "would loop forever); the counters are incomplete");
+}
+
+// The arguments both range entry points share, checked before the device is touched -- null pointers (`buffers`: the
+// caller's outputs and workspace are all given), known opponents, the dealing mode, empty ranges -- and the launch fields
+// that carry them: ghost cards, known hands, the two class masks.  `p` comes from fill_params.
+int range_params(npk::EquityParams& p, const uint8_t* hole, const uint8_t* board, const uint8_t* n_players,
+                 const uint8_t* ghost, const uint8_t* known_opp, int n_known, const uint64_t* opp_allowed,
+                 const uint64_t* hero_allowed, bool buffers, int deal_mode)
+{
+    if ((!hole && !hero_allowed) || !board || !n_players || !buffers || !opp_allowed)
+        return fail(NPK_ERR_INVALID_ARGUMENT, "null pointer");
+    if (n_known < 0 || n_known > 9 || (n_known > 0 && !known_opp))
+        return fail(NPK_ERR_INVALID_ARGUMENT, "n_known must be 0..9 and known_opp must be given when it is not 0");
+    if (n_known > 0 && hero_allowed)
+        return fail(NPK_ERR_INVALID_ARGUMENT, "a hero range together with known opponent hands is not supported (the reference "
+                                              "draws the hero before it removes the known hands, montecarlo_python.py:132-163)");
+    int rc = check_deal_mode(deal_mode);
+    if (rc) return rc;
+    const uint64_t top = (1ull << (169 - 128)) - 1ull;
+    if (!(opp_allowed[0] | opp_allowed[1] | (opp_allowed[2] & top)))
+        return fail(NPK_ERR_RANGE, "the opponent range is empty (the reference would never finish a draw)");
+    if (hero_allowed && !(hero_allowed[0] | hero_allowed[1] | (hero_allowed[2] & top)))
+        return fail(NPK_ERR_RANGE, "the hero range is empty (the reference would never finish a draw)");
+    p.ghost = ghost;
+    p.known_opp = n_known > 0 ? known_opp : nullptr; p.n_known = (uint32_t)n_known;
+    for (int i = 0; i < 3; i++) {
+        const uint64_t o = i == 2 ? opp_allowed[i] & top : opp_allowed[i];
+        const uint64_t h = hero_allowed ? (i == 2 ? hero_allowed[i] & top : hero_allowed[i]) : 0;
+        p.opp_mask[2 * i] = (uint32_t)o; p.opp_mask[2 * i + 1] = (uint32_t)(o >> 32);
+        p.hero_mask[2 * i] = (uint32_t)h; p.hero_mask[2 * i + 1] = (uint32_t)(h >> 32);
+    }
+    p.hero_range = hero_allowed ? 1u : 0u;
+    return NPK_OK;
+}
+
+// `passes` is a by-product of the reference's attempt loop: only the generic kernel, which plays that loop literally,
+// can count it; everyone else gets the pair-list sampler (csrc/npk_ranges.cu), which redraws far less often
+int launch_ranges(const DeviceState* ds, const npk::EquityParams& p, int deal_mode, long long items, cudaStream_t s)
+{
+    const int grid = grid_for(*ds, items, npk::kRefThreads / 32);
+    const cudaError_t e = p.passes ? npk::launch_equity_ranges(deal_mode, p, grid, s)
+                                   : npk::launch_equity_ranges_fast(deal_mode, p, grid, s);
+    return e == cudaSuccess ? NPK_OK : cuda_fail(e, "equity_ranges_kernel launch");
+}
+}  // namespace
 
 int npk_equity_ranges_batch(const uint8_t* hole, const uint8_t* board, const uint8_t* n_players, const uint8_t* ghost,
                             int64_t Q, int64_t trials, const uint64_t* opp_allowed, const uint64_t* hero_allowed,
@@ -1308,37 +1417,17 @@ int npk_equity_ranges_known_batch(const uint8_t* hole, const uint8_t* board, con
     DeviceState* ds;
     int rc = batch_start(&ds, Q, trials, trial_offset);
     if (rc) return rc == kEmptyBatch ? NPK_OK : rc;
-    if ((!hole && !hero_allowed) || !board || !n_players || !wins_strict || !ties || !workspace || !opp_allowed)
-        return fail(NPK_ERR_INVALID_ARGUMENT, "null pointer");
-    if (n_known < 0 || n_known > 9 || (n_known > 0 && !known_opp))
-        return fail(NPK_ERR_INVALID_ARGUMENT, "n_known must be 0..9 and known_opp must be given when it is not 0");
-    if (n_known > 0 && hero_allowed)
-        return fail(NPK_ERR_INVALID_ARGUMENT, "a hero range together with known opponent hands is not supported (the reference "
-                                              "draws the hero before it removes the known hands, montecarlo_python.py:132-163)");
-    if ((rc = check_deal_mode(deal_mode))) return rc;
-    const uint64_t top = (1ull << (169 - 128)) - 1ull;
-    if (!(opp_allowed[0] | opp_allowed[1] | (opp_allowed[2] & top)))
-        return fail(NPK_ERR_RANGE, "the opponent range is empty (the reference would never finish a draw)");
-    if (hero_allowed && !(hero_allowed[0] | hero_allowed[1] | (hero_allowed[2] & top)))
-        return fail(NPK_ERR_RANGE, "the hero range is empty (the reference would never finish a draw)");
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     uint8_t* ws = static_cast<uint8_t*>(workspace);
-    if ((rc = clear_workspace(ws, s))) return rc;
-
     npk::EquityParams p;
     const long long chunks = fill_params(p, *ds, hero_allowed ? nullptr : hole, board, n_players, Q, trials, trial_offset,
                                          query_offset, seed, deal_mode, wins_strict, ties, win_types, passes,
                                          reinterpret_cast<uint32_t*>(ws + kWsAbort), 32);
-    p.ghost = ghost;
-    p.known_opp = n_known > 0 ? known_opp : nullptr; p.n_known = (uint32_t)n_known;
+    if ((rc = range_params(p, hole, board, n_players, ghost, known_opp, n_known, opp_allowed, hero_allowed,
+                           wins_strict && ties && workspace, deal_mode)))
+        return rc;
+    if ((rc = clear_workspace(ws, s))) return rc;
     p.work_counter = reinterpret_cast<unsigned long long*>(ws + kWsCounters);
-    for (int i = 0; i < 3; i++) {
-        const uint64_t o = i == 2 ? opp_allowed[i] & top : opp_allowed[i];
-        const uint64_t h = hero_allowed ? (i == 2 ? hero_allowed[i] & top : hero_allowed[i]) : 0;
-        p.opp_mask[2 * i] = (uint32_t)o; p.opp_mask[2 * i + 1] = (uint32_t)(o >> 32);
-        p.hero_mask[2 * i] = (uint32_t)h; p.hero_mask[2 * i + 1] = (uint32_t)(h >> 32);
-    }
-    p.hero_range = hero_allowed ? 1u : 0u;
 
     const bool validate = (flags & NPK_FLAG_VALIDATE) != 0;
     cudaError_t e;
@@ -1349,22 +1438,93 @@ int npk_equity_ranges_known_batch(const uint8_t* hole, const uint8_t* board, con
         e = cudaMemcpyAsync(&bad, ws + kWsInvalid, 4, cudaMemcpyDeviceToHost, s);
         if (e == cudaSuccess) e = cudaStreamSynchronize(s);
         if (e != cudaSuccess) return cuda_fail(e, "query validation");
-        if (bad) return fail(NPK_ERR_INVALID_CARDS, std::to_string(bad) + " invalid quer" + (bad == 1 ? "y" : "ies") +
-                             " (card id >= 52, duplicate cards, gap in the board, ghost card on the board or in a "
-                             "hand, more known opponents than opponents, or players outside 1..10)");
+        if (bad) return fail(NPK_ERR_INVALID_CARDS, ranges_invalid_message(bad));
     }
-    // `passes` is a by-product of the reference's attempt loop: only the generic kernel, which plays that loop literally,
-    // can count it; everyone else gets the pair-list sampler (csrc/npk_ranges.cu), which redraws far less often
-    e = passes ? npk::launch_equity_ranges(deal_mode, p, grid_for(*ds, Q * chunks, npk::kRefThreads / 32), s)
-               : npk::launch_equity_ranges_fast(deal_mode, p, grid_for(*ds, Q * chunks, npk::kRefThreads / 32), s);
-    if (e != cudaSuccess) return cuda_fail(e, "equity_ranges_kernel launch");
+    if ((rc = launch_ranges(ds, p, deal_mode, Q * chunks, s))) return rc;
     if (validate) {
         uint32_t aborted = 0;
         e = cudaMemcpyAsync(&aborted, ws + kWsAbort, 4, cudaMemcpyDeviceToHost, s);
         if (e == cudaSuccess) e = cudaStreamSynchronize(s);
         if (e != cudaSuccess) return cuda_fail(e, "equity_ranges_kernel");
-        if (aborted) return fail(NPK_ERR_RANGE, "a draw needed more than 65536 attempts: no remaining hand satisfies the "
-                                                "range (the reference would loop forever); the counters are incomplete");
+        if (aborted) return ranges_aborted();
+    }
+    return NPK_OK;
+}
+
+int npk_equity_ranges_batch_adaptive(const uint8_t* hole, const uint8_t* board, const uint8_t* n_players, const uint8_t* ghost,
+                                     const uint8_t* known_opp, int n_known, int64_t Q, int64_t min_trials, int64_t max_trials,
+                                     double max_stderr, const uint64_t* opp_allowed, const uint64_t* hero_allowed,
+                                     uint64_t seed, int64_t query_offset, int deal_mode, uint32_t flags,
+                                     uint64_t* wins_strict, uint64_t* ties, uint64_t* win_types, uint64_t* passes,
+                                     uint64_t* trials, void* workspace, void* stream)
+{
+    // the arguments of the rule first: these errors need no device
+    if (!std::isfinite(max_stderr) || max_stderr <= 0.0)
+        return fail(NPK_ERR_INVALID_ARGUMENT, "stderr must be a finite number > 0");
+    if (min_trials < 1) return fail(NPK_ERR_INVALID_ARGUMENT, "min_trials must be >= 1");
+    if (min_trials > max_trials) return fail(NPK_ERR_INVALID_ARGUMENT, "min_trials must not exceed max_trials");
+    DeviceState* ds;
+    int rc = batch_start(&ds, Q, max_trials, 0);
+    if (rc) return rc == kEmptyBatch ? NPK_OK : rc;
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    uint8_t* ws = static_cast<uint8_t*>(workspace);
+    const std::vector<long long> cp = adaptive_checkpoints(min_trials, max_trials);
+    npk::EquityParams p;
+    fill_params(p, *ds, hero_allowed ? nullptr : hole, board, n_players, Q, cp[0], 0, query_offset, seed, deal_mode,
+                wins_strict, ties, win_types, passes, reinterpret_cast<uint32_t*>(ws + kWsAbort), 32);
+    if ((rc = range_params(p, hole, board, n_players, ghost, known_opp, n_known, opp_allowed, hero_allowed,
+                           wins_strict && ties && trials && workspace, deal_mode)))
+        return rc;
+    uint32_t* hdr = reinterpret_cast<uint32_t*>(ws + adaptive_base(Q));
+    uint8_t* active = ws + adaptive_base(Q) + kAdHeaderBytes;
+    int32_t* qindex = reinterpret_cast<int32_t*>(ws + kWsIndex);
+    auto* w = reinterpret_cast<unsigned long long*>(wins_strict);
+    auto* t = reinterpret_cast<unsigned long long*>(ties);
+    auto* n_trials = reinterpret_cast<unsigned long long*>(trials);
+    const unsigned int grid = (unsigned int)((Q + 255) / 256);
+
+    // the abort flag is cleared once: a round that hits the attempt limit stops every later round at once
+    if ((rc = clear_workspace(ws, s))) return rc;
+    cudaError_t e = cudaMemsetAsync(hdr, 0, kAdHeaderBytes, s);
+    if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(workspace)");
+    ranges_adaptive_init_kernel<<<grid, 256, 0, s>>>(p.hole, board, n_players, ghost, p.known_opp, n_known, Q, w, t,
+                                                     p.win_types, p.passes, n_trials, active, hdr, qindex, cp[0],
+                                                     ds->sm_count);
+    if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "ranges_adaptive_init_kernel launch");
+    if (flags & NPK_FLAG_VALIDATE) {
+        uint32_t bad = 0;
+        e = cudaMemcpyAsync(&bad, hdr + kAdInvalid, 4, cudaMemcpyDeviceToHost, s);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+        if (e != cudaSuccess) return cuda_fail(e, "query validation");
+        if (bad) return fail(NPK_ERR_INVALID_CARDS, ranges_invalid_message(bad));
+    }
+
+    // one round per checkpoint, back to back on the stream: the trials [T_{k-1}, T_k) of the queries listed in qindex, then
+    // the rule, which lists the queries left and plans the next round
+    p.plan = hdr + kAdPlan;
+    p.qindex = qindex;
+    p.work_counter = reinterpret_cast<unsigned long long*>(ws + kWsCounters);
+    long long done = 0;
+    for (size_t k = 0; k < cp.size(); k++) {
+        e = cudaMemsetAsync(p.work_counter, 0, sizeof(unsigned long long), s);
+        if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(workspace)");
+        p.trials = cp[k] - done;
+        p.trial_offset = done;
+        uint32_t chunk, chunks;                 // the grid: sized for every query, the most this round can have
+        npk::item_plan(Q, p.trials, ds->sm_count, 32, chunk, chunks);
+        if ((rc = launch_ranges(ds, p, deal_mode, Q * (long long)chunks, s))) return rc;
+        const bool final_round = k + 1 == cp.size();
+        adaptive_retire_kernel<<<grid, 256, 0, s>>>(Q, w, t, n_trials, active, hdr, cp[k], max_stderr, final_round ? 1 : 0,
+                                                    final_round ? 0 : cp[k + 1] - cp[k], ds->sm_count, qindex, 32);
+        if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "adaptive_retire_kernel launch");
+        done = cp[k];
+    }
+    if (flags & NPK_FLAG_VALIDATE) {
+        uint32_t aborted = 0;
+        e = cudaMemcpyAsync(&aborted, ws + kWsAbort, 4, cudaMemcpyDeviceToHost, s);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+        if (e != cudaSuccess) return cuda_fail(e, "equity_ranges_kernel");
+        if (aborted) return ranges_aborted();
     }
     return NPK_OK;
 }

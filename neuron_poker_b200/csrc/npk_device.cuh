@@ -46,7 +46,8 @@ struct SmemTables {
 // restore shows up there).  A failed check records its code in DeviceTables::check (npk_checked_status reads it).
 // Codes: 1 rowoff gather, 2 value gather, 3 flush gather, 4 Fisher-Yates slot, 5 Lehmer slot, 6 duplicate Lehmer slot,
 //        7 deck not restored, 8 descriptor index, 9 pair list of the range sampler (entry index, card ids),
-//        10 unseen-card slot or pair index of the showdown-equity enumeration.
+//        10 unseen-card slot or pair index of the showdown-equity enumeration,
+//        11 query slot of a device-planned range round, or the query id read from its qindex.
 #ifdef NPK_CHECKED
 #define NPK_CHECK(ptr, cond, code) do { if (!(cond)) atomicMax((ptr), (unsigned)(code)); } while (0)
 #else

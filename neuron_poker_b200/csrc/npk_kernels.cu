@@ -5,7 +5,7 @@
 //                                       with the C++ sibling's dealing semantics (Montecarlo.cpp:293-312)
 //   equity_refdeal_kernel<NOPP,NB>  K1' same loop with the Python reference's own (biased) dealer
 //                                       (montecarlo_python.py:165-189)
-//   equity_ranges_kernel<MODE>      K1'' generic dealer with opponent / hero ranges and ghost cards (the reference's attempt
+//   equity_ranges_kernel<MODE,PLAN> K1'' generic dealer with opponent / hero ranges and ghost cards (the reference's attempt
 //                                       loop played literally; the pair-list sampler lives in npk_ranges.cu, the persistent
 //                                       all-shapes kernel for mixed batches in npk_mixed.cu, the per-trial code in npk_mc.cuh)
 //   rank7_kernel / rank7_colex      K2  batched 7-card rank ids (hand_evaluator.py:27-119 `_calc_score` ordering)
@@ -72,7 +72,8 @@ __device__ __forceinline__ bool class_allowed(const uint32_t (&mask)[6], int c1,
     return (mask[k >> 5] >> (k & 31)) & 1u;
 }
 
-template <int MODE>
+// PLAN = 1: a round of an adaptive call (npk_equity_ranges_batch_adaptive), whose items are planned on the device.
+template <int MODE, int PLAN>
 __global__ void __launch_bounds__(kRefThreads, 1) equity_ranges_kernel(const EquityParams p)
 {
     extern __shared__ __align__(128) uint8_t smem[];
@@ -80,11 +81,11 @@ __global__ void __launch_bounds__(kRefThreads, 1) equity_ranges_kernel(const Equ
     const SmemAddr st = smem_addr(stage_tables(p.tables, smem + 128, bar));
     const int lane = threadIdx.x & 31;
 
-    const long long n_items = p.nq * p.chunks;
+    const long long n_items = range_items<PLAN>(p);
 
     for (long long item = next_item(p.work_counter, lane); item < n_items; item = next_item(p.work_counter, lane)) {
         long long q, t_begin, t_end;
-        item_range(p, item, q, t_begin, t_end);
+        range_item<PLAN>(p, item, q, t_begin, t_end);
         int known = 0;
         for (int i = 0; i < 5; i++) known += p.board[5 * q + i] != 0xFF;
         // opponents dealt at random; the others' cards are known (montecarlo_python.py:132-163: removed from the deck like the
@@ -673,7 +674,8 @@ size_t aux_smem(const DeviceTables& t) { return 128 + t.value_bytes + t.rowoff_b
 cudaError_t launch_equity_ranges(int deal_mode, const EquityParams& p, int grid, cudaStream_t s)
 {
     size_t smem = aux_smem(p.tables);
-    auto k = deal_mode == 1 ? equity_ranges_kernel<1> : equity_ranges_kernel<0>;
+    auto k = !p.plan ? (deal_mode == 1 ? equity_ranges_kernel<1, 0> : equity_ranges_kernel<0, 0>)
+                     : (deal_mode == 1 ? equity_ranges_kernel<1, 1> : equity_ranges_kernel<0, 1>);
     cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     k<<<grid, kRefThreads, smem, s>>>(p);

@@ -111,8 +111,10 @@ struct EquityParams {
                                   // player_card_list, montecarlo_python.py:132-163), or null
     uint32_t n_known;             // how many of the n_players - 1 opponents those are
     uint32_t* abort_flag;         // raised when one draw needs more than kMaxRangeAttempts attempts
-    // ---- adaptive calls (npk_equity_batch_adaptive): {chunk, chunks} of this round, written on the device by the kernel
-    // that retired the previous round's queries; the all-shapes kernel reads them instead of chunk / chunks when non-null
+    // ---- adaptive calls (npk_equity_batch_adaptive, npk_equity_ranges_batch_adaptive): {chunk, chunks, queries} of this
+    // round, written on the device by the kernel that retired the previous round's queries; the all-shapes and range kernels
+    // read them instead of chunk / chunks (and the range kernels read `queries` instead of nq, the query slots from qindex)
+    // when non-null
     const uint32_t* plan;
 };
 

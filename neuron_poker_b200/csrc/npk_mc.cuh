@@ -26,6 +26,31 @@ __device__ __forceinline__ void item_range(const EquityParams& p, long long item
     end = min(p.trials, begin + (long long)p.chunk);
 }
 
+// Items of the range kernels.  PLAN = 1: a round of an adaptive range call, where p.plan = {chunk, chunks, queries} and the
+// query slots p.qindex [queries] (the queries still active) are written on the device by the kernel that retired the previous
+// round's queries.  PLAN = 0: queries 0..nq-1 as planned by the host.
+template <int PLAN>
+__device__ __forceinline__ long long range_items(const EquityParams& p)
+{
+    return PLAN ? (long long)p.plan[2] * p.plan[1] : p.nq * p.chunks;
+}
+
+template <int PLAN>
+__device__ __forceinline__ void range_item(const EquityParams& p, long long item, long long& q, long long& begin, long long& end)
+{
+    if (PLAN) {
+        const uint32_t chunk = p.plan[0], chunks = p.plan[1];
+        const long long slot = item / chunks;
+        begin = (item - slot * chunks) * chunk;
+        end = min(p.trials, begin + (long long)chunk);
+        NPK_CHECK(p.tables.check, slot < (long long)p.plan[2], 11);
+        q = p.qindex[slot];
+        NPK_CHECK(p.tables.check, q >= 0 && q < p.nq, 11);
+    } else {
+        item_range(p, item, q, begin, end);
+    }
+}
+
 // Per-query constants shared by every trial of a work item.
 struct QueryStatic {
     uint32_t hero_sum;    // desc(h0) + desc(h1)

@@ -56,7 +56,8 @@ __device__ __forceinline__ uint32_t build_list(const uint16_t* s_pair, const uin
     return n;
 }
 
-template <int MODE>
+// PLAN = 1: a round of an adaptive call (npk_equity_ranges_batch_adaptive), whose items are planned on the device.
+template <int MODE, int PLAN>
 __global__ void __launch_bounds__(kRefThreads, 1) equity_ranges_fast_kernel(const EquityParams p)
 {
     extern __shared__ __align__(128) uint8_t smem[];
@@ -87,10 +88,10 @@ __global__ void __launch_bounds__(kRefThreads, 1) equity_ranges_fast_kernel(cons
     }
     __syncthreads();
 
-    const long long n_items = p.nq * p.chunks;
+    const long long n_items = range_items<PLAN>(p);
     for (long long item = next_item(p.work_counter, lane); item < n_items; item = next_item(p.work_counter, lane)) {
         long long q, t_begin, t_end;
-        item_range(p, item, q, t_begin, t_end);
+        range_item<PLAN>(p, item, q, t_begin, t_end);
         int known = 0;
         for (int i = 0; i < 5; i++) known += p.board[5 * q + i] != 0xFF;
         const int nknown = (int)p.n_known;                    // opponents whose cards are known (montecarlo_python.py:132-163)
@@ -230,7 +231,8 @@ cudaError_t launch_equity_ranges_fast(int deal_mode, const EquityParams& p, int 
 {
     const size_t smem = 128 + (size_t)p.tables.value_bytes + p.tables.rowoff_bytes + p.tables.flush_bytes + kDescBytes + 2688 + 384 +
                         (size_t)(kRefThreads / 32) * 2 * 1344 * 2;
-    auto k = deal_mode == 1 ? equity_ranges_fast_kernel<1> : equity_ranges_fast_kernel<0>;
+    auto k = p.plan ? (deal_mode == 1 ? equity_ranges_fast_kernel<1, 1> : equity_ranges_fast_kernel<0, 1>)
+                    : (deal_mode == 1 ? equity_ranges_fast_kernel<1, 0> : equity_ranges_fast_kernel<0, 0>);
     cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     k<<<grid, kRefThreads, smem, s>>>(p);

@@ -369,20 +369,8 @@ def get_equity_ranges_batch(hole, board, n_players, trials, opponent_range=1, he
     set of class spellings (the hero is drawn from it every trial, `hole` may be None); ghost: None or [Q,2] uint8
     (0xFF = none).  Returns dict of int64 CUDA tensors like get_equity_batch."""
     import torch
-    dev = _resolve_device(device)
-    board = _as_cuda_u8(board, dev, (5,))
-    n_players = _as_cuda_u8(n_players, dev, ())
-    Q = board.shape[0]
-    hole = None if hero_range is not None else _as_cuda_u8(hole, dev, (2,))
-    ghost = None if ghost is None else _as_cuda_u8(ghost, dev, (2,))
-    n_known = 0
-    if known_opponents is not None:
-        known_opponents = torch.as_tensor(known_opponents, dtype=torch.uint8).to(dev).contiguous()
-        if known_opponents.dim() != 3 or known_opponents.shape[0] != Q or known_opponents.shape[2] != 2:
-            raise ValueError("known_opponents must have shape [Q, n_known, 2]")
-        n_known = int(known_opponents.shape[1])
-    opp_mask = ranges.opponent_mask(opponent_range)
-    hero_mask = None if hero_range is None else ranges.mask_from_classes(hero_range)
+    dev, a = _range_args(hole, board, n_players, opponent_range, hero_range, ghost, known_opponents, device)
+    Q = a.Q
     L = _lib.ensure_init(dev.index)
     with torch.cuda.device(dev):
         out = {} if out is None else out
@@ -392,10 +380,8 @@ def get_equity_ranges_batch(hole, board, n_players, trials, opponent_range=1, he
                 out[name] = torch.zeros(shape, dtype=torch.int64, device=dev)
         ws = torch.empty(int(L.npk_equity_workspace_bytes(Q)), dtype=torch.uint8, device=dev)
         stream = torch.cuda.current_stream(dev).cuda_stream
-        _lib.check(L.npk_equity_ranges_known_batch(hole.data_ptr() if hole is not None else None, board.data_ptr(),
-                                             n_players.data_ptr(), ghost.data_ptr() if ghost is not None else None,
-                                             known_opponents.data_ptr() if n_known else None, n_known, Q,
-                                             int(trials), _u64(opp_mask), _u64(hero_mask) if hero_mask is not None else None,
+        _lib.check(L.npk_equity_ranges_known_batch(a.hole, a.board, a.n_players, a.ghost, a.known, a.n_known, Q,
+                                             int(trials), _u64(a.opp_mask), a.hero_mask,
                                              ctypes.c_uint64(int(seed_value) & (2**64 - 1)), int(trial_offset),
                                              int(query_offset), _DEAL[deal_mode],
                                              _lib.NPK_FLAG_VALIDATE if validate else 0, out["wins"].data_ptr(),
@@ -404,6 +390,34 @@ def get_equity_ranges_batch(hole, board, n_players, trials, opponent_range=1, he
         ws.record_stream(torch.cuda.current_stream(dev))
     out["trials"] = int(trials)
     return out
+
+
+def _range_args(hole, board, n_players, opponent_range, hero_range, ghost, known_opponents, device):
+    """The arguments of the batched range calls as libnpk takes them: device pointers (or None), n_known, Q and the class
+    masks.  The namespace holds the tensors and mask arrays too, so that the pointers stay valid while it lives."""
+    import torch
+    from types import SimpleNamespace
+    dev = _resolve_device(device)
+    a = SimpleNamespace()
+    a.t_board = _as_cuda_u8(board, dev, (5,))
+    a.t_players = _as_cuda_u8(n_players, dev, ())
+    a.Q = Q = a.t_board.shape[0]
+    a.t_hole = None if hero_range is not None else _as_cuda_u8(hole, dev, (2,))
+    a.t_ghost = None if ghost is None else _as_cuda_u8(ghost, dev, (2,))
+    a.n_known, a.t_known = 0, None
+    if known_opponents is not None:
+        a.t_known = torch.as_tensor(known_opponents, dtype=torch.uint8).to(dev).contiguous()
+        if a.t_known.dim() != 3 or a.t_known.shape[0] != Q or a.t_known.shape[2] != 2:
+            raise ValueError("known_opponents must have shape [Q, n_known, 2]")
+        a.n_known = int(a.t_known.shape[1])
+    a.opp_mask = ranges.opponent_mask(opponent_range)
+    a.hero_mask_array = None if hero_range is None else ranges.mask_from_classes(hero_range)
+    a.hole = a.t_hole.data_ptr() if a.t_hole is not None else None
+    a.board, a.n_players = a.t_board.data_ptr(), a.t_players.data_ptr()
+    a.ghost = a.t_ghost.data_ptr() if a.t_ghost is not None else None
+    a.known = a.t_known.data_ptr() if a.n_known else None
+    a.hero_mask = _u64(a.hero_mask_array) if a.hero_mask_array is not None else None
+    return dev, a
 
 
 
@@ -541,5 +555,40 @@ def get_equity_batch_adaptive(hole, board, n_players, max_trials, stderr, min_tr
                                                out["win_types"].data_ptr() if win_types else None,
                                                out["passes"].data_ptr() if passes else None, out["trials"].data_ptr(),
                                                ws.data_ptr(), stream))
+        ws.record_stream(torch.cuda.current_stream(dev))
+    return out
+
+
+def get_equity_ranges_batch_adaptive(hole, board, n_players, max_trials, stderr, min_trials=256, opponent_range=1,
+                                     hero_range=None, ghost=None, known_opponents=None, seed_value=0, deal_mode="reference",
+                                     query_offset=0, device=None, validate=True, win_types=False, passes=False):
+    """get_equity_batch_adaptive for the range calls (npk_equity_ranges_batch_adaptive, asynchronous on the current torch
+    stream unless validate=True): every query runs until the standard error of its equity (wins + ties) / trials is at most
+    `stderr`, checked at adaptive_checkpoints(min_trials, max_trials), or until max_trials.  The range arguments are those of
+    get_equity_ranges_batch, and the counters of a query are exactly those of get_equity_ranges_batch(trials=T_stop) with the
+    same seed, query_offset, ranges, ghost cards, known hands and sampler (passes=True: the generic kernel, else the pair-list
+    sampler).  Returns the dict of get_equity_batch_adaptive: `trials` is an int64 CUDA tensor [Q] of every query's T_stop
+    (0 for an invalid query when validate=False)."""
+    import torch
+    dev, a = _range_args(hole, board, n_players, opponent_range, hero_range, ghost, known_opponents, device)
+    Q = a.Q
+    L = _lib.ensure_init(dev.index)
+    with torch.cuda.device(dev):
+        out = {}
+        for name, shape, want in (("wins", (Q,), True), ("ties", (Q,), True), ("win_types", (Q, 9), win_types),
+                                  ("passes", (Q,), passes), ("trials", (Q,), True)):
+            if want:
+                out[name] = (torch.empty if Q else torch.zeros)(shape, dtype=torch.int64, device=dev)   # zeroed by the call
+        ws = torch.empty(int(L.npk_equity_adaptive_workspace_bytes(Q)), dtype=torch.uint8, device=dev)
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        _lib.check(L.npk_equity_ranges_batch_adaptive(a.hole, a.board, a.n_players, a.ghost, a.known, a.n_known, Q,
+                                                      int(min_trials), int(max_trials), ctypes.c_double(float(stderr)),
+                                                      _u64(a.opp_mask), a.hero_mask,
+                                                      ctypes.c_uint64(int(seed_value) & (2**64 - 1)), int(query_offset),
+                                                      _DEAL[deal_mode], _lib.NPK_FLAG_VALIDATE if validate else 0,
+                                                      out["wins"].data_ptr(), out["ties"].data_ptr(),
+                                                      out["win_types"].data_ptr() if win_types else None,
+                                                      out["passes"].data_ptr() if passes else None, out["trials"].data_ptr(),
+                                                      ws.data_ptr(), stream))
         ws.record_stream(torch.cuda.current_stream(dev))
     return out

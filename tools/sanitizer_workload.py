@@ -114,6 +114,18 @@ for mode in ("reference", "uniform"):
     check(npk.get_equity_ranges_batch(ho2, bo2, np.full(6, 4, dtype=np.uint8), 400, opponent_range=0.4, seed_value=6,
                                       deal_mode=mode, known_opponents=kn, passes=mode == "reference"), 400, "known hands " + mode)
 print("ok known opponent hands", mc.equity, flush=True)
+# ranges to a target precision: rounds of both range kernels on the device-listed queries still active
+ho3, bo3, pl3 = queries(64, 4, 5)
+pl3[::4] = 1                                                        # retire at T_0: later rounds list a subset
+for mode in ("reference", "uniform"):
+    for passes in (True, False):
+        ad = npk.get_equity_ranges_batch_adaptive(ho3, bo3, pl3, 700, 0.03, min_trials=64, opponent_range=0.3, seed_value=8,
+                                                  deal_mode=mode, win_types=True, passes=passes)
+        torch.cuda.synchronize()
+        tr = ad["trials"].cpu().numpy()
+        assert ((tr >= 64) & (tr <= 700)).all() and ((ad["wins"] + ad["ties"]).cpu().numpy() <= tr).all(), mode
+        assert (tr[::4] == 64).all() and (tr > 64).any(), mode
+print("ok adaptive ranges", flush=True)
 
 # exact showdown equity of known hands: every player count and board size, dead cards, both dealers, garbage bytes
 se_h = np.full((40, 10, 2), 255, dtype=np.uint8); se_b = np.full((40, 5), 255, dtype=np.uint8)
