@@ -146,6 +146,24 @@ int cuda_fail(cudaError_t e, const char* what)
     return fail(NPK_ERR_CUDA, std::string(what) + ": " + cudaGetErrorString(e));
 }
 
+// Copy one u32 of device memory to `out` once the work enqueued on `s` before it has finished.
+int read_word(const void* src, cudaStream_t s, uint32_t* out, const char* what)
+{
+    cudaError_t e = cudaMemcpyAsync(out, src, 4, cudaMemcpyDeviceToHost, s);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+    return e == cudaSuccess ? NPK_OK : cuda_fail(e, what);
+}
+
+// The causes of an invalid query of the batched calls, as their NPK_ERR_INVALID_CARDS messages list them.
+constexpr const char* kQueryCauses = "card id >= 52, duplicate cards, gap in the board, or players outside 1..10";
+constexpr const char* kRangeQueryCauses = "card id >= 52, duplicate cards, gap in the board, ghost card on the board or in a "
+                                          "hand, more known opponents than opponents, or players outside 1..10";
+
+std::string invalid_queries(uint32_t n, const char* causes, const char* tail = "")
+{
+    return std::to_string(n) + " invalid quer" + (n == 1 ? "y" : "ies") + " (" + causes + ")" + tail;
+}
+
 int ensure_host_tables()
 {
     std::lock_guard<std::mutex> lk(g_mu);
@@ -321,28 +339,40 @@ __device__ __forceinline__ void append_queries(uint32_t* cursor, int32_t* list, 
     if (keep) list[base + __popc(votes & ((1u << lane) - 1u))] = (int32_t)q;
 }
 
-// Zero the outputs (the stopping rule reads the counters, so the call owns them) and mark the valid queries of the caller's
-// shapes active; plan the first round.
-__global__ void __launch_bounds__(256) adaptive_init_kernel(const uint8_t* hole, const uint8_t* board, const uint8_t* n_players,
-                                                            long long Q, unsigned long long shape_mask,
-                                                            unsigned long long* wins, unsigned long long* ties,
-                                                            unsigned long long* win_types, unsigned long long* passes,
-                                                            unsigned long long* trials, uint8_t* active, uint32_t* hdr,
-                                                            long long first_trials, int sm_count)
+// The query test of npk_equity_batch_adaptive: 1 = run it, 0 = a valid query outside the caller's shapes, -1 = invalid.
+// (The range call's is RangeTest.)
+struct ShapeTest {
+    const uint8_t *hole, *board, *n_players;
+    unsigned long long shape_mask;
+    __device__ int operator()(long long q) const
+    {
+        const int g = classify_query(hole, board, n_players, q);
+        return g < 0 ? -1 : (int)(shape_mask >> g & 1ull);
+    }
+};
+
+// Zero the outputs (the stopping rule reads the counters, so the call owns them), mark the queries `test` accepts active,
+// list them in `qindex` when it is given, and plan the first round.  Grid: one thread per query (append_queries wants whole
+// warps).
+template <class Test>
+__global__ void __launch_bounds__(256) adaptive_init_kernel(Test test, long long Q, unsigned long long* wins,
+                                                            unsigned long long* ties, unsigned long long* win_types,
+                                                            unsigned long long* passes, unsigned long long* trials,
+                                                            uint8_t* active, uint32_t* hdr, int32_t* qindex,
+                                                            long long first_trials, int sm_count, int lanes_worth)
 {
-    uint32_t n = 0, bad = 0;
-    for (long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x; q < Q; q += (long long)gridDim.x * blockDim.x) {
+    const long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    int v = 0;
+    if (q < Q) {
         wins[q] = 0; ties[q] = 0; trials[q] = 0;
         if (win_types)
             for (int i = 0; i < 9; i++) win_types[9 * q + i] = 0;
         if (passes) passes[q] = 0;
-        const int g = classify_query(hole, board, n_players, q);
-        const bool a = g >= 0 && (shape_mask >> g & 1ull);
-        active[q] = a ? 1 : 0;
-        n += a;
-        bad += g < 0;
+        v = test(q);
+        active[q] = v > 0 ? 1 : 0;
     }
-    adaptive_count(n, bad, hdr, first_trials, sm_count, 64);
+    if (qindex) append_queries(hdr + kAdCursor, qindex, v > 0, q);
+    adaptive_count(v > 0 ? 1u : 0u, v < 0 ? 1u : 0u, hdr, first_trials, sm_count, lanes_worth);
 }
 
 // After the round that ends at checkpoint t: retire every active query the rule stops (all of them in the final round),
@@ -375,6 +405,59 @@ std::vector<long long> adaptive_checkpoints(long long min_trials, long long max_
     std::vector<long long> t{min_trials};
     while (t.back() < max_trials) t.push_back(t.back() > max_trials / 2 ? max_trials : 2 * t.back());
     return t;
+}
+
+// The arguments of the stopping rule, checked before anything else: these errors need no device.
+int check_rule(int64_t min_trials, int64_t max_trials, double max_stderr)
+{
+    if (!std::isfinite(max_stderr) || max_stderr <= 0.0)
+        return fail(NPK_ERR_INVALID_ARGUMENT, "stderr must be a finite number > 0");
+    if (min_trials < 1) return fail(NPK_ERR_INVALID_ARGUMENT, "min_trials must be >= 1");
+    if (min_trials > max_trials) return fail(NPK_ERR_INVALID_ARGUMENT, "min_trials must not exceed max_trials");
+    return NPK_OK;
+}
+
+// The checkpoint sequence of an adaptive call, back to back on `s`; `p` holds the call's outputs and launch fields.  Start with
+// adaptive_init_kernel (with `validate`, an invalid query is an error before any trial: one read-back, the message
+// invalid_queries(n, causes, tail)), then one round per checkpoint: `round(active)` enqueues the trials [T_{k-1}, T_k)
+// (p.trial_offset, p.trials) of the queries still active, and the rule retires queries and plans the next round, appending
+// the queries left to `qindex` when it is given.  Items are planned in multiples of `lanes_worth` trials.
+template <class Test, class Round>
+int run_adaptive(const DeviceState& ds, npk::EquityParams& p, const Test& test, int64_t Q, int64_t min_trials,
+                 int64_t max_trials, double max_stderr, uint64_t* trials, uint8_t* ws, int32_t* qindex, int lanes_worth,
+                 bool validate, const char* what, const char* causes, const char* tail, cudaStream_t s, const Round& round)
+{
+    uint32_t* hdr = reinterpret_cast<uint32_t*>(ws + adaptive_base(Q));
+    uint8_t* active = ws + adaptive_base(Q) + kAdHeaderBytes;
+    auto* n_trials = reinterpret_cast<unsigned long long*>(trials);
+    const std::vector<long long> cp = adaptive_checkpoints(min_trials, max_trials);
+    const unsigned int grid = (unsigned int)((Q + 255) / 256);
+
+    cudaError_t e = cudaMemsetAsync(hdr, 0, kAdHeaderBytes, s);
+    if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(workspace)");
+    adaptive_init_kernel<<<grid, 256, 0, s>>>(test, Q, p.wins, p.ties, p.win_types, p.passes, n_trials, active, hdr, qindex,
+                                              cp[0], ds.sm_count, lanes_worth);
+    if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "adaptive_init_kernel launch");
+    int rc;
+    if (validate) {
+        uint32_t bad = 0;
+        if ((rc = read_word(hdr + kAdInvalid, s, &bad, what))) return rc;
+        if (bad) return fail(NPK_ERR_INVALID_CARDS, invalid_queries(bad, causes, tail));
+    }
+    p.plan = hdr + kAdPlan;
+    long long done = 0;
+    for (size_t k = 0; k < cp.size(); k++) {
+        p.trials = cp[k] - done;
+        p.trial_offset = done;
+        if ((rc = round(active))) return rc;
+        const bool final_round = k + 1 == cp.size();
+        adaptive_retire_kernel<<<grid, 256, 0, s>>>(Q, p.wins, p.ties, n_trials, active, hdr, cp[k], max_stderr,
+                                                    final_round ? 1 : 0, final_round ? 0 : cp[k + 1] - cp[k], ds.sm_count,
+                                                    qindex, lanes_worth);
+        if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "adaptive_retire_kernel launch");
+        done = cp[k];
+    }
+    return NPK_OK;
 }
 
 // Work items of a launch (npk::item_plan).  Returns the number of items per query.
@@ -633,9 +716,7 @@ int npk_equity_batch(const uint8_t* hole, const uint8_t* board, const uint8_t* n
         e = cudaMemcpyAsync(host, ws + kWsCounts, 4 * 129, cudaMemcpyDeviceToHost, s);
         if (e == cudaSuccess) e = cudaStreamSynchronize(s);
         if (e != cudaSuccess) return cuda_fail(e, "query classification");
-        if (host[128]) return fail(NPK_ERR_INVALID_CARDS, std::to_string(host[128]) +
-                                   " invalid quer" + (host[128] == 1 ? "y" : "ies") +
-                                   " (card id >= 52, duplicate cards, gap in the board, or players outside 1..10)");
+        if (host[128]) return fail(NPK_ERR_INVALID_CARDS, invalid_queries(host[128], kQueryCauses));
         if (host[(uniform_players - 1) * 6 + uniform_known] != (uint32_t)Q)
             return fail(NPK_ERR_INVALID_ARGUMENT, "queries do not all have the declared uniform shape");
         p.work_counter = reinterpret_cast<unsigned long long*>(ws + kWsCounters) + 1;
@@ -645,12 +726,9 @@ int npk_equity_batch(const uint8_t* hole, const uint8_t* board, const uint8_t* n
     rc = enqueue_mixed(ds, p, hole, board, n_players, Q, ~0ull, ws, s);
     if (rc || !validate) return rc;
     uint32_t bad = 0;
-    e = cudaMemcpyAsync(&bad, ws + kWsInvalid, 4, cudaMemcpyDeviceToHost, s);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-    if (e != cudaSuccess) return cuda_fail(e, "mixed batch");
-    if (bad) return fail(NPK_ERR_INVALID_CARDS, std::to_string(bad) + " invalid quer" + (bad == 1 ? "y" : "ies") +
-                         " (card id >= 52, duplicate cards, gap in the board, or players outside 1..10); their counters "
-                         "are untouched, the other queries have been computed");
+    if ((rc = read_word(ws + kWsInvalid, s, &bad, "mixed batch"))) return rc;
+    if (bad) return fail(NPK_ERR_INVALID_CARDS, invalid_queries(bad, kQueryCauses, "; their counters are untouched, the other "
+                                                                                   "queries have been computed"));
     return NPK_OK;
 }
 
@@ -685,10 +763,9 @@ int npk_equity_batch_status(const void* workspace, void* stream, uint32_t* inval
     const uint8_t* ws = static_cast<const uint8_t*>(workspace);
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     uint32_t v[2] = {0, 0};
-    cudaError_t e = cudaMemcpyAsync(&v[0], ws + kWsInvalid, 4, cudaMemcpyDeviceToHost, s);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(&v[1], ws + kWsSkipped, 4, cudaMemcpyDeviceToHost, s);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-    if (e != cudaSuccess) return cuda_fail(e, "npk_equity_batch_status");
+    if ((rc = read_word(ws + kWsInvalid, s, &v[0], "npk_equity_batch_status")) ||
+        (rc = read_word(ws + kWsSkipped, s, &v[1], "npk_equity_batch_status")))
+        return rc;
     if (invalid) *invalid = v[0];
     if (skipped) *skipped = v[1];
     return NPK_OK;
@@ -701,14 +778,10 @@ int npk_equity_batch_adaptive(const uint8_t* hole, const uint8_t* board, const u
                               int64_t query_offset, int deal_mode, uint32_t flags, uint64_t* wins_strict, uint64_t* ties,
                               uint64_t* win_types, uint64_t* passes, uint64_t* trials, void* workspace, void* stream)
 {
-    // the arguments of the rule first: these errors need no device
-    if (!std::isfinite(max_stderr) || max_stderr <= 0.0)
-        return fail(NPK_ERR_INVALID_ARGUMENT, "stderr must be a finite number > 0");
-    if (min_trials < 1) return fail(NPK_ERR_INVALID_ARGUMENT, "min_trials must be >= 1");
-    if (min_trials > max_trials) return fail(NPK_ERR_INVALID_ARGUMENT, "min_trials must not exceed max_trials");
+    int rc = check_rule(min_trials, max_trials, max_stderr);
+    if (rc) return rc;
     DeviceState* ds;
-    int rc = batch_start(&ds, Q, max_trials, 0);
-    if (rc) return rc == kEmptyBatch ? NPK_OK : rc;
+    if ((rc = batch_start(&ds, Q, max_trials, 0))) return rc == kEmptyBatch ? NPK_OK : rc;
     if (!hole || !board || !n_players || !wins_strict || !ties || !trials || !workspace)
         return fail(NPK_ERR_INVALID_ARGUMENT, "null pointer");
     if ((rc = check_deal_mode(deal_mode))) return rc;
@@ -716,50 +789,16 @@ int npk_equity_batch_adaptive(const uint8_t* hole, const uint8_t* board, const u
     if (!shape_mask) return fail(NPK_ERR_INVALID_ARGUMENT, "empty shape mask");
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     uint8_t* ws = static_cast<uint8_t*>(workspace);
-    uint32_t* hdr = reinterpret_cast<uint32_t*>(ws + adaptive_base(Q));
-    uint8_t* active = ws + adaptive_base(Q) + kAdHeaderBytes;
-    auto* w = reinterpret_cast<unsigned long long*>(wins_strict);
-    auto* t = reinterpret_cast<unsigned long long*>(ties);
-    auto* n_trials = reinterpret_cast<unsigned long long*>(trials);
-    const std::vector<long long> cp = adaptive_checkpoints(min_trials, max_trials);
-    const int cg = (int)std::min<long long>((Q + 255) / 256, 4 * ds->sm_count);
-    const unsigned int retire_grid = (unsigned int)((Q + 255) / 256);
-
-    cudaError_t e = cudaMemsetAsync(hdr, 0, kAdHeaderBytes, s);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(workspace)");
-    adaptive_init_kernel<<<cg, 256, 0, s>>>(hole, board, n_players, Q, shape_mask, w, t,
-                                            reinterpret_cast<unsigned long long*>(win_types),
-                                            reinterpret_cast<unsigned long long*>(passes), n_trials, active, hdr, cp[0],
-                                            ds->sm_count);
-    if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "adaptive_init_kernel launch");
-    if (flags & NPK_FLAG_VALIDATE) {
-        uint32_t bad = 0;
-        e = cudaMemcpyAsync(&bad, hdr + kAdInvalid, 4, cudaMemcpyDeviceToHost, s);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-        if (e != cudaSuccess) return cuda_fail(e, "adaptive batch");
-        if (bad) return fail(NPK_ERR_INVALID_CARDS, std::to_string(bad) + " invalid quer" + (bad == 1 ? "y" : "ies") +
-                             " (card id >= 52, duplicate cards, gap in the board, or players outside 1..10); nothing has "
-                             "been computed");
-    }
-
-    // one round per checkpoint, back to back on the stream: the trials [T_{k-1}, T_k) of the queries still active, then the rule
     npk::EquityParams p;
-    fill_params(p, *ds, hole, board, n_players, Q, cp[0], 0, query_offset, seed, deal_mode, wins_strict, ties, win_types,
+    fill_params(p, *ds, hole, board, n_players, Q, min_trials, 0, query_offset, seed, deal_mode, wins_strict, ties, win_types,
                 passes, reinterpret_cast<uint32_t*>(ws + kWsAbort));
-    p.plan = hdr + kAdPlan;
-    long long done = 0;
-    for (size_t k = 0; k < cp.size(); k++) {
-        if ((rc = clear_workspace(ws, s))) return rc;
-        p.trials = cp[k] - done;
-        p.trial_offset = done;
-        if ((rc = enqueue_mixed(ds, p, hole, board, n_players, Q, ~0ull, ws, s, active))) return rc;
-        const bool final_round = k + 1 == cp.size();
-        adaptive_retire_kernel<<<retire_grid, 256, 0, s>>>(Q, w, t, n_trials, active, hdr, cp[k], max_stderr, final_round ? 1 : 0,
-                                                         final_round ? 0 : cp[k + 1] - cp[k], ds->sm_count, nullptr, 64);
-        if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "adaptive_retire_kernel launch");
-        done = cp[k];
-    }
-    return NPK_OK;
+    // a round classifies the queries still active and runs the all-shapes kernel on them
+    return run_adaptive(*ds, p, ShapeTest{hole, board, n_players, shape_mask}, Q, min_trials, max_trials, max_stderr, trials,
+                        ws, nullptr, 64, (flags & NPK_FLAG_VALIDATE) != 0, "adaptive batch", kQueryCauses,
+                        "; nothing has been computed", s, [&](const uint8_t* active) {
+                            const int rc = clear_workspace(ws, s);
+                            return rc ? rc : enqueue_mixed(ds, p, hole, board, n_players, Q, ~0ull, ws, s, active);
+                        });
 }
 
 namespace {
@@ -1313,38 +1352,15 @@ __global__ void validate_ranges_kernel(const uint8_t* hole, const uint8_t* board
         if (!range_query_valid(hole, board, n_players, ghost, known_opp, n_known, q)) atomicAdd(invalid, 1u);
 }
 
-// The adaptive range call's start: zero the outputs, mark the valid queries active, list them in qindex for the first round
-// and plan it.  Grid: one thread per query (append_queries wants whole warps).
-__global__ void __launch_bounds__(256) ranges_adaptive_init_kernel(const uint8_t* hole, const uint8_t* board,
-                                                                   const uint8_t* n_players, const uint8_t* ghost,
-                                                                   const uint8_t* known_opp, int n_known, long long Q,
-                                                                   unsigned long long* wins, unsigned long long* ties,
-                                                                   unsigned long long* win_types, unsigned long long* passes,
-                                                                   unsigned long long* trials, uint8_t* active, uint32_t* hdr,
-                                                                   int32_t* qindex, long long first_trials, int sm_count)
-{
-    const long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    bool a = false;
-    uint32_t bad = 0;
-    if (q < Q) {
-        wins[q] = 0; ties[q] = 0; trials[q] = 0;
-        if (win_types)
-            for (int i = 0; i < 9; i++) win_types[9 * q + i] = 0;
-        if (passes) passes[q] = 0;
-        a = range_query_valid(hole, board, n_players, ghost, known_opp, n_known, q);
-        active[q] = a ? 1 : 0;
-        bad = !a;
+// The query test of npk_equity_ranges_batch_adaptive (adaptive_init_kernel): 1 = valid, -1 = invalid.
+struct RangeTest {
+    const uint8_t *hole, *board, *n_players, *ghost, *known_opp;
+    int n_known;
+    __device__ int operator()(long long q) const
+    {
+        return range_query_valid(hole, board, n_players, ghost, known_opp, n_known, q) ? 1 : -1;
     }
-    append_queries(hdr + kAdCursor, qindex, a, q);
-    adaptive_count(a ? 1u : 0u, bad, hdr, first_trials, sm_count, 32);
-}
-
-std::string ranges_invalid_message(uint32_t bad)
-{
-    return std::to_string(bad) + " invalid quer" + (bad == 1 ? "y" : "ies") +
-           " (card id >= 52, duplicate cards, gap in the board, ghost card on the board or in a hand, more known opponents "
-           "than opponents, or players outside 1..10)";
-}
+};
 
 int ranges_aborted()
 {
@@ -1430,25 +1446,17 @@ int npk_equity_ranges_known_batch(const uint8_t* hole, const uint8_t* board, con
     p.work_counter = reinterpret_cast<unsigned long long*>(ws + kWsCounters);
 
     const bool validate = (flags & NPK_FLAG_VALIDATE) != 0;
-    cudaError_t e;
     if (validate) {
         const int cg = (int)std::min<long long>((Q + 255) / 256, 4 * ds->sm_count);
         validate_ranges_kernel<<<cg, 256, 0, s>>>(p.hole, board, n_players, ghost, p.known_opp, n_known, Q, ws);
         uint32_t bad = 0;
-        e = cudaMemcpyAsync(&bad, ws + kWsInvalid, 4, cudaMemcpyDeviceToHost, s);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-        if (e != cudaSuccess) return cuda_fail(e, "query validation");
-        if (bad) return fail(NPK_ERR_INVALID_CARDS, ranges_invalid_message(bad));
+        if ((rc = read_word(ws + kWsInvalid, s, &bad, "query validation"))) return rc;
+        if (bad) return fail(NPK_ERR_INVALID_CARDS, invalid_queries(bad, kRangeQueryCauses));
     }
-    if ((rc = launch_ranges(ds, p, deal_mode, Q * chunks, s))) return rc;
-    if (validate) {
-        uint32_t aborted = 0;
-        e = cudaMemcpyAsync(&aborted, ws + kWsAbort, 4, cudaMemcpyDeviceToHost, s);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-        if (e != cudaSuccess) return cuda_fail(e, "equity_ranges_kernel");
-        if (aborted) return ranges_aborted();
-    }
-    return NPK_OK;
+    if ((rc = launch_ranges(ds, p, deal_mode, Q * chunks, s)) || !validate) return rc;
+    uint32_t aborted = 0;
+    if ((rc = read_word(ws + kWsAbort, s, &aborted, "equity_ranges_kernel"))) return rc;
+    return aborted ? ranges_aborted() : NPK_OK;
 }
 
 int npk_equity_ranges_batch_adaptive(const uint8_t* hole, const uint8_t* board, const uint8_t* n_players, const uint8_t* ghost,
@@ -1458,75 +1466,39 @@ int npk_equity_ranges_batch_adaptive(const uint8_t* hole, const uint8_t* board, 
                                      uint64_t* wins_strict, uint64_t* ties, uint64_t* win_types, uint64_t* passes,
                                      uint64_t* trials, void* workspace, void* stream)
 {
-    // the arguments of the rule first: these errors need no device
-    if (!std::isfinite(max_stderr) || max_stderr <= 0.0)
-        return fail(NPK_ERR_INVALID_ARGUMENT, "stderr must be a finite number > 0");
-    if (min_trials < 1) return fail(NPK_ERR_INVALID_ARGUMENT, "min_trials must be >= 1");
-    if (min_trials > max_trials) return fail(NPK_ERR_INVALID_ARGUMENT, "min_trials must not exceed max_trials");
+    int rc = check_rule(min_trials, max_trials, max_stderr);
+    if (rc) return rc;
     DeviceState* ds;
-    int rc = batch_start(&ds, Q, max_trials, 0);
-    if (rc) return rc == kEmptyBatch ? NPK_OK : rc;
+    if ((rc = batch_start(&ds, Q, max_trials, 0))) return rc == kEmptyBatch ? NPK_OK : rc;
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     uint8_t* ws = static_cast<uint8_t*>(workspace);
-    const std::vector<long long> cp = adaptive_checkpoints(min_trials, max_trials);
     npk::EquityParams p;
-    fill_params(p, *ds, hero_allowed ? nullptr : hole, board, n_players, Q, cp[0], 0, query_offset, seed, deal_mode,
+    fill_params(p, *ds, hero_allowed ? nullptr : hole, board, n_players, Q, min_trials, 0, query_offset, seed, deal_mode,
                 wins_strict, ties, win_types, passes, reinterpret_cast<uint32_t*>(ws + kWsAbort), 32);
     if ((rc = range_params(p, hole, board, n_players, ghost, known_opp, n_known, opp_allowed, hero_allowed,
                            wins_strict && ties && trials && workspace, deal_mode)))
         return rc;
-    uint32_t* hdr = reinterpret_cast<uint32_t*>(ws + adaptive_base(Q));
-    uint8_t* active = ws + adaptive_base(Q) + kAdHeaderBytes;
     int32_t* qindex = reinterpret_cast<int32_t*>(ws + kWsIndex);
-    auto* w = reinterpret_cast<unsigned long long*>(wins_strict);
-    auto* t = reinterpret_cast<unsigned long long*>(ties);
-    auto* n_trials = reinterpret_cast<unsigned long long*>(trials);
-    const unsigned int grid = (unsigned int)((Q + 255) / 256);
+    p.qindex = qindex;
+    p.work_counter = reinterpret_cast<unsigned long long*>(ws + kWsCounters);
+    const bool validate = (flags & NPK_FLAG_VALIDATE) != 0;
 
     // the abort flag is cleared once: a round that hits the attempt limit stops every later round at once
     if ((rc = clear_workspace(ws, s))) return rc;
-    cudaError_t e = cudaMemsetAsync(hdr, 0, kAdHeaderBytes, s);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(workspace)");
-    ranges_adaptive_init_kernel<<<grid, 256, 0, s>>>(p.hole, board, n_players, ghost, p.known_opp, n_known, Q, w, t,
-                                                     p.win_types, p.passes, n_trials, active, hdr, qindex, cp[0],
-                                                     ds->sm_count);
-    if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "ranges_adaptive_init_kernel launch");
-    if (flags & NPK_FLAG_VALIDATE) {
-        uint32_t bad = 0;
-        e = cudaMemcpyAsync(&bad, hdr + kAdInvalid, 4, cudaMemcpyDeviceToHost, s);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-        if (e != cudaSuccess) return cuda_fail(e, "query validation");
-        if (bad) return fail(NPK_ERR_INVALID_CARDS, ranges_invalid_message(bad));
-    }
-
-    // one round per checkpoint, back to back on the stream: the trials [T_{k-1}, T_k) of the queries listed in qindex, then
-    // the rule, which lists the queries left and plans the next round
-    p.plan = hdr + kAdPlan;
-    p.qindex = qindex;
-    p.work_counter = reinterpret_cast<unsigned long long*>(ws + kWsCounters);
-    long long done = 0;
-    for (size_t k = 0; k < cp.size(); k++) {
-        e = cudaMemsetAsync(p.work_counter, 0, sizeof(unsigned long long), s);
-        if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(workspace)");
-        p.trials = cp[k] - done;
-        p.trial_offset = done;
-        uint32_t chunk, chunks;                 // the grid: sized for every query, the most this round can have
-        npk::item_plan(Q, p.trials, ds->sm_count, 32, chunk, chunks);
-        if ((rc = launch_ranges(ds, p, deal_mode, Q * (long long)chunks, s))) return rc;
-        const bool final_round = k + 1 == cp.size();
-        adaptive_retire_kernel<<<grid, 256, 0, s>>>(Q, w, t, n_trials, active, hdr, cp[k], max_stderr, final_round ? 1 : 0,
-                                                    final_round ? 0 : cp[k + 1] - cp[k], ds->sm_count, qindex, 32);
-        if ((e = cudaGetLastError()) != cudaSuccess) return cuda_fail(e, "adaptive_retire_kernel launch");
-        done = cp[k];
-    }
-    if (flags & NPK_FLAG_VALIDATE) {
-        uint32_t aborted = 0;
-        e = cudaMemcpyAsync(&aborted, ws + kWsAbort, 4, cudaMemcpyDeviceToHost, s);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-        if (e != cudaSuccess) return cuda_fail(e, "equity_ranges_kernel");
-        if (aborted) return ranges_aborted();
-    }
-    return NPK_OK;
+    // a round runs the range kernel on the queries listed in qindex; there is no re-classification
+    rc = run_adaptive(*ds, p, RangeTest{p.hole, board, n_players, ghost, p.known_opp, n_known}, Q, min_trials, max_trials,
+                      max_stderr, trials, ws, qindex, 32, validate, "query validation", kRangeQueryCauses, "", s,
+                      [&](const uint8_t*) {
+                          const cudaError_t e = cudaMemsetAsync(p.work_counter, 0, sizeof(unsigned long long), s);
+                          if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(workspace)");
+                          uint32_t chunk, chunks;        // the grid: sized for every query, the most this round can have
+                          npk::item_plan(Q, p.trials, ds->sm_count, 32, chunk, chunks);
+                          return launch_ranges(ds, p, deal_mode, Q * (long long)chunks, s);
+                      });
+    if (rc || !validate) return rc;
+    uint32_t aborted = 0;
+    if ((rc = read_word(ws + kWsAbort, s, &aborted, "equity_ranges_kernel"))) return rc;
+    return aborted ? ranges_aborted() : NPK_OK;
 }
 
 int npk_equity_ranges_host(const uint8_t* hole, const uint8_t* board, const uint8_t* n_players, const uint8_t* ghost,

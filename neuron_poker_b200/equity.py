@@ -64,6 +64,11 @@ def _u8(a):
     return a.ctypes.data_as(ctypes.c_void_p)
 
 
+def _seed(seed_value):
+    """A Philox seed as libnpk takes it: the integer modulo 2^64."""
+    return ctypes.c_uint64(int(seed_value) & (2**64 - 1))
+
+
 class _CallBuffers(threading.local):
     """Per-thread result buffer of the one-query calls: allocated once and addressed by integer (a ctypes void* parameter
     accepts an int), so a get_equity call creates no arrays and no ctypes objects."""
@@ -171,12 +176,12 @@ def equity_counts_batch(hole, board, n_players, trials, seed_value=0, deal_mode=
         if Q == 0:
             return PendingCounts(L, None, out)
         ticket = L.npk_equity_host_submit(_u8(hole), _u8(board), _u8(n_players), Q, int(trials),
-                                          ctypes.c_uint64(int(seed_value) & (2**64 - 1)), _DEAL[deal_mode],
+                                          _seed(seed_value), _DEAL[deal_mode],
                                           (1 if win_types else 0) | (2 if passes else 0))
         _lib.check(ticket)
         return PendingCounts(L, ticket, out)
     _lib.check(L.npk_equity_host(_u8(hole), _u8(board), _u8(n_players), Q, int(trials),
-                                 ctypes.c_uint64(int(seed_value) & (2**64 - 1)), _DEAL[deal_mode], _u8(out["wins"]),
+                                 _seed(seed_value), _DEAL[deal_mode], _u8(out["wins"]),
                                  _u8(out["ties"]), _u8(out["win_types"]) if win_types else None,
                                  _u8(out["passes"]) if passes else None))
     return out
@@ -244,10 +249,6 @@ def numpy_montecarlo(my_cards, table_cards_alpha_numeric, iterations, player_amo
     return 100.0 * (r["wins"] + r["ties"]) / int(iterations)
 
 
-def _u64(a):
-    return a.ctypes.data_as(ctypes.c_void_p)
-
-
 def equity_counts_ranges(player_cards, table_cards, players, runs, opponent_range=1, ghost_cards='',
                          deal_mode="reference", seed_value=None, known_opponents=()):
     """One run_montecarlo call with ranges through npk_equity_ranges_host (blocking).
@@ -302,9 +303,9 @@ def equity_counts_ranges(player_cards, table_cards, players, runs, opponent_rang
     known_a = np.array(known, dtype=np.uint8) if n_known else None
     rc = L.npk_equity_ranges_known_host(_u8(hole_a) if hole_a is not None else None, _u8(board_a), _u8(npl),
                                         _u8(ghost_a) if ghost_a is not None else None,
-                                        _u8(known_a) if known_a is not None else None, n_known, 1, runs, _u64(opp_mask),
-                                        _u64(hero_mask) if hero_mask is not None else None,
-                                        ctypes.c_uint64(s & (2**64 - 1)), _DEAL[deal_mode], _u8(out_w), _u8(out_t),
+                                        _u8(known_a) if known_a is not None else None, n_known, 1, runs, _u8(opp_mask),
+                                        _u8(hero_mask) if hero_mask is not None else None,
+                                        _seed(s), _DEAL[deal_mode], _u8(out_w), _u8(out_t),
                                         _u8(out_ty), _u8(out_p))
     _lib.check(rc)
     return {"wins": int(out_w[0]), "ties": int(out_t[0]), "runs": runs, "win_types": [int(x) for x in out_ty],
@@ -359,6 +360,30 @@ class MonteCarlo(object):
 
 
 # ---- batched API on device tensors -----------------------------------------------------------------------------------
+def _batched_call(name, args, dev, Q, win_types, passes, adaptive=False, out=None):
+    """libnpk's batched call `name`(*args, wins, ties, win_types, passes[, trials], workspace, stream) on the current torch
+    stream of `dev`, with a workspace of its own.  Returns the outputs, int64 CUDA tensors viewing the u64 counters.  A fixed
+    call adds to zeroed counters and uses those the caller's `out` already holds; an adaptive call zeroes its outputs itself
+    and adds trials [Q]."""
+    import torch
+    L = _lib.ensure_init(dev.index)
+    fields = [("wins", (Q,), True), ("ties", (Q,), True), ("win_types", (Q, 9), win_types), ("passes", (Q,), passes)]
+    if adaptive:
+        fields.append(("trials", (Q,), True))
+    with torch.cuda.device(dev):
+        out = {} if out is None else out
+        for field, shape, want in fields:
+            if want and field not in out:
+                out[field] = (torch.empty if adaptive and Q else torch.zeros)(shape, dtype=torch.int64, device=dev)
+        ws_bytes = L.npk_equity_adaptive_workspace_bytes if adaptive else L.npk_equity_workspace_bytes
+        ws = torch.empty(int(ws_bytes(Q)), dtype=torch.uint8, device=dev)
+        stream = torch.cuda.current_stream(dev)
+        _lib.check(getattr(L, name)(*args, *(out[field].data_ptr() if want else None for field, _, want in fields),
+                                    ws.data_ptr(), stream.cuda_stream))
+        ws.record_stream(stream)
+    return out
+
+
 def get_equity_ranges_batch(hole, board, n_players, trials, opponent_range=1, hero_range=None, ghost=None, seed_value=0,
                             deal_mode="reference", trial_offset=0, query_offset=0, device=None, validate=True,
                             win_types=False, passes=False, out=None, known_opponents=None):
@@ -368,26 +393,12 @@ def get_equity_ranges_batch(hole, board, n_players, trials, opponent_range=1, he
     opponent_range: fraction or set of class spellings shared by every query; hero_range: None (fixed `hole` [Q,2]) or a
     set of class spellings (the hero is drawn from it every trial, `hole` may be None); ghost: None or [Q,2] uint8
     (0xFF = none).  Returns dict of int64 CUDA tensors like get_equity_batch."""
-    import torch
     dev, a = _range_args(hole, board, n_players, opponent_range, hero_range, ghost, known_opponents, device)
-    Q = a.Q
-    L = _lib.ensure_init(dev.index)
-    with torch.cuda.device(dev):
-        out = {} if out is None else out
-        for name, shape, want in (("wins", (Q,), True), ("ties", (Q,), True), ("win_types", (Q, 9), win_types),
-                                  ("passes", (Q,), passes)):
-            if want and name not in out:
-                out[name] = torch.zeros(shape, dtype=torch.int64, device=dev)
-        ws = torch.empty(int(L.npk_equity_workspace_bytes(Q)), dtype=torch.uint8, device=dev)
-        stream = torch.cuda.current_stream(dev).cuda_stream
-        _lib.check(L.npk_equity_ranges_known_batch(a.hole, a.board, a.n_players, a.ghost, a.known, a.n_known, Q,
-                                             int(trials), _u64(a.opp_mask), a.hero_mask,
-                                             ctypes.c_uint64(int(seed_value) & (2**64 - 1)), int(trial_offset),
-                                             int(query_offset), _DEAL[deal_mode],
-                                             _lib.NPK_FLAG_VALIDATE if validate else 0, out["wins"].data_ptr(),
-                                             out["ties"].data_ptr(), out["win_types"].data_ptr() if win_types else None,
-                                             out["passes"].data_ptr() if passes else None, ws.data_ptr(), stream))
-        ws.record_stream(torch.cuda.current_stream(dev))
+    out = _batched_call("npk_equity_ranges_known_batch",
+                        (a.hole, a.board, a.n_players, a.ghost, a.known, a.n_known, a.Q, int(trials), _u8(a.opp_mask),
+                         a.hero_mask, _seed(seed_value), int(trial_offset), int(query_offset), _DEAL[deal_mode],
+                         _lib.NPK_FLAG_VALIDATE if validate else 0),
+                        dev, a.Q, win_types, passes, out=out)
     out["trials"] = int(trials)
     return out
 
@@ -416,7 +427,7 @@ def _range_args(hole, board, n_players, opponent_range, hero_range, ghost, known
     a.board, a.n_players = a.t_board.data_ptr(), a.t_players.data_ptr()
     a.ghost = a.t_ghost.data_ptr() if a.t_ghost is not None else None
     a.known = a.t_known.data_ptr() if a.n_known else None
-    a.hero_mask = _u64(a.hero_mask_array) if a.hero_mask_array is not None else None
+    a.hero_mask = _u8(a.hero_mask_array) if a.hero_mask_array is not None else None
     return dev, a
 
 
@@ -465,39 +476,23 @@ def get_equity_batch(hole, board, n_players, trials, seed_value=0, deal_mode="un
     Returns dict of int64 CUDA tensors: wins [Q], ties [Q] (+ win_types [Q,9], passes [Q]); the counters are u64 on
     the device and viewed as int64.  `out` may hold preallocated zeroed tensors to accumulate into.
     """
-    import torch
     dev = _resolve_device(device)
     hole = _as_cuda_u8(hole, dev, (2,))
     board = _as_cuda_u8(board, dev, (5,))
     n_players = _as_cuda_u8(n_players, dev, ())
     Q = hole.shape[0]
-    L = _lib.ensure_init(dev.index)
-    with torch.cuda.device(dev):
-        out = {} if out is None else out
-        for name, shape, want in (("wins", (Q,), True), ("ties", (Q,), True), ("win_types", (Q, 9), win_types),
-                                  ("passes", (Q,), passes)):
-            if want and name not in out:
-                out[name] = torch.zeros(shape, dtype=torch.int64, device=dev)
-        ws = torch.empty(int(L.npk_equity_workspace_bytes(Q)), dtype=torch.uint8, device=dev)
+    queries = (hole.data_ptr(), board.data_ptr(), n_players.data_ptr(), Q, int(trials))
+    if shapes is not None and uniform_shape is None:
+        out = _batched_call("npk_equity_batch_async",
+                            queries + (ctypes.c_uint64(int(shapes)), _seed(seed_value), int(trial_offset), int(query_offset),
+                                       _DEAL[deal_mode]),
+                            dev, Q, win_types, passes, out=out)
+    else:
         up, uk = (-1, -1) if uniform_shape is None else (int(uniform_shape[0]), int(uniform_shape[1]))
-        stream = torch.cuda.current_stream(dev).cuda_stream
-        if shapes is not None and uniform_shape is None:
-            _lib.check(L.npk_equity_batch_async(hole.data_ptr(), board.data_ptr(), n_players.data_ptr(), Q, int(trials),
-                                                ctypes.c_uint64(int(shapes)), ctypes.c_uint64(int(seed_value) & (2**64 - 1)),
-                                                int(trial_offset), int(query_offset), _DEAL[deal_mode],
-                                                out["wins"].data_ptr(), out["ties"].data_ptr(),
-                                                out["win_types"].data_ptr() if win_types else None,
-                                                out["passes"].data_ptr() if passes else None, ws.data_ptr(), stream))
-            ws.record_stream(torch.cuda.current_stream(dev))
-            out["trials"] = int(trials)
-            return out
-        _lib.check(L.npk_equity_batch(hole.data_ptr(), board.data_ptr(), n_players.data_ptr(), Q, int(trials), up, uk,
-                                      ctypes.c_uint64(int(seed_value) & (2**64 - 1)), int(trial_offset),
-                                      int(query_offset), _DEAL[deal_mode], _lib.NPK_FLAG_VALIDATE if validate else 0,
-                                      out["wins"].data_ptr(), out["ties"].data_ptr(),
-                                      out["win_types"].data_ptr() if win_types else None,
-                                      out["passes"].data_ptr() if passes else None, ws.data_ptr(), stream))
-        ws.record_stream(torch.cuda.current_stream(dev))
+        out = _batched_call("npk_equity_batch",
+                            queries + (up, uk, _seed(seed_value), int(trial_offset), int(query_offset), _DEAL[deal_mode],
+                                       _lib.NPK_FLAG_VALIDATE if validate else 0),
+                            dev, Q, win_types, passes, out=out)
     out["trials"] = int(trials)
     return out
 
@@ -531,32 +526,17 @@ def get_equity_batch_adaptive(hole, board, n_players, max_trials, stderr, min_tr
     are exactly those of get_equity_batch(trials=T_stop) with the same seed and query_offset, whatever else is in the batch.
     Returns the dict of get_equity_batch, except that `trials` is an int64 CUDA tensor [Q] holding every query's T_stop
     (0 for a query outside `shapes`, or an invalid one when validate=False)."""
-    import torch
     dev = _resolve_device(device)
     hole = _as_cuda_u8(hole, dev, (2,))
     board = _as_cuda_u8(board, dev, (5,))
     n_players = _as_cuda_u8(n_players, dev, ())
     Q = hole.shape[0]
-    L = _lib.ensure_init(dev.index)
-    with torch.cuda.device(dev):
-        out = {}
-        for name, shape, want in (("wins", (Q,), True), ("ties", (Q,), True), ("win_types", (Q, 9), win_types),
-                                  ("passes", (Q,), passes), ("trials", (Q,), True)):
-            if want:
-                out[name] = (torch.empty if Q else torch.zeros)(shape, dtype=torch.int64, device=dev)   # zeroed by the call
-        ws = torch.empty(int(L.npk_equity_adaptive_workspace_bytes(Q)), dtype=torch.uint8, device=dev)
-        stream = torch.cuda.current_stream(dev).cuda_stream
-        _lib.check(L.npk_equity_batch_adaptive(hole.data_ptr(), board.data_ptr(), n_players.data_ptr(), Q, int(min_trials),
-                                               int(max_trials), ctypes.c_double(float(stderr)),
-                                               ctypes.c_uint64(ALL_SHAPES if shapes is None else int(shapes) & ALL_SHAPES),
-                                               ctypes.c_uint64(int(seed_value) & (2**64 - 1)), int(query_offset),
-                                               _DEAL[deal_mode], _lib.NPK_FLAG_VALIDATE if validate else 0,
-                                               out["wins"].data_ptr(), out["ties"].data_ptr(),
-                                               out["win_types"].data_ptr() if win_types else None,
-                                               out["passes"].data_ptr() if passes else None, out["trials"].data_ptr(),
-                                               ws.data_ptr(), stream))
-        ws.record_stream(torch.cuda.current_stream(dev))
-    return out
+    return _batched_call("npk_equity_batch_adaptive",
+                         (hole.data_ptr(), board.data_ptr(), n_players.data_ptr(), Q, int(min_trials), int(max_trials),
+                          ctypes.c_double(float(stderr)),
+                          ctypes.c_uint64(ALL_SHAPES if shapes is None else int(shapes) & ALL_SHAPES), _seed(seed_value),
+                          int(query_offset), _DEAL[deal_mode], _lib.NPK_FLAG_VALIDATE if validate else 0),
+                         dev, Q, win_types, passes, adaptive=True)
 
 
 def get_equity_ranges_batch_adaptive(hole, board, n_players, max_trials, stderr, min_trials=256, opponent_range=1,
@@ -569,26 +549,9 @@ def get_equity_ranges_batch_adaptive(hole, board, n_players, max_trials, stderr,
     same seed, query_offset, ranges, ghost cards, known hands and sampler (passes=True: the generic kernel, else the pair-list
     sampler).  Returns the dict of get_equity_batch_adaptive: `trials` is an int64 CUDA tensor [Q] of every query's T_stop
     (0 for an invalid query when validate=False)."""
-    import torch
     dev, a = _range_args(hole, board, n_players, opponent_range, hero_range, ghost, known_opponents, device)
-    Q = a.Q
-    L = _lib.ensure_init(dev.index)
-    with torch.cuda.device(dev):
-        out = {}
-        for name, shape, want in (("wins", (Q,), True), ("ties", (Q,), True), ("win_types", (Q, 9), win_types),
-                                  ("passes", (Q,), passes), ("trials", (Q,), True)):
-            if want:
-                out[name] = (torch.empty if Q else torch.zeros)(shape, dtype=torch.int64, device=dev)   # zeroed by the call
-        ws = torch.empty(int(L.npk_equity_adaptive_workspace_bytes(Q)), dtype=torch.uint8, device=dev)
-        stream = torch.cuda.current_stream(dev).cuda_stream
-        _lib.check(L.npk_equity_ranges_batch_adaptive(a.hole, a.board, a.n_players, a.ghost, a.known, a.n_known, Q,
-                                                      int(min_trials), int(max_trials), ctypes.c_double(float(stderr)),
-                                                      _u64(a.opp_mask), a.hero_mask,
-                                                      ctypes.c_uint64(int(seed_value) & (2**64 - 1)), int(query_offset),
-                                                      _DEAL[deal_mode], _lib.NPK_FLAG_VALIDATE if validate else 0,
-                                                      out["wins"].data_ptr(), out["ties"].data_ptr(),
-                                                      out["win_types"].data_ptr() if win_types else None,
-                                                      out["passes"].data_ptr() if passes else None, out["trials"].data_ptr(),
-                                                      ws.data_ptr(), stream))
-        ws.record_stream(torch.cuda.current_stream(dev))
-    return out
+    return _batched_call("npk_equity_ranges_batch_adaptive",
+                         (a.hole, a.board, a.n_players, a.ghost, a.known, a.n_known, a.Q, int(min_trials), int(max_trials),
+                          ctypes.c_double(float(stderr)), _u8(a.opp_mask), a.hero_mask, _seed(seed_value),
+                          int(query_offset), _DEAL[deal_mode], _lib.NPK_FLAG_VALIDATE if validate else 0),
+                         dev, a.Q, win_types, passes, adaptive=True)
