@@ -17,6 +17,7 @@
  *   npk_rank7_batch     _calc_score ordering                      tools/hand_evaluator.py:27-119
  *   npk_showdown_batch  get_winner / eval_best_hand               tools/hand_evaluator.py:9-24 (used by gym_env/env.py:576-593)
  *   npk_enum_batch      no counterpart (the reference only samples); exact enumeration used for bit-exact checks
+ *   npk_enum_dealer_batch  the exact value get_equity (:401-406) converges to, under the reference's dealer
  *   npk_showdown_equity_batch  run_montecarlo with every hand in player_card_list known (:132-163, ghost cards :206-208),
  *                       computed exactly (every board completion) and for every player, split pots included
  *
@@ -310,6 +311,23 @@ int npk_rank7_colex(int64_t first, int64_t count, uint16_t* ranks, void* stream)
  * reports it as NPK_ERR_INVALID_ARGUMENT instead). */
 int npk_enum_batch(const uint8_t* hole, const uint8_t* board, const uint8_t* n_players, int64_t Q, uint64_t* win,
                    uint64_t* tie, uint64_t* lose, uint32_t flags, void* stream);
+
+/* Exact enumeration under a chosen dealer: the shapes, validation and outputs of npk_enum_batch, which is this call with
+ * NPK_DEAL_UNIFORM.  A deal_mode other than NPK_DEAL_UNIFORM / NPK_DEAL_REFERENCE is NPK_ERR_INVALID_ARGUMENT before the
+ * device is touched.
+ * NPK_DEAL_REFERENCE weights every deal by how often the reference's dealer (montecarlo_python.py:165-189) makes it, so
+ * that the counts are integers.  R = the n unseen cards in ascending id order, m = missing board cards.
+ *   opponent hand, slots a < b of R: weight w = 2 - [b == a + 1].  The dealer draws i1 in [0,n), i2 in [0,n-1), redraws
+ *       while i1 == i2 and pops i1, then i2 from the shortened list: all (n-1)^2 accepted pairs are equally likely and the
+ *       second card is never the successor of the first.  sum w = (n-1)^2.
+ *   board: each card is pop(randint(0, len-1)), so the last card of the list is never dealt; every m-subset of R minus
+ *       the opponents' cards minus its highest card has weight 1.
+ *   three players (complete board): the ordered pair of hands has weight w(o1) * w(o2 | o1), with the adjacency of o2
+ *       tested in R minus o1's cards.
+ * Totals win + tie + lose: heads-up (n-1)^2 C(n-3, m); three players (n-1)^2 (n-3)^2.  The value get_equity converges to
+ * with this dealer (ties count as wins) = (win + tie) / (win + tie + lose). */
+int npk_enum_dealer_batch(const uint8_t* hole, const uint8_t* board, const uint8_t* n_players, int64_t Q, int deal_mode,
+                          uint64_t* win, uint64_t* tie, uint64_t* lose, uint32_t flags, void* stream);
 
 /* Batched showdown: holes [N,maxp,2], n_players [N] (1..maxp), board [N,5] complete.  winner [N] = first index among the
  * best hands (hand_evaluator.py:23 stable sort), wtype [N] = its hand type 0..8, ranks [N,maxp] or NULL. */

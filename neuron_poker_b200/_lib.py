@@ -79,6 +79,7 @@ def lib():
                 L.npk_rank7_batch.argtypes = [u8, i64, u16, ctypes.c_uint32, vp]
                 L.npk_rank7_colex.argtypes = [i64, i64, u16, vp]
                 L.npk_enum_batch.argtypes = [u8, u8, u8, i64, u64, u64, u64, ctypes.c_uint32, vp]
+                L.npk_enum_dealer_batch.argtypes = [u8, u8, u8, i64, i32, u64, u64, u64, ctypes.c_uint32, vp]
                 L.npk_showdown_batch.argtypes = [u8, u8, u8, i64, i32, vp, u8, u16, ctypes.c_uint32, vp]
                 L.npk_showdown_equity_workspace_bytes.argtypes = [i64]
                 L.npk_showdown_equity_workspace_bytes.restype = i64

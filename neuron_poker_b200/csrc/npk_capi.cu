@@ -1657,8 +1657,16 @@ int npk_rank7_colex(int64_t first, int64_t count, uint16_t* ranks, void* stream)
 int npk_enum_batch(const uint8_t* hole, const uint8_t* board, const uint8_t* n_players, int64_t Q, uint64_t* win,
                    uint64_t* tie, uint64_t* lose, uint32_t flags, void* stream)
 {
+    return npk_enum_dealer_batch(hole, board, n_players, Q, NPK_DEAL_UNIFORM, win, tie, lose, flags, stream);
+}
+
+int npk_enum_dealer_batch(const uint8_t* hole, const uint8_t* board, const uint8_t* n_players, int64_t Q, int deal_mode,
+                          uint64_t* win, uint64_t* tie, uint64_t* lose, uint32_t flags, void* stream)
+{
+    int rc = check_deal_mode(deal_mode);
+    if (rc) return rc;
     DeviceState* ds;
-    int rc = current_state(&ds);
+    rc = current_state(&ds);
     if (rc) return rc;
     if (Q <= 0) return Q == 0 ? NPK_OK : fail(NPK_ERR_INVALID_ARGUMENT, "negative Q");
     if (!hole || !board || !n_players || !win || !tie || !lose) return fail(NPK_ERR_INVALID_ARGUMENT, "null pointer");
@@ -1674,7 +1682,7 @@ int npk_enum_batch(const uint8_t* hole, const uint8_t* board, const uint8_t* n_p
     p.tie = reinterpret_cast<unsigned long long*>(tie);
     p.lose = reinterpret_cast<unsigned long long*>(lose);
     const int grid = (int)std::min<long long>(Q, ds->sm_count);
-    cudaError_t e = npk::launch_enum(p, grid, static_cast<cudaStream_t>(stream));
+    cudaError_t e = npk::launch_enum(p, deal_mode, grid, static_cast<cudaStream_t>(stream));
     return e == cudaSuccess ? NPK_OK : cuda_fail(e, "enum_kernel launch");
 }
 

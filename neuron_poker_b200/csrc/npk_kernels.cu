@@ -9,7 +9,8 @@
 //                                       loop played literally; the pair-list sampler lives in npk_ranges.cu, the persistent
 //                                       all-shapes kernel for mixed batches in npk_mixed.cu, the per-trial code in npk_mc.cuh)
 //   rank7_kernel / rank7_colex      K2  batched 7-card rank ids (hand_evaluator.py:27-119 `_calc_score` ordering)
-//   enum_headsup_kernel             K3  exact heads-up enumeration of opponents and missing board cards
+//   enum_kernel<REF>                K3  exact enumeration of opponents and missing board cards, uniform dealing (REF = 0)
+//                                       or weighted by the reference's dealer (REF = 1, montecarlo_python.py:165-189)
 //   showdown_kernel                 K4  batched get_winner (hand_evaluator.py:9-17)
 //
 // Everything is integer work on 32-bit lanes: no tensor cores, no floating point.  Two trials per lane and iteration; the rank
@@ -363,6 +364,16 @@ __global__ void __launch_bounds__(kAuxThreads, 1) rank7_colex_kernel(const Devic
 // and the hero's value once, and its lanes walk over the opponent pairs -- per matchup one 3-input add, the table
 // gathers and the flush test, exactly the per-player work of the Monte-Carlo kernels.  The list of pairs (a < b) of
 // unseen cards is built once per query in shared memory and doubles as the list of two-card completions.
+//
+// REF = 1 counts what the reference's dealer deals (montecarlo_python.py:165-189) instead of every deal once.  Slots are
+// positions in the unseen cards R (ascending ids, n of them).  An opponent's hand, slots a < b, comes with weight
+// w = 2 - [b == a + 1]: of the (n-1)^2 equally likely accepted index pairs, (i1, i2) deals slot i2 second when i2 < i1 and
+// slot i2 + 1 when i2 > i1, so the second card is never the successor of the first.  Board cards are popped from indices
+// 0..len-2, so the highest slot left after the opponents' cards is never dealt: a completion holding that excluded slot
+// counts 0, every other completion 1.  With a second opponent (complete board only) its weight is tested in the list
+// without the first opponent's cards: a2 < b2 are adjacent when every slot strictly between them is one of those.
+// Totals: heads-up (n-1)^2 C(n-3, missing), three players (n-1)^2 (n-3)^2.
+template <int REF>
 __global__ void __launch_bounds__(kAuxThreads, 1) enum_kernel(const EnumParams p)
 {
     extern __shared__ __align__(128) uint8_t smem[];
@@ -439,9 +450,16 @@ __global__ void __launch_bounds__(kAuxThreads, 1) enum_kernel(const EnumParams p
                         const uint32_t pr = s_pair[ip];
                         const int a = pr & 255, b = pr >> 8;
                         if (a == c0 || a == c1 || b == c0 || b == c1) continue;
+                        uint32_t w = 1;
+                        if (REF) {
+                            const int x = b != n - 1 ? n - 1 : (a != n - 2 ? n - 2 : n - 3);   // the pair's excluded slot
+                            if (x == c0 || x == c1) continue;
+                            w = 2 - (b == a + 1);
+                        }
                         const uint32_t d0 = s_deck[a], d1 = s_deck[b];
                         const uint32_t ov = eval_player(st, bsum + d0 + d1, bfield | flush_bit(d0, bf.fsx) | flush_bit(d1, bf.fsx), bf.thr);
-                        win += hv > ov; tie += hv == ov; lose += hv < ov;
+                        if (REF) { win += hv > ov ? w : 0u; tie += hv == ov ? w : 0u; lose += hv < ov ? w : 0u; }
+                        else { win += hv > ov; tie += hv == ov; lose += hv < ov; }
                     }
                 }
             }
@@ -468,13 +486,18 @@ __global__ void __launch_bounds__(kAuxThreads, 1) enum_kernel(const EnumParams p
                 }
                 bool clash = false;
                 for (int k = 0; k < missing; k++) clash |= (comp[k] == a) | (comp[k] == b);
+                if (REF) {
+                    const int x = b != n - 1 ? n - 1 : (a != n - 2 ? n - 2 : n - 3);
+                    for (int k = 0; k < missing; k++) clash |= comp[k] == x;
+                }
                 if (clash) continue;
                 uint32_t h7[7], o7[7];
                 h7[0] = hd[0]; h7[1] = hd[1]; o7[0] = s_deck[a]; o7[1] = s_deck[b];
                 for (int k = 0; k < known; k++) { h7[2 + k] = bd[k]; o7[2 + k] = bd[k]; }
                 for (int k = 0; k < missing; k++) { h7[2 + known + k] = s_deck[comp[k]]; o7[2 + known + k] = h7[2 + known + k]; }
                 const uint32_t hv = eval7_desc(st, h7), ov = eval7_desc(st, o7);
-                win += hv > ov; tie += hv == ov; lose += hv < ov;
+                if (REF) { const uint32_t wt = 2 - (b == a + 1); win += hv > ov ? wt : 0u; tie += hv == ov ? wt : 0u; lose += hv < ov ? wt : 0u; }
+                else { win += hv > ov; tie += hv == ov; lose += hv < ov; }
             }
         } else if (nopp == 2 && known == 5) {
             uint32_t h7[7] = {hd[0], hd[1], bd[0], bd[1], bd[2], bd[3], bd[4]};
@@ -490,12 +513,20 @@ __global__ void __launch_bounds__(kAuxThreads, 1) enum_kernel(const EnumParams p
                 const uint32_t p1 = s_pair[i1];
                 const int a1 = p1 & 255, b1 = p1 >> 8;
                 const uint32_t v1 = s_pairval[i1];
+                const uint32_t w1 = 2 - (b1 == a1 + 1);
                 for (int i2 = lane; i2 < npairs; i2 += 32) {
                     const uint32_t p2 = s_pair[i2];
                     const int a2 = p2 & 255, b2 = p2 >> 8;
                     if (a1 == a2 || a1 == b2 || b1 == a2 || b1 == b2) continue;
                     const uint32_t best = max(v1, (uint32_t)s_pairval[i2]);
-                    win += hv > best; tie += hv == best; lose += hv < best;
+                    if (REF) {
+                        // slots of the first hand strictly between a2 and b2 are gone from the second opponent's list
+                        const int between = (a2 < a1 && a1 < b2) + (a2 < b1 && b1 < b2);
+                        const uint32_t w = w1 * (2 - (b2 - a2 - 1 == between));
+                        win += hv > best ? w : 0u; tie += hv == best ? w : 0u; lose += hv < best ? w : 0u;
+                    } else {
+                        win += hv > best; tie += hv == best; lose += hv < best;
+                    }
                 }
             }
         }
@@ -700,12 +731,13 @@ cudaError_t launch_rank7_colex(const DeviceTables& t, long long first, long long
     return cudaGetLastError();
 }
 
-cudaError_t launch_enum(const EnumParams& p, int grid, cudaStream_t s)
+cudaError_t launch_enum(const EnumParams& p, int deal_mode, int grid, cudaStream_t s)
 {
     size_t smem = aux_smem(p.tables);
-    cudaError_t e = cudaFuncSetAttribute(enum_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    auto k = deal_mode == 1 ? enum_kernel<1> : enum_kernel<0>;
+    cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
-    enum_kernel<<<grid, kAuxThreads, smem, s>>>(p);
+    k<<<grid, kAuxThreads, smem, s>>>(p);
     return cudaGetLastError();
 }
 

@@ -184,7 +184,7 @@ cudaError_t launch_equity_ranges(int deal_mode, const EquityParams& p, int grid,
 cudaError_t launch_equity_ranges_fast(int deal_mode, const EquityParams& p, int grid, cudaStream_t s);
 cudaError_t launch_rank7(const DeviceTables& t, const uint8_t* cards, long long n, uint16_t* out, int grid, cudaStream_t s);
 cudaError_t launch_rank7_colex(const DeviceTables& t, long long first, long long count, uint16_t* out, int grid, cudaStream_t s);
-cudaError_t launch_enum(const EnumParams& p, int grid, cudaStream_t s);
+cudaError_t launch_enum(const EnumParams& p, int deal_mode, int grid, cudaStream_t s);   // deal_mode: NPK_DEAL_*
 cudaError_t launch_showdown(const DeviceTables& t, const uint8_t* holes, const uint8_t* n_players, const uint8_t* board,
                             long long n, int maxp, int32_t* winner, uint8_t* wtype, uint16_t* ranks, int grid, cudaStream_t s);
 cudaError_t launch_int_peak(int variant, uint32_t* out, int iters, int grid, cudaStream_t s);

@@ -8,7 +8,7 @@ import ctypes
 import numpy as np
 
 from . import _lib
-from .cards import HAND_TYPES, NO_CARD, card_ids
+from .cards import HAND_TYPES, NO_CARD, card_ids, encode_query
 
 N_HANDS_7 = 133784560  # C(52,7)
 
@@ -105,9 +105,12 @@ def eval_best_hand(hands):
     return hands[best], HAND_TYPES[ty]
 
 
-def enumerate_equity(hole, board, n_players=None, device=None, validate=None):
+def enumerate_equity(hole, board, n_players=None, device=None, validate=None, deal_mode="uniform"):
     """Exact enumeration (no sampling): hole [Q,2], board [Q,5] with 0xFF padding, n_players [Q] (2, or 3 on a complete
-    board).  Returns int64 CUDA tensors (win, tie, lose) of hero-strictly-best / tied / beaten counts."""
+    board).  Returns int64 CUDA tensors (win, tie, lose) of hero-strictly-best / tied / beaten counts.
+    deal_mode "uniform" counts every deal once; "reference" weights every deal by how often the reference's dealer makes it
+    (include/npk.h, npk_enum_dealer_batch), so that (win + tie) / (win + tie + lose) is the value get_equity converges to."""
+    from .equity import _DEAL
     torch = _torch()
     dev = _dev(device)
     flags = _want_check(hole, validate)
@@ -125,9 +128,29 @@ def enumerate_equity(hole, board, n_players=None, device=None, validate=None):
     tie = torch.zeros(Q, dtype=torch.int64, device=dev)
     lose = torch.zeros(Q, dtype=torch.int64, device=dev)
     with torch.cuda.device(dev):
-        _lib.check(L.npk_enum_batch(hole.data_ptr(), board.data_ptr(), n_players.data_ptr(), Q, win.data_ptr(),
-                                    tie.data_ptr(), lose.data_ptr(), flags, torch.cuda.current_stream(dev).cuda_stream))
+        _lib.check(L.npk_enum_dealer_batch(hole.data_ptr(), board.data_ptr(), n_players.data_ptr(), Q,
+                                           _DEAL.get(deal_mode, -1), win.data_ptr(), tie.data_ptr(), lose.data_ptr(), flags,
+                                           torch.cuda.current_stream(dev).cuda_stream))
     return win, tie, lose
+
+
+def exact_equity(player_cards, table_cards, players, deal_mode="reference"):
+    """The exact value get_equity(player_cards, table_cards, players, runs) converges to as runs grows: every deal of the
+    opponents' hands and the missing table cards enumerated on the GPU, weighted by how often the reference's dealer makes
+    it (ties count as wins).  deal_mode="uniform" gives the value under uniform dealing instead.
+    Enumerated shapes: two players with 0..5 table cards, three players with five.  Invalid or repeated cards raise
+    ValueError, like get_equity; so does any other shape."""
+    hole, board = encode_query(player_cards, table_cards)
+    players, known = int(players), len(card_ids(table_cards))
+    if not (players == 2 or (players == 3 and known == 5)):
+        raise ValueError("exact_equity enumerates two players with 0..5 table cards or three players with five table cards, "
+                         "not %d players with %d" % (players, known))
+    if deal_mode not in ("uniform", "reference"):
+        raise ValueError("deal_mode must be 'uniform' or 'reference'")
+    w, t, l = enumerate_equity(hole[None], board[None], np.array([players], dtype=np.uint8), deal_mode=deal_mode,
+                               validate=True)
+    w, t, l = int(w[0]), int(t[0]), int(l[0])
+    return (w + t) / (w + t + l)
 
 
 SHARE_UNIT = 2520   # NPK_SHARE_UNIT: lcm(1..10), a pot split k ways gives each of the k players 2520 / k
