@@ -20,6 +20,8 @@
  *   npk_enum_dealer_batch  the exact value get_equity (:401-406) converges to, under the reference's dealer
  *   npk_showdown_equity_batch  run_montecarlo with every hand in player_card_list known (:132-163, ghost cards :206-208),
  *                       computed exactly (every board completion) and for every player, split pots included
+ *   npk_exact_equity_batch  run_montecarlo with one or two unknown opponents beside known hands and ghost cards, computed
+ *                       exactly under either dealer: the value it converges to
  *
  * Cards are bytes: id = 4*rank + suit with ranks "23456789TJQKA" and suits "CDHS" -- the order of
  * MonteCarlo.create_card_deck (tools/montecarlo_python.py:114-119).  0xFF marks "no card" in board arrays.
@@ -357,6 +359,34 @@ int64_t npk_showdown_equity_workspace_bytes(int64_t N);
 int npk_showdown_equity_batch(const uint8_t* holes, const uint8_t* n_players, const uint8_t* board, const uint64_t* dead,
                               int64_t N, int maxp, int deal_mode, uint32_t flags, uint64_t* win, uint64_t* tie, uint64_t* share,
                               uint64_t* completions, void* workspace, void* stream);
+
+/*
+ * Exact equity against one or two UNKNOWN opponents, with known opponent hands and dead cards: run_montecarlo with entries of
+ * player_card_list beyond the hero known (montecarlo_python.py:132-163) and ghost cards (:206-208), without sampling.
+ *   holes [N,maxk,2]  the hero, then the known opponents (maxk 1..8)   n_known [N] hands of `holes` in the spot, hero included
+ *   n_random [N] unknown opponents k (1..2), n_known + k <= 10        board [N,5] 0xFF padding
+ *   dead [N] or NULL  one bit per card id removed from the deck
+ * R = the unseen cards (52 minus hands, board and dead cards) in ascending id order, n = |R|, m = missing board cards.  Outputs
+ * (u64, OVERWRITTEN) are counts from the hero's side: win (hero strictly best of all players), tie (hero tied for best), lose.
+ * (win + tie) / (win + tie + lose) is run_montecarlo's equity, where ties count as wins.
+ *   NPK_DEAL_UNIFORM    every ordered tuple of disjoint unknown hands counts once, and so does every m-subset of what is left:
+ *                       totals C(n,2) C(n-2,m) for k = 1, C(n,2) C(n-2,2) C(n-4,m) for k = 2.
+ *   NPK_DEAL_REFERENCE  the weights of npk_enum_dealer_batch, applied to R (the list left after the known hands and the dead
+ *                       cards): the first unknown hand, slots a < b, has weight 2 - [b == a + 1]; the second 2 - [every slot
+ *                       strictly between a2 and b2 belongs to the first hand]; a completion holding x = max(R minus the unknown
+ *                       hands' cards) counts 0.  Totals (n-1)^2 C(n-3,m) for k = 1, (n-1)^2 (n-3)^2 C(n-5,m) for k = 2.
+ * With no known opponent and k = 1, or k = 2 on a complete board, the counts equal npk_enum_dealer_batch's in both modes.
+ * A deal_mode other than NPK_DEAL_UNIFORM / NPK_DEAL_REFERENCE or maxk outside 1..8 is NPK_ERR_INVALID_ARGUMENT before the device
+ * is touched.  workspace: npk_exact_equity_workspace_bytes(N) bytes, private to the call until it completes.  Asynchronous and
+ * free of host round trips (graph-capturable) unless NPK_FLAG_VALIDATE is set: NPK_ERR_INVALID_CARDS for an id >= 52, a card twice
+ * across hands, board and dead mask, a gap in the board or a dead bit >= 52; NPK_ERR_INVALID_ARGUMENT for n_known outside
+ * 1..maxk, n_random outside 1..2, more than 10 players, or too few cards: n < 2k + m, or n < 2k + m + 1 under REFERENCE when
+ * m >= 1.  Without the flag such a spot is memory-safe and gets zero counters.
+ */
+int64_t npk_exact_equity_workspace_bytes(int64_t N);
+int npk_exact_equity_batch(const uint8_t* holes, const uint8_t* n_known, const uint8_t* n_random, const uint8_t* board,
+                           const uint64_t* dead, int64_t N, int maxk, int deal_mode, uint32_t flags, uint64_t* win, uint64_t* tie,
+                           uint64_t* lose, void* workspace, void* stream);
 
 /* Integer-issue microbenchmark on the current device (the roofline denominator of the Monte-Carlo kernel):
  * variant 0 = LOP3 chains (alu pipe), 1 = IMAD chains (fma pipe), 2 = both interleaved.  Reports executed

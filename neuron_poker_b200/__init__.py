@@ -8,8 +8,9 @@ Public surface = the reference's own plugin interface for this path:
     get_winner(player_hands, table_cards), eval_best_hand(hands)    tools/hand_evaluator.py:9, :20
 plus batched entry points on CUDA tensors (get_equity_batch, get_equity_batch_adaptive -- each query to a target standard
 error --, get_equity_ranges_batch, get_equity_ranges_batch_adaptive, rank7, showdown, enumerate_equity,
-showdown_equity_batch), the exact equity of known hands (showdown_equity), the exact value get_equity converges to
-(exact_equity)
+showdown_equity_batch, exact_equity_batch), the exact equity of known hands (showdown_equity), the exact value get_equity
+converges to (exact_equity), the exact value run_montecarlo converges to against one or two unknown opponents beside known
+hands and ghost cards (exact_equity_counts)
 and the vectorised environment (holdem.HoldemTables: gym_env/env.py::HoldemTable for N tables on the GPU).
 All compute runs in libnpk.so's CUDA kernels; importing this package does not import torch.
 """
@@ -19,7 +20,8 @@ from .equity import (DEAL_REFERENCE, DEAL_UNIFORM, MonteCarlo, equity_counts, eq
                      get_equity_ranges_batch, get_equity_ranges_batch_adaptive, montecarlo,
                      numpy_montecarlo, resident, seed)
 from . import dist, holdem, ranges  # noqa: F401
-from .evaluator import (enumerate_equity, eval_best_hand, exact_equity, get_winner, host_rank7, host_tables, rank7,  # noqa: F401
-                        rank7_colex, showdown, showdown_equity, showdown_equity_batch)
+from .evaluator import (enumerate_equity, eval_best_hand, exact_equity, exact_equity_batch, exact_equity_counts,  # noqa: F401
+                        get_winner, host_rank7, host_tables, rank7, rank7_colex, showdown, showdown_equity,
+                        showdown_equity_batch)
 
 __version__ = "0.1.0"

@@ -1561,9 +1561,11 @@ int npk_equity_ranges_known_host(const uint8_t* hole, const uint8_t* board, cons
 // at the end of the board only) and the shape must be one enum_kernel implements.
 // mode 2 (npk_showdown_equity_batch): the same board rule, the optional dead mask of the row takes part in the duplicate test
 // (a bit >= 52 is an invalid card), and the cards left to deal from -- one fewer in REFERENCE mode -- must cover the board.
+// mode 3 (npk_exact_equity_batch): mode 2's rules with n_players = the known hands, plus n_random[i] in 1..2, at most 10
+// players, and cards left for the unknown hands and the board -- one more under REFERENCE when a board card is to come.
 __global__ void check_rows_kernel(const uint8_t* a, int len_a, const uint8_t* b, int len_b, const uint8_t* n_players,
                                   int maxp, int enum_mode, long long n, uint32_t* bad /*[2]: cards, shape*/,
-                                  const uint64_t* dead, int deal_mode)
+                                  const uint64_t* dead, int deal_mode, const uint8_t* n_random)
 {
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
         unsigned long long mask = 0;
@@ -1593,7 +1595,12 @@ __global__ void check_rows_kernel(const uint8_t* a, int len_a, const uint8_t* b,
             mask |= d;
         }
         if (wrong) atomicAdd(&bad[0], 1u);
-        if (enum_mode == 2) {
+        if (enum_mode == 3) {
+            const int missing = 5 - known, k = n_random[i];
+            const int left = 52 - __popcll(mask & ((1ull << 52) - 1ull));
+            const int need = 2 * k + missing + (deal_mode == NPK_DEAL_REFERENCE && missing > 0 ? 1 : 0);
+            if (k < 1 || k > 2 || n_players[i] + k > 10 || left < need) atomicAdd(&bad[1], 1u);
+        } else if (enum_mode == 2) {
             const int missing = 5 - known;
             const int left = 52 - __popcll(mask & ((1ull << 52) - 1ull)) - (deal_mode == NPK_DEAL_REFERENCE && missing > 0 ? 1 : 0);
             if (left < missing) atomicAdd(&bad[1], 1u);
@@ -1607,14 +1614,14 @@ __global__ void check_rows_kernel(const uint8_t* a, int len_a, const uint8_t* b,
 namespace {
 int check_rows(DeviceState* ds, const uint8_t* a, int len_a, const uint8_t* b, int len_b, const uint8_t* n_players, int maxp,
                int enum_mode, int64_t n, cudaStream_t s, const char* shape_msg, const uint64_t* dead = nullptr,
-               int deal_mode = NPK_DEAL_UNIFORM)
+               int deal_mode = NPK_DEAL_UNIFORM, const uint8_t* n_random = nullptr)
 {
     uint32_t* d_bad = nullptr;
     cudaError_t e = cudaMalloc(&d_bad, 8);
     if (e == cudaSuccess) e = cudaMemsetAsync(d_bad, 0, 8, s);
     if (e != cudaSuccess) { cudaFree(d_bad); return cuda_fail(e, "validation scratch"); }
     const int grid = (int)std::min<long long>((n + 255) / 256, 8 * ds->sm_count);
-    check_rows_kernel<<<grid, 256, 0, s>>>(a, len_a, b, len_b, n_players, maxp, enum_mode, n, d_bad, dead, deal_mode);
+    check_rows_kernel<<<grid, 256, 0, s>>>(a, len_a, b, len_b, n_players, maxp, enum_mode, n, d_bad, dead, deal_mode, n_random);
     uint32_t bad[2] = {0, 0};
     e = cudaMemcpyAsync(bad, d_bad, 8, cudaMemcpyDeviceToHost, s);
     if (e == cudaSuccess) e = cudaStreamSynchronize(s);
@@ -1735,6 +1742,39 @@ int npk_showdown_equity_batch(const uint8_t* holes, const uint8_t* n_players, co
     p.workspace = static_cast<uint8_t*>(workspace);
     cudaError_t e = npk::launch_showdown_equity(p, s);
     return e == cudaSuccess ? NPK_OK : cuda_fail(e, "showdown_equity_kernel launch");
+}
+
+int64_t npk_exact_equity_workspace_bytes(int64_t N) { return npk::exact_equity_workspace_bytes(N); }
+
+int npk_exact_equity_batch(const uint8_t* holes, const uint8_t* n_known, const uint8_t* n_random, const uint8_t* board,
+                           const uint64_t* dead, int64_t N, int maxk, int deal_mode, uint32_t flags, uint64_t* win, uint64_t* tie,
+                           uint64_t* lose, void* workspace, void* stream)
+{
+    int rc = check_deal_mode(deal_mode);
+    if (rc) return rc;
+    if (maxk < 1 || maxk > 8) return fail(NPK_ERR_INVALID_ARGUMENT, "maxk must be 1..8");
+    DeviceState* ds;
+    rc = batch_start(&ds, N, 1, 0);
+    if (rc) return rc == kEmptyBatch ? NPK_OK : rc;
+    if (!holes || !n_known || !n_random || !board || !win || !tie || !lose || !workspace)
+        return fail(NPK_ERR_INVALID_ARGUMENT, "null pointer");
+    const cudaStream_t s = static_cast<cudaStream_t>(stream);
+    if (flags & NPK_FLAG_VALIDATE) {
+        rc = check_rows(ds, holes, 2 * maxk, board, 5, n_known, maxk, 3, N, s,
+                        " spot(s) with n_known outside 1..maxk, n_random outside 1..2, more than 10 players or too few cards "
+                        "left for the unknown hands and the board", dead, deal_mode, n_random);
+        if (rc) return rc;
+    }
+    npk::ExactEquityParams p{};
+    p.tables = ds->t;
+    p.holes = holes; p.n_known = n_known; p.n_random = n_random; p.board = board; p.dead = dead;
+    p.n = N; p.maxk = maxk; p.sm_count = ds->sm_count;
+    p.win = reinterpret_cast<unsigned long long*>(win);
+    p.tie = reinterpret_cast<unsigned long long*>(tie);
+    p.lose = reinterpret_cast<unsigned long long*>(lose);
+    p.workspace = static_cast<uint8_t*>(workspace);
+    cudaError_t e = npk::launch_exact_equity(p, deal_mode, s);
+    return e == cudaSuccess ? NPK_OK : cuda_fail(e, "exact_equity_kernel launch");
 }
 
 // ---- vectorised HoldemTable (include/npk_holdem.h) ------------------------------------------------------------------------

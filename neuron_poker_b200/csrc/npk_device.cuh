@@ -47,7 +47,8 @@ struct SmemTables {
 // Codes: 1 rowoff gather, 2 value gather, 3 flush gather, 4 Fisher-Yates slot, 5 Lehmer slot, 6 duplicate Lehmer slot,
 //        7 deck not restored, 8 descriptor index, 9 pair list of the range sampler (entry index, card ids),
 //        10 unseen-card slot or pair index of the showdown-equity enumeration,
-//        11 query slot of a device-planned range round, or the query id read from its qindex.
+//        11 query slot of a device-planned range round, or the query id read from its qindex,
+//        12 unseen-card slot, hand-list entry, compact rank or pair index of the exact-equity enumeration.
 #ifdef NPK_CHECKED
 #define NPK_CHECK(ptr, cond, code) do { if (!(cond)) atomicMax((ptr), (unsigned)(code)); } while (0)
 #else

@@ -171,7 +171,26 @@ struct ShowdownEquityParams {
     uint8_t* workspace;           // showdown_equity_workspace_bytes(n)
 };
 
+// exact equity against one or two unknown opponents (npk_exact_equity.cu)
+struct ExactEquityParams {
+    DeviceTables tables;
+    const uint8_t* holes;         // [n, maxk, 2]: the hero, then the known opponents
+    const uint8_t* n_known;       // [n] hands in `holes` that take part, hero included (1..maxk)
+    const uint8_t* n_random;      // [n] unknown opponents (1..2)
+    const uint8_t* board;         // [n, 5], 0xFF padding
+    const uint64_t* dead;         // [n] masks, or null
+    long long n;
+    int maxk;
+    int sm_count;
+    unsigned long long* win;      // [n]
+    unsigned long long* tie;      // [n]
+    unsigned long long* lose;     // [n]
+    uint8_t* workspace;           // exact_equity_workspace_bytes(n): plan header, prefix and the per-spot unit counts
+};
+
 size_t aux_smem(const DeviceTables& t);
+long long exact_equity_workspace_bytes(long long n);
+cudaError_t launch_exact_equity(const ExactEquityParams& p, int deal_mode, cudaStream_t s);   // deal_mode: NPK_DEAL_*
 long long showdown_equity_workspace_bytes(long long n);
 cudaError_t launch_showdown_equity(const ShowdownEquityParams& p, cudaStream_t s);
 cudaError_t launch_equity_uniform(int nopp, int nb, const EquityParams& p, long long items, int sm_count, cudaStream_t s);

@@ -10,30 +10,29 @@
 // numbered C(b, 2) + a (the list of enum_kernel): a warp fixes the top cards, sums their descriptors, suit counters and rank
 // masks once, and its lanes walk the pairs of the block -- no unranking and no clash test per completion.
 //
-// Work split: the completions of all spots of a batch form one global sequence (an exclusive prefix of the per-spot counts in the
-// workspace); a work item is a fixed-size range of that sequence, so one heads-up preflop spot spreads over every SM while a
-// single item carries several small spots.  Three kernels, all on the caller's stream and without a host round trip:
+// Work split (npk_enum_plan.cuh): the completions of all spots of a batch form one global sequence (an exclusive prefix of the
+// per-spot counts in the workspace); a work item is a fixed-size range of that sequence, so one heads-up preflop spot spreads
+// over every SM while a single item carries several small spots.  Three kernels, all on the caller's stream and without a
+// host round trip:
 //   se_prepare_kernel   per spot: completions, zeroed outputs
 //   se_plan_kernel      one CTA: prefix of the completions, item size, work counter reset
 //   showdown_equity_kernel  persistent, one CTA per SM: tables staged once per CTA, warps pull items from the work counter
 #include <algorithm>
+#include "npk_enum_plan.cuh"
 #include "npk_mc.cuh"
 
 namespace npk {
 
 constexpr int kSeThreads = 512;
 constexpr int kSeWarps = kSeThreads / 32;
-constexpr int kSePlanThreads = 1024;
 // completions per work item: a lane scores at most one item's worth per spot, so its win and tie counts stay below 2^16 and
 // share below 2^32 (32,768 * 2,520)
 constexpr uint32_t kSeMaxItem = 32768, kSeMinItem = 512;
-// workspace: [0,8) work counter | [8,12) completions per item | [64, 64 + 8 (N+1)) exclusive prefix of the completions
-constexpr int kSeWsCounter = 0, kSeWsItem = 8, kSeWsPrefix = 64;
 // dynamic shared memory behind the tables: descriptors [64] | pair list [1326] u16 | C(c, k) [6][64] u32 | warp decks [16][64]
 constexpr uint32_t kSePairOff = kDescBytes, kSeBinomOff = kSePairOff + 2688, kSeDeckOff = kSeBinomOff + 6 * 64 * 4,
                    kSeExtraBytes = kSeDeckOff + kSeWarps * 64 * 4;
 
-long long showdown_equity_workspace_bytes(long long n) { return kSeWsPrefix + 8 * ((n > 0 ? n : 0) + 1); }
+long long showdown_equity_workspace_bytes(long long n) { return plan_workspace_bytes(n); }
 
 struct SpotShape {
     uint64_t avail;    // unseen cards U, one bit per id
@@ -61,81 +60,22 @@ __device__ __forceinline__ SpotShape spot_shape(const ShowdownEquityParams& p, l
     return sh;
 }
 
-__device__ __forceinline__ unsigned long long se_binom(int n, int k)
-{
-    if (k < 0 || n < k) return 0;
-    unsigned long long r = 1;
-    for (int i = 1; i <= k; i++) r = r * (unsigned long long)(n - k + i) / (unsigned long long)i;
-    return r;
-}
-
 __global__ void __launch_bounds__(256) se_prepare_kernel(const ShowdownEquityParams p)
 {
     for (long long s = (long long)blockIdx.x * blockDim.x + threadIdx.x; s < p.n; s += (long long)gridDim.x * blockDim.x) {
         const SpotShape sh = spot_shape(p, s);
-        p.completions[s] = sh.players && sh.n >= sh.missing ? se_binom(sh.n, sh.missing) : 0ull;
+        p.completions[s] = sh.players && sh.n >= sh.missing ? plan_binom(sh.n, sh.missing) : 0ull;
         for (int q = 0; q < p.maxp; q++) {
             p.win[s * p.maxp + q] = 0; p.tie[s * p.maxp + q] = 0; p.share[s * p.maxp + q] = 0;
         }
     }
 }
 
-// One CTA: exclusive prefix of the completions (four spots per thread and pass), then the item size -- about four items per
-// warp of the grid, within [kSeMinItem, kSeMaxItem] -- and the work counter for the enumeration kernel.
-__global__ void __launch_bounds__(kSePlanThreads) se_plan_kernel(const ShowdownEquityParams p)
+// One CTA: exclusive prefix of the completions, then the item size -- about four items per warp of the grid, within
+// [kSeMinItem, kSeMaxItem] -- and the work counter for the enumeration kernel.
+__global__ void __launch_bounds__(kPlanThreads) se_plan_kernel(const ShowdownEquityParams p)
 {
-    __shared__ unsigned long long s_warp[32];
-    __shared__ unsigned long long s_carry;
-    unsigned long long* prefix = reinterpret_cast<unsigned long long*>(p.workspace + kSeWsPrefix);
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    if (threadIdx.x == 0) s_carry = 0;
-    __syncthreads();
-    for (long long base = 0; base < p.n; base += 4 * kSePlanThreads) {
-        unsigned long long v[4], sum = 0;
-#pragma unroll
-        for (int k = 0; k < 4; k++) {
-            const long long i = base + 4 * threadIdx.x + k;
-            v[k] = i < p.n ? p.completions[i] : 0ull;
-            sum += v[k];
-        }
-        unsigned long long incl = sum;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const unsigned long long t = __shfl_up_sync(0xffffffffu, incl, o);
-            if (lane >= o) incl += t;
-        }
-        if (lane == 31) s_warp[warp] = incl;
-        __syncthreads();
-        if (warp == 0) {
-            unsigned long long w = s_warp[lane];
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-                const unsigned long long t = __shfl_up_sync(0xffffffffu, w, o);
-                if (lane >= o) w += t;
-            }
-            s_warp[lane] = w;
-        }
-        __syncthreads();
-        unsigned long long excl = s_carry + (warp ? s_warp[warp - 1] : 0ull) + incl - sum;
-#pragma unroll
-        for (int k = 0; k < 4; k++) {
-            const long long i = base + 4 * threadIdx.x + k;
-            if (i < p.n) prefix[i] = excl;
-            excl += v[k];
-        }
-        __syncthreads();
-        if (threadIdx.x == 0) s_carry += s_warp[31];
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) {
-        const unsigned long long total = s_carry;
-        prefix[p.n] = total;
-        unsigned long long item = total / (4ull * (unsigned long long)p.sm_count * kSeWarps);
-        item = (item + 31) / 32 * 32;
-        item = item < kSeMinItem ? kSeMinItem : (item > kSeMaxItem ? kSeMaxItem : item);
-        *reinterpret_cast<uint32_t*>(p.workspace + kSeWsItem) = (uint32_t)item;
-        *reinterpret_cast<unsigned long long*>(p.workspace + kSeWsCounter) = 0ull;
-    }
+    plan_items(p.completions, p.n, p.workspace, 4ull * (unsigned long long)p.sm_count * kSeWarps, 32, kSeMinItem, kSeMaxItem);
 }
 
 // One completion scored for P players: `bsum` / `bfield` / `bf` describe the complete board.  wt packs win (bits 0..15) and
@@ -300,16 +240,16 @@ __global__ void __launch_bounds__(kSeThreads, 1) showdown_equity_kernel(const Sh
         while ((b + 1) * b / 2 <= i) b++;
         s_pair[i] = (uint16_t)((i - b * (b - 1) / 2) | b << 8);
     }
-    for (int i = threadIdx.x; i < 6 * 64; i += blockDim.x) s_binom[i] = (uint32_t)se_binom(i & 63, i >> 6);
+    for (int i = threadIdx.x; i < 6 * 64; i += blockDim.x) s_binom[i] = (uint32_t)plan_binom(i & 63, i >> 6);
     __syncthreads();
     SeSmem sm;
     sm.desc = s_desc; sm.pair = s_pair; sm.binom = s_binom;
     sm.deck = reinterpret_cast<uint32_t*>(extra + kSeDeckOff) + 64 * warp;
 
-    const unsigned long long* prefix = reinterpret_cast<const unsigned long long*>(p.workspace + kSeWsPrefix);
-    unsigned long long* counter = reinterpret_cast<unsigned long long*>(p.workspace + kSeWsCounter);
+    const unsigned long long* prefix = reinterpret_cast<const unsigned long long*>(p.workspace + kPlanWsPrefix);
+    unsigned long long* counter = reinterpret_cast<unsigned long long*>(p.workspace + kPlanWsCounter);
     const unsigned long long total = prefix[p.n];
-    const unsigned long long item_size = *reinterpret_cast<const uint32_t*>(p.workspace + kSeWsItem);
+    const unsigned long long item_size = *reinterpret_cast<const uint32_t*>(p.workspace + kPlanWsItem);
     const long long n_items = (long long)((total + item_size - 1) / item_size);
     for (long long item = next_item(counter, lane); item < n_items; item = next_item(counter, lane)) {
         unsigned long long g0 = (unsigned long long)item * item_size;
@@ -357,7 +297,7 @@ cudaError_t launch_showdown_equity(const ShowdownEquityParams& p, cudaStream_t s
 {
     const int prep_grid = (int)std::min<long long>((p.n + 255) / 256, 8ll * p.sm_count);
     se_prepare_kernel<<<prep_grid, 256, 0, s>>>(p);
-    se_plan_kernel<<<1, kSePlanThreads, 0, s>>>(p);
+    se_plan_kernel<<<1, kPlanThreads, 0, s>>>(p);
     const size_t smem = 128 + (size_t)p.tables.value_bytes + p.tables.rowoff_bytes + p.tables.flush_bytes + kSeExtraBytes;
     cudaError_t e = cudaFuncSetAttribute(showdown_equity_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;

@@ -231,6 +231,80 @@ def showdown_equity(hands, table_cards=(), dead_cards=(), deal_mode="uniform"):
     return {"equity": [x / (SHARE_UNIT * comp) for x in share], "win": win, "tie": tie, "completions": comp}
 
 
+def exact_equity_batch(holes, n_known, n_random, board, dead=None, deal_mode="reference", device=None, validate=None):
+    """Exact equity against one or two unknown opponents, with known opponent hands and dead cards: every deal of the unknown
+    hands and every completion of the board enumerated on the GPU.
+    holes [N,maxk,2] (maxk 1..8): the hero, then the known opponents; n_known [N]: hands of `holes` in the spot, hero included;
+    n_random [N]: unknown opponents (1 or 2); board [N,5] with 0xFF padding; dead [N,k] card ids removed from the deck (0xFF
+    padding) or None.  deal_mode "uniform" counts every deal once; "reference" weights it by how often the reference's dealer
+    makes it (include/npk.h, npk_exact_equity_batch).  Returns a dict of int64 CUDA tensors win, tie, lose [N] (hero strictly
+    best / tied for best / beaten); (win + tie) / (win + tie + lose) is the value run_montecarlo converges to."""
+    from .equity import _DEAL
+    torch = _torch()
+    dev = _dev(device)
+    flags = _want_check(holes, validate)
+    holes, board = _u8_tensor(holes, dev), _u8_tensor(board, dev)
+    n_known, n_random = _u8_tensor(n_known, dev), _u8_tensor(n_random, dev)
+    N = holes.shape[0]
+    maxk = holes.shape[1] if holes.dim() == 3 else 0
+    if holes.dim() != 3 or holes.shape[2] != 2 or board.shape != (N, 5) or n_known.shape != (N,) or n_random.shape != (N,):
+        raise ValueError("expected holes [N,maxk,2], n_known [N], n_random [N] and board [N,5]")
+    masks = _dead_masks(dead, N, dev) if dead is not None and N else None
+    L = _lib.ensure_init(dev.index)
+    out = {k: torch.empty(N, dtype=torch.int64, device=dev) for k in ("win", "tie", "lose")}
+    ws = torch.empty(int(L.npk_exact_equity_workspace_bytes(N)), dtype=torch.uint8, device=dev)
+    with torch.cuda.device(dev):
+        _lib.check(L.npk_exact_equity_batch(holes.data_ptr(), n_known.data_ptr(), n_random.data_ptr(), board.data_ptr(),
+                                            masks.data_ptr() if masks is not None else None, N, maxk, _DEAL.get(deal_mode, -1),
+                                            flags, out["win"].data_ptr(), out["tie"].data_ptr(), out["lose"].data_ptr(),
+                                            ws.data_ptr(), torch.cuda.current_stream(dev).cuda_stream))
+    return out
+
+
+def exact_equity_counts(player_cards, table_cards, players, known_opponents=(), ghost_cards='', deal_mode="reference"):
+    """The exact value run_montecarlo(player_card_list = [player_cards] + known_opponents, table_cards, players, ghost_cards)
+    converges to, for one or two unknown opponents: players - 1 - len(known_opponents) must be 1 or 2.  Argument names and
+    checks follow equity_counts_ranges; player_cards and every known opponent are two cards (no ranges).
+    Returns dict(equity = (win + tie) / (win + tie + lose), win, tie, lose)."""
+    players = int(players)
+    if players < 1:
+        raise IndexError("list index out of range")
+    if players > 10:
+        raise ValueError("at most 10 players")
+    if deal_mode not in ("uniform", "reference"):
+        raise ValueError("deal_mode must be 'uniform' or 'reference'")
+    board = card_ids(table_cards)
+    if len(board) > 5:
+        raise ValueError("table_cards holds more than five cards")
+    ghost = card_ids(ghost_cards) if ghost_cards not in ('', None) else []
+    if ghost and len(ghost) != 2:
+        raise ValueError("ghost_cards must be '' or two cards")
+    hole = card_ids(player_cards)
+    if len(hole) != 2:
+        raise ValueError("player_cards must hold exactly two cards, got %d" % len(hole))
+    known = []
+    for hand in known_opponents:
+        ids = card_ids(hand)
+        if len(ids) != 2:
+            raise ValueError("a known opponent's hand must hold exactly two cards, got %d" % len(ids))
+        known.append(ids)
+    if len(set(hole + sum(known, []) + board + ghost)) != 2 + 2 * len(known) + len(board) + len(ghost):
+        raise ValueError("duplicate cards in player_cards / known_opponents / table_cards / ghost_cards")
+    k = players - 1 - len(known)
+    if k == 0:
+        raise ValueError("every opponent is known: showdown_equity gives the exact equity of known hands")
+    if k not in (1, 2):
+        raise ValueError("exact_equity_counts enumerates one or two unknown opponents, not %d" % k)
+    holes = np.array([[hole] + known], dtype=np.uint8)
+    try:
+        out = exact_equity_batch(holes, [1 + len(known)], [k], [board + [NO_CARD] * (5 - len(board))],
+                                 np.array([ghost or [NO_CARD]], dtype=np.uint8), deal_mode=deal_mode, validate=True)
+    except _lib.NpkError as exc:
+        raise ValueError(str(exc)) from None
+    win, tie, lose = (int(out[x][0]) for x in ("win", "tie", "lose"))
+    return {"equity": (win + tie) / (win + tie + lose), "win": win, "tie": tie, "lose": lose}
+
+
 def host_tables():
     """Host copies of the lookup tables built by libnpk (no GPU needed): dict of numpy arrays."""
     L = _lib.lib()

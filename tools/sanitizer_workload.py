@@ -145,6 +145,26 @@ npk.showdown_equity_batch(torch.randint(0, 256, (256, 10, 2), dtype=torch.uint8,
 torch.cuda.synchronize()
 print("ok showdown equity", flush=True)
 
+# exact equity against one or two unknown opponents: known hands, every board size, dead cards, both dealers, garbage bytes
+ee_h = np.full((48, 4, 2), 255, dtype=np.uint8); ee_b = np.full((48, 5), 255, dtype=np.uint8)
+ee_d = np.full((48, 2), 255, dtype=np.uint8); ee_k = np.zeros(48, dtype=np.uint8); ee_r = np.zeros(48, dtype=np.uint8)
+for i in range(48):
+    K, k, nb = 1 + i % 4, 1 + (i // 4) % 2, (5, 4, 3, 5, 4, 0)[i // 8]
+    k = 1 if nb < 4 else k
+    c = rng.permutation(52)[:2 * K + nb + 2]
+    ee_h[i, :K] = c[:2 * K].reshape(K, 2); ee_b[i, :nb] = c[2 * K:2 * K + nb]; ee_d[i] = c[2 * K + nb:]
+    ee_k[i], ee_r[i] = K, k
+for mode in ("uniform", "reference"):
+    o = npk.exact_equity_batch(ee_h, ee_k, ee_r, ee_b, ee_d, deal_mode=mode)
+    assert ((o["win"] + o["tie"] + o["lose"]) > 0).all()
+npk.exact_equity_batch(torch.randint(0, 256, (256, 8, 2), dtype=torch.uint8, device="cuda"),
+                       torch.randint(0, 256, (256,), dtype=torch.uint8, device="cuda"),
+                       torch.randint(0, 4, (256,), dtype=torch.uint8, device="cuda"),
+                       torch.randint(0, 256, (256, 5), dtype=torch.uint8, device="cuda"),
+                       torch.randint(0, 256, (256, 3), dtype=torch.uint8, device="cuda"))
+torch.cuda.synchronize()
+print("ok exact equity", flush=True)
+
 # vectorised HoldemTable: self-play with both dealers, observation vector, showdowns
 tb = HoldemTables(96, n_players=6, seed=3, autoplay=[1] * 6)
 tb.enable_observations()
