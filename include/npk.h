@@ -22,6 +22,7 @@
  *                       computed exactly (every board completion) and for every player, split pots included
  *   npk_exact_equity_batch  run_montecarlo with one or two unknown opponents beside known hands and ghost cards, computed
  *                       exactly under either dealer: the value it converges to
+ *   npk_*_equity_win_types_batch  the same two, with run_montecarlo's winTypesDict (:226-231): the wins by hand type
  *
  * Cards are bytes: id = 4*rank + suit with ranks "23456789TJQKA" and suits "CDHS" -- the order of
  * MonteCarlo.create_card_deck (tools/montecarlo_python.py:114-119).  0xFF marks "no card" in board arrays.
@@ -359,6 +360,16 @@ int64_t npk_showdown_equity_workspace_bytes(int64_t N);
 int npk_showdown_equity_batch(const uint8_t* holes, const uint8_t* n_players, const uint8_t* board, const uint64_t* dead,
                               int64_t N, int maxp, int deal_mode, uint32_t flags, uint64_t* win, uint64_t* tie, uint64_t* share,
                               uint64_t* completions, void* workspace, void* stream);
+/* npk_showdown_equity_batch plus the hand types of the wins: win_types [N,maxp,9] (u64, OVERWRITTEN), where
+ * win_types[s][p][t] = the completions in which player p holds the best rank, alone or tied, and that rank has hand type t
+ * (0 high card .. 8 straight flush, as npk_showdown_batch's wtype).  sum_t win_types[s][p][t] = win[s][p] + tie[s][p].
+ * Player 0's bins over completions are run_montecarlo's winTypesDict (montecarlo_python.py:226-231) when every hand is known.
+ * Same arguments, validation, workspace and other outputs as npk_showdown_equity_batch, which is this call with
+ * win_types = NULL. */
+int npk_showdown_equity_win_types_batch(const uint8_t* holes, const uint8_t* n_players, const uint8_t* board,
+                                        const uint64_t* dead, int64_t N, int maxp, int deal_mode, uint32_t flags, uint64_t* win,
+                                        uint64_t* tie, uint64_t* share, uint64_t* completions, uint64_t* win_types,
+                                        void* workspace, void* stream);
 
 /*
  * Exact equity against one or two UNKNOWN opponents, with known opponent hands and dead cards: run_montecarlo with entries of
@@ -387,6 +398,15 @@ int64_t npk_exact_equity_workspace_bytes(int64_t N);
 int npk_exact_equity_batch(const uint8_t* holes, const uint8_t* n_known, const uint8_t* n_random, const uint8_t* board,
                            const uint64_t* dead, int64_t N, int maxk, int deal_mode, uint32_t flags, uint64_t* win, uint64_t* tie,
                            uint64_t* lose, void* workspace, void* stream);
+/* npk_exact_equity_batch plus the hand types of the hero's wins: win_types [N,9] (u64, OVERWRITTEN), where win_types[s][t] =
+ * the weighted count (the same weights as win and tie, in either deal_mode) of the deals in which the hero is strictly best or
+ * tied for best with a rank of hand type t (0 high card .. 8 straight flush).  sum_t win_types[s][t] = win[s] + tie[s].
+ * win_types[s][t] / (win + tie + lose) is what run_montecarlo's winTypesDict (montecarlo_python.py:226-231) converges to.
+ * Same arguments, validation, workspace and other outputs as npk_exact_equity_batch, which is this call with
+ * win_types = NULL. */
+int npk_exact_equity_win_types_batch(const uint8_t* holes, const uint8_t* n_known, const uint8_t* n_random, const uint8_t* board,
+                                     const uint64_t* dead, int64_t N, int maxk, int deal_mode, uint32_t flags, uint64_t* win,
+                                     uint64_t* tie, uint64_t* lose, uint64_t* win_types, void* workspace, void* stream);
 
 /* Integer-issue microbenchmark on the current device (the roofline denominator of the Monte-Carlo kernel):
  * variant 0 = LOP3 chains (alu pipe), 1 = IMAD chains (fma pipe), 2 = both interleaved.  Reports executed

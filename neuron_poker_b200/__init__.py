@@ -10,7 +10,8 @@ plus batched entry points on CUDA tensors (get_equity_batch, get_equity_batch_ad
 error --, get_equity_ranges_batch, get_equity_ranges_batch_adaptive, rank7, showdown, enumerate_equity,
 showdown_equity_batch, exact_equity_batch), the exact equity of known hands (showdown_equity), the exact value get_equity
 converges to (exact_equity), the exact value run_montecarlo converges to against one or two unknown opponents beside known
-hands and ghost cards (exact_equity_counts)
+hands and ghost cards (exact_equity_counts); with win_types=True the exact calls also give the wins by hand type, the
+winTypesDict run_montecarlo converges to
 and the vectorised environment (holdem.HoldemTables: gym_env/env.py::HoldemTable for N tables on the GPU).
 All compute runs in libnpk.so's CUDA kernels; importing this package does not import torch.
 """

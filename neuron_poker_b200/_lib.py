@@ -88,6 +88,10 @@ def lib():
                 L.npk_exact_equity_workspace_bytes.argtypes = [i64]
                 L.npk_exact_equity_workspace_bytes.restype = i64
                 L.npk_exact_equity_batch.argtypes = [u8, u8, u8, u8, u64, i64, i32, i32, ctypes.c_uint32, u64, u64, u64, vp, vp]
+                L.npk_showdown_equity_win_types_batch.argtypes = [u8, u8, u8, u64, i64, i32, i32, ctypes.c_uint32, u64, u64, u64,
+                                                                  u64, u64, vp, vp]
+                L.npk_exact_equity_win_types_batch.argtypes = [u8, u8, u8, u8, u64, i64, i32, i32, ctypes.c_uint32, u64, u64, u64,
+                                                               u64, vp, vp]
                 L.npk_checked_status.argtypes = [ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_uint32)]
                 L.npk_int_peak.argtypes = [i32, i32, ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_float)]
                 L.npk_philox_debug.argtypes = [u32, ctypes.c_uint32, ctypes.c_uint32, i32, u32, vp]

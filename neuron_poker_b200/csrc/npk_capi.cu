@@ -1718,6 +1718,15 @@ int npk_showdown_equity_batch(const uint8_t* holes, const uint8_t* n_players, co
                               int64_t N, int maxp, int deal_mode, uint32_t flags, uint64_t* win, uint64_t* tie, uint64_t* share,
                               uint64_t* completions, void* workspace, void* stream)
 {
+    return npk_showdown_equity_win_types_batch(holes, n_players, board, dead, N, maxp, deal_mode, flags, win, tie, share,
+                                               completions, nullptr, workspace, stream);
+}
+
+int npk_showdown_equity_win_types_batch(const uint8_t* holes, const uint8_t* n_players, const uint8_t* board,
+                                        const uint64_t* dead, int64_t N, int maxp, int deal_mode, uint32_t flags, uint64_t* win,
+                                        uint64_t* tie, uint64_t* share, uint64_t* completions, uint64_t* win_types,
+                                        void* workspace, void* stream)
+{
     DeviceState* ds;
     int rc = batch_start(&ds, N, 1, 0);
     if (rc) return rc == kEmptyBatch ? NPK_OK : rc;
@@ -1739,6 +1748,7 @@ int npk_showdown_equity_batch(const uint8_t* holes, const uint8_t* n_players, co
     p.tie = reinterpret_cast<unsigned long long*>(tie);
     p.share = reinterpret_cast<unsigned long long*>(share);
     p.completions = reinterpret_cast<unsigned long long*>(completions);
+    p.win_types = reinterpret_cast<unsigned long long*>(win_types);
     p.workspace = static_cast<uint8_t*>(workspace);
     cudaError_t e = npk::launch_showdown_equity(p, s);
     return e == cudaSuccess ? NPK_OK : cuda_fail(e, "showdown_equity_kernel launch");
@@ -1749,6 +1759,14 @@ int64_t npk_exact_equity_workspace_bytes(int64_t N) { return npk::exact_equity_w
 int npk_exact_equity_batch(const uint8_t* holes, const uint8_t* n_known, const uint8_t* n_random, const uint8_t* board,
                            const uint64_t* dead, int64_t N, int maxk, int deal_mode, uint32_t flags, uint64_t* win, uint64_t* tie,
                            uint64_t* lose, void* workspace, void* stream)
+{
+    return npk_exact_equity_win_types_batch(holes, n_known, n_random, board, dead, N, maxk, deal_mode, flags, win, tie, lose,
+                                            nullptr, workspace, stream);
+}
+
+int npk_exact_equity_win_types_batch(const uint8_t* holes, const uint8_t* n_known, const uint8_t* n_random, const uint8_t* board,
+                                     const uint64_t* dead, int64_t N, int maxk, int deal_mode, uint32_t flags, uint64_t* win,
+                                     uint64_t* tie, uint64_t* lose, uint64_t* win_types, void* workspace, void* stream)
 {
     int rc = check_deal_mode(deal_mode);
     if (rc) return rc;
@@ -1772,6 +1790,7 @@ int npk_exact_equity_batch(const uint8_t* holes, const uint8_t* n_known, const u
     p.win = reinterpret_cast<unsigned long long*>(win);
     p.tie = reinterpret_cast<unsigned long long*>(tie);
     p.lose = reinterpret_cast<unsigned long long*>(lose);
+    p.win_types = reinterpret_cast<unsigned long long*>(win_types);
     p.workspace = static_cast<uint8_t*>(workspace);
     cudaError_t e = npk::launch_exact_equity(p, deal_mode, s);
     return e == cudaSuccess ? NPK_OK : cuda_fail(e, "exact_equity_kernel launch");

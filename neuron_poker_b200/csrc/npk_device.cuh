@@ -48,7 +48,8 @@ struct SmemTables {
 //        7 deck not restored, 8 descriptor index, 9 pair list of the range sampler (entry index, card ids),
 //        10 unseen-card slot or pair index of the showdown-equity enumeration,
 //        11 query slot of a device-planned range round, or the query id read from its qindex,
-//        12 unseen-card slot, hand-list entry, compact rank or pair index of the exact-equity enumeration.
+//        12 unseen-card slot, hand-list entry, compact rank or pair index of the exact-equity enumeration,
+//        13 win-type bin (hand type, player) of the exact-equity and showdown-equity enumerations.
 #ifdef NPK_CHECKED
 #define NPK_CHECK(ptr, cond, code) do { if (!(cond)) atomicMax((ptr), (unsigned)(code)); } while (0)
 #else
@@ -256,6 +257,15 @@ __device__ __forceinline__ uint32_t eval7_desc(const SmemAddr& a, const uint32_t
         v = lds_u16(a.flush + 2u * field);            // a flush excludes full house / quads in 7 cards
     }
     return v;
+}
+
+// hand type of rank id v: 0 high card .. 8 straight flush (type_start[t] = first rank id of type t)
+__device__ __forceinline__ uint32_t hand_type(const DeviceTables& t, uint32_t v)
+{
+    uint32_t ty = 0;
+#pragma unroll
+    for (int i = 1; i < 9; i++) ty += v >= t.type_start[i];
+    return ty;
 }
 
 }  // namespace npk

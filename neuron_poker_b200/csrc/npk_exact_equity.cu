@@ -15,13 +15,17 @@
 //          slots above T between them.
 // The outcome is the hero against max(best known hand, unknown hands).  Counts are integers added per lane, reduced per warp and
 // added to the spot's counters with one atomic per warp whenever the spot changes: they do not depend on the grid or the plan.
+// With TYPES = 1 the kernel also fills win_types[9 s + t], the win + tie weight of the deals in which the hero's rank id has
+// hand type t.  The hero's value is fixed for a whole completion, so each thread adds its win + tie weight of the completion
+// to one of nine register bins (constant indices, selected by the type) once the completion's hands are walked, and the bins
+// are flushed like the counts: at most one atomic per non-zero bin per warp and spot.
 //
 // Work split (npk_enum_plan.cuh): one global sequence of units over the batch, a completion is one unit with one unknown
 // opponent and kEeUnitsK2 with two (about the ratio of their work); it belongs to the item that holds its first unit.  Items
 // are taken per CTA.  Three kernels, all on the caller's stream and without a host round trip:
 //   ee_prepare_kernel   per spot: units, zeroed outputs
 //   ee_plan_kernel      one CTA: prefix of the units, item size, work counter reset
-//   exact_equity_kernel<REF>  persistent, one CTA per SM: tables staged once per CTA, CTAs pull items from the work counter
+//   exact_equity_kernel<REF, TYPES>  persistent, one CTA per SM: tables staged once per CTA, CTAs pull items from the work counter
 #include <algorithm>
 #include "npk_enum_plan.cuh"
 #include "npk_mc.cuh"
@@ -33,6 +37,7 @@ constexpr int kEeWarps = kEeThreads / 32;
 constexpr unsigned long long kEeUnitsK2 = 256;
 // units per item: about four items per CTA, at least one completion per warp.  A lane then adds below 2^32: at most 2^16 + 1
 // one-opponent completions of <= 42 hands of weight <= 2, or 2^12 two-opponent completions of <= 83 x 42 pairs of weight <= 8.
+// A win-type bin holds part of the lane's win + tie, so it stays below 2^32 too.
 constexpr unsigned long long kEeMinItem = kEeWarps, kEeMaxItem = 1ull << 20;
 // dynamic shared memory behind the tables: descriptors [64] | pair list [1326] u16 | C(c, k) [6][64] u32 | R [64] u32 |
 // free cards of the current completion, per warp and one for the CTA: descriptors [17][64] u32, R slots [17][64] u8 |
@@ -85,6 +90,8 @@ __global__ void __launch_bounds__(256) ee_prepare_kernel(const ExactEquityParams
         const EeSpot sp = ee_spot(p, s);
         units[s] = sp.k && sp.n >= 2 * sp.k + sp.missing ? plan_binom(sp.n, sp.missing) * (sp.k == 2 ? kEeUnitsK2 : 1ull) : 0ull;
         p.win[s] = 0; p.tie[s] = 0; p.lose[s] = 0;
+        if (p.win_types)
+            for (int t = 0; t < 9; t++) p.win_types[9 * s + t] = 0;
     }
 }
 
@@ -193,6 +200,34 @@ __device__ __forceinline__ void ee_flush(const ExactEquityParams& p, long long s
     }
 }
 
+// the hand type of rank id v (0 high card .. 8 straight flush)
+__device__ __forceinline__ uint32_t ee_type(const ExactEquityParams& p, uint32_t v)
+{
+    const uint32_t ty = hand_type(p.tables, v);
+    NPK_CHECK(p.tables.check, ty < 9, 13);
+    return ty;
+}
+
+// add d, a thread's win + tie weight of one completion, to the bin of the hero's type ty
+__device__ __forceinline__ void ee_bin(uint32_t (&bins)[9], uint32_t ty, uint32_t d)
+{
+#pragma unroll
+    for (int t = 0; t < 9; t++) bins[t] += t == (int)ty ? d : 0u;
+}
+
+// sum the lanes' win-type bins of spot s and add the non-zero ones to its outputs
+__device__ __forceinline__ void ee_flush_types(const ExactEquityParams& p, long long s, const uint32_t (&bins)[9], int lane)
+{
+#pragma unroll
+    for (int t = 0; t < 9; t++) {
+        if (!__any_sync(0xffffffffu, bins[t])) continue;
+        unsigned long long B = bins[t];
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) B += __shfl_down_sync(0xffffffffu, B, o);
+        if (lane == 0) atomicAdd(&p.win_types[9 * s + t], B);
+    }
+}
+
 // the free cards of a completion (slot mask cm) into free / slot, by `count` threads starting at `t`
 __device__ __forceinline__ void ee_free_cards(const EeSmem& sm, int n, uint64_t cm, int t, int count)
 {
@@ -216,7 +251,7 @@ __device__ __forceinline__ uint64_t ee_mask(int m, const int (&c)[5])
 
 // One unknown opponent: completions r0..r1-1 of spot s, split over the warps (several warps share a completion when there
 // are fewer completions than warps); the lanes walk the free hands.
-template <int REF>
+template <int REF, int TYPES>
 __device__ __forceinline__ void ee_one(const ExactEquityParams& p, const SmemAddr& st, const EeSmem& sm, const EeSpot& sp,
                                        const EeBoard& kb, long long s, uint32_t r0, uint32_t r1, int warp, int lane)
 {
@@ -224,6 +259,7 @@ __device__ __forceinline__ void ee_one(const ExactEquityParams& p, const SmemAdd
     const int wpc = nc >= (uint32_t)kEeWarps ? 1 : kEeWarps / (int)nc;    // warps sharing one completion
     const int groups = kEeWarps / wpc, g = warp / wpc, sub = warp % wpc;
     uint32_t win = 0, tie = 0, lose = 0;
+    uint32_t bins[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
     if (g < groups) {
         const uint32_t q0 = r0 + (uint32_t)((unsigned long long)nc * g / groups);
         const uint32_t q1 = r0 + (uint32_t)((unsigned long long)nc * (g + 1) / groups);
@@ -239,6 +275,7 @@ __device__ __forceinline__ void ee_one(const ExactEquityParams& p, const SmemAdd
             const EeTable t = ee_table(kb, sm.deck, m, c);
             uint32_t hv, kv;
             ee_known(p, st, sm.desc, t, s, sp.nk, hv, kv);
+            const uint32_t wt0 = win + tie;
             for (int ip = sub * 32 + lane; ip < H; ip += 32 * wpc) {
                 NPK_CHECK(p.tables.check, ip < 1326, 12);
                 const uint32_t pr = sm.pair[ip];
@@ -254,18 +291,21 @@ __device__ __forceinline__ void ee_one(const ExactEquityParams& p, const SmemAdd
                 const uint32_t best = max(kv, ee_eval(st, t, sm.free[a], sm.free[b]));
                 win += hv > best ? w : 0u; tie += hv == best ? w : 0u; lose += hv < best ? w : 0u;
             }
+            if (TYPES) ee_bin(bins, ee_type(p, hv), win + tie - wt0);
         }
     }
     ee_flush(p, s, win, tie, lose, lane);
+    if (TYPES) ee_flush_types(p, s, bins, lane);
 }
 
 // Two unknown opponents: completions r0..r1-1 of spot s, one at a time on the whole CTA.
-template <int REF>
+template <int REF, int TYPES>
 __device__ __forceinline__ void ee_two(const ExactEquityParams& p, const SmemAddr& st, const EeSmem& sm, const EeSpot& sp,
                                        const EeBoard& kb, long long s, uint32_t r0, uint32_t r1, int warp, int lane)
 {
     const int n = sp.n, m = sp.missing, nf = n - m, H = nf * (nf - 1) / 2;
     uint32_t win = 0, tie = 0, lose = 0;
+    uint32_t bins[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
     int c[5] = {0, 0, 0, 0, 0};
     ee_unrank(p, sm.binom, n, m, r0, c);
     for (uint32_t r = r0; r < r1; r++) {
@@ -292,6 +332,7 @@ __device__ __forceinline__ void ee_two(const ExactEquityParams& p, const SmemAdd
         }
         uint32_t hv, kv;
         ee_known(p, st, sm.desc, t, s, sp.nk, hv, kv);
+        const uint32_t wt0 = win + tie;
         __syncthreads();
         for (int i1 = warp; i1 < H; i1 += kEeWarps) {
             const uint32_t h1 = sm.hand[i1];
@@ -315,11 +356,13 @@ __device__ __forceinline__ void ee_two(const ExactEquityParams& p, const SmemAdd
                 win += hv > best ? w : 0u; tie += hv == best ? w : 0u; lose += hv < best ? w : 0u;
             }
         }
+        if (TYPES) ee_bin(bins, ee_type(p, hv), win + tie - wt0);
     }
     ee_flush(p, s, win, tie, lose, lane);
+    if (TYPES) ee_flush_types(p, s, bins, lane);
 }
 
-template <int REF>
+template <int REF, int TYPES>
 __global__ void __launch_bounds__(kEeThreads, 1) exact_equity_kernel(const ExactEquityParams p)
 {
     extern __shared__ __align__(128) uint8_t smem[];
@@ -392,8 +435,8 @@ __global__ void __launch_bounds__(kEeThreads, 1) exact_equity_kernel(const Exact
                 card_bits(d, l, h);
                 kb.sum += d; kb.cnt += suit_inc(d); kb.lo |= l; kb.hi |= h;
             }
-            if (sp.k == 1) ee_one<REF>(p, st, sm1, sp, kb, s, r0, r1, warp, lane);
-            else ee_two<REF>(p, st, sm2, sp, kb, s, r0, r1, warp, lane);
+            if (sp.k == 1) ee_one<REF, TYPES>(p, st, sm1, sp, kb, s, r0, r1, warp, lane);
+            else ee_two<REF, TYPES>(p, st, sm2, sp, kb, s, r0, r1, warp, lane);
         }
     }
 }
@@ -404,7 +447,8 @@ cudaError_t launch_exact_equity(const ExactEquityParams& p, int deal_mode, cudaS
     ee_prepare_kernel<<<prep_grid, 256, 0, s>>>(p);
     ee_plan_kernel<<<1, kPlanThreads, 0, s>>>(p);
     const size_t smem = 128 + (size_t)p.tables.value_bytes + p.tables.rowoff_bytes + p.tables.flush_bytes + kEeExtraBytes;
-    auto k = deal_mode == 1 ? exact_equity_kernel<1> : exact_equity_kernel<0>;
+    auto k = p.win_types ? (deal_mode == 1 ? exact_equity_kernel<1, 1> : exact_equity_kernel<0, 1>)
+                         : (deal_mode == 1 ? exact_equity_kernel<1, 0> : exact_equity_kernel<0, 0>);
     cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     k<<<p.sm_count, kEeThreads, smem, s>>>(p);

@@ -169,6 +169,7 @@ struct ShowdownEquityParams {
     unsigned long long* share;    // [n, maxp]
     unsigned long long* completions;   // [n]
     uint8_t* workspace;           // showdown_equity_workspace_bytes(n)
+    unsigned long long* win_types;// [n, maxp, 9] or null: completions each player wins or ties, by the type of its rank
 };
 
 // exact equity against one or two unknown opponents (npk_exact_equity.cu)
@@ -186,6 +187,7 @@ struct ExactEquityParams {
     unsigned long long* tie;      // [n]
     unsigned long long* lose;     // [n]
     uint8_t* workspace;           // exact_equity_workspace_bytes(n): plan header, prefix and the per-spot unit counts
+    unsigned long long* win_types;// [n, 9] or null: win + tie weight of the deals, by the type of the hero's rank
 };
 
 size_t aux_smem(const DeviceTables& t);

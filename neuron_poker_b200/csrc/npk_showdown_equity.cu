@@ -10,13 +10,18 @@
 // numbered C(b, 2) + a (the list of enum_kernel): a warp fixes the top cards, sums their descriptors, suit counters and rank
 // masks once, and its lanes walk the pairs of the block -- no unranking and no clash test per completion.
 //
+// With TYPES = 1 the kernel also fills win_types[(s maxp + q) 9 + t], the completions player q wins or ties with a rank of hand
+// type t: per completion the winners' type is that of the best rank, and each lane adds 1 to the (winner, type) entry of its
+// warp's bins in shared memory ([maxp][9] u32 per warp).  At the end of a segment the warp adds the non-zero bins to the spot's
+// outputs (one atomic each) and clears them.
+//
 // Work split (npk_enum_plan.cuh): the completions of all spots of a batch form one global sequence (an exclusive prefix of the
 // per-spot counts in the workspace); a work item is a fixed-size range of that sequence, so one heads-up preflop spot spreads
 // over every SM while a single item carries several small spots.  Three kernels, all on the caller's stream and without a
 // host round trip:
 //   se_prepare_kernel   per spot: completions, zeroed outputs
 //   se_plan_kernel      one CTA: prefix of the completions, item size, work counter reset
-//   showdown_equity_kernel  persistent, one CTA per SM: tables staged once per CTA, warps pull items from the work counter
+//   showdown_equity_kernel<TYPES>  persistent, one CTA per SM: tables staged once per CTA, warps pull items from the work counter
 #include <algorithm>
 #include "npk_enum_plan.cuh"
 #include "npk_mc.cuh"
@@ -29,8 +34,9 @@ constexpr int kSeWarps = kSeThreads / 32;
 // share below 2^32 (32,768 * 2,520)
 constexpr uint32_t kSeMaxItem = 32768, kSeMinItem = 512;
 // dynamic shared memory behind the tables: descriptors [64] | pair list [1326] u16 | C(c, k) [6][64] u32 | warp decks [16][64]
+// | with TYPES: warp win-type bins [16][10][9] u32 (a bin counts at most one item's completions)
 constexpr uint32_t kSePairOff = kDescBytes, kSeBinomOff = kSePairOff + 2688, kSeDeckOff = kSeBinomOff + 6 * 64 * 4,
-                   kSeExtraBytes = kSeDeckOff + kSeWarps * 64 * 4;
+                   kSeExtraBytes = kSeDeckOff + kSeWarps * 64 * 4, kSeBinBytes = kSeWarps * 90 * 4;
 
 long long showdown_equity_workspace_bytes(long long n) { return plan_workspace_bytes(n); }
 
@@ -68,6 +74,8 @@ __global__ void __launch_bounds__(256) se_prepare_kernel(const ShowdownEquityPar
         for (int q = 0; q < p.maxp; q++) {
             p.win[s * p.maxp + q] = 0; p.tie[s * p.maxp + q] = 0; p.share[s * p.maxp + q] = 0;
         }
+        if (p.win_types)
+            for (int i = 0; i < 9 * p.maxp; i++) p.win_types[9 * p.maxp * s + i] = 0;
     }
 }
 
@@ -80,12 +88,13 @@ __global__ void __launch_bounds__(kPlanThreads) se_plan_kernel(const ShowdownEqu
 
 // One completion scored for P players: `bsum` / `bfield` / `bf` describe the complete board.  wt packs win (bits 0..15) and
 // tie (bits 16..31) counts; sh collects the split-pot shares of ties only (a win's 2520 is added at the reduction).
-template <int P>
-__device__ __forceinline__ void se_score(const SmemAddr& st, uint32_t bsum, uint32_t bfield, const BoardFlush& bf,
-                                         const uint32_t (&hs)[P], const uint32_t (&hl)[P], const uint32_t (&hh)[P],
-                                         uint32_t (&wt)[P], uint32_t (&sh)[P])
+// TYPES: every player holding the best rank adds 1 to bins[q * 9 + its type].
+template <int P, int TYPES>
+__device__ __forceinline__ void se_score(const ShowdownEquityParams& p, const SmemAddr& st, uint32_t bsum, uint32_t bfield,
+                                         const BoardFlush& bf, const uint32_t (&hs)[P], const uint32_t (&hl)[P],
+                                         const uint32_t (&hh)[P], uint32_t (&wt)[P], uint32_t (&sh)[P], uint32_t* bins)
 {
-    uint32_t v[P], best = 0, k = 0;
+    uint32_t v[P], best = 0, k = 0, qi = 0;
 #pragma unroll
     for (int q = 0; q < P; q++) {
         v[q] = eval_player(st, bsum + hs[q], bfield | prmt(hl[q], hh[q], bf.sel), bf.thr);
@@ -96,12 +105,22 @@ __device__ __forceinline__ void se_score(const SmemAddr& st, uint32_t bsum, uint
         const uint32_t eq = v[q] == best;
         wt[q] += eq;
         k += eq;
+        if (TYPES) qi = eq ? q : qi;
+    }
+    uint32_t ty = 0;
+    if (TYPES) {
+        ty = hand_type(p.tables, best);
+        NPK_CHECK(p.tables.check, ty < 9 && qi < (uint32_t)P, 13);
+        if (k == 1) atomicAdd(&bins[qi * 9 + ty], 1u);
     }
     if (k > 1) {
         const uint32_t part = 2520u / k;
 #pragma unroll
         for (int q = 0; q < P; q++)
-            if (v[q] == best) { wt[q] += 0xFFFFu; sh[q] += part; }
+            if (v[q] == best) {
+                wt[q] += 0xFFFFu; sh[q] += part;
+                if (TYPES) atomicAdd(&bins[q * 9 + ty], 1u);
+            }
     }
 }
 
@@ -110,10 +129,11 @@ struct SeSmem {
     const uint16_t* pair;      // [1326] a | b << 8, number C(b,2) + a
     const uint32_t* binom;     // [k * 64 + c] = C(c, k), k = 0..5
     uint32_t* deck;            // this warp's [52] descriptors of U, ascending id
+    uint32_t* bins;            // TYPES: this warp's win-type bins [P][9], zero between segments
 };
 
 // Completions r0..r1-1 (colex ranks) of spot s, P players, on one warp; adds the counts into the outputs.
-template <int P>
+template <int P, int TYPES>
 __device__ __forceinline__ void se_segment(const ShowdownEquityParams& p, const SmemAddr& st, const SeSmem& sm, const SpotShape& sh,
                                         long long s, uint32_t r0, uint32_t r1, int lane)
 {
@@ -176,7 +196,7 @@ __device__ __forceinline__ void se_segment(const ShowdownEquityParams& p, const 
                 const uint32_t d0 = deck[a], d1 = deck[b];
                 const BoardFlush bf = board_flush(tcnt + suit_inc(d0) + suit_inc(d1));
                 const uint32_t bfield = prmt(tlo, thi, bf.sel) | flush_bit(d0, bf.fsx) | flush_bit(d1, bf.fsx);
-                se_score<P>(st, tsum + d0 + d1, bfield, bf, hs, hl, hh, wt, shr);
+                se_score<P, TYPES>(p, st, tsum + d0 + d1, bfield, bf, hs, hl, hh, wt, shr, sm.bins);
             }
             pos += len;
             first = 0;
@@ -203,7 +223,7 @@ __device__ __forceinline__ void se_segment(const ShowdownEquityParams& p, const 
                 bsum += d; bcnt += suit_inc(d); blo |= l; bhi |= h;
             }
             const BoardFlush bf = board_flush(bcnt);
-            se_score<P>(st, bsum, prmt(blo, bhi, bf.sel), bf, hs, hl, hh, wt, shr);
+            se_score<P, TYPES>(p, st, bsum, prmt(blo, bhi, bf.sel), bf, hs, hl, hh, wt, shr, sm.bins);
         }
     }
 
@@ -221,8 +241,17 @@ __device__ __forceinline__ void se_segment(const ShowdownEquityParams& p, const 
         if (mt) atomicAdd(&p.tie[o], (unsigned long long)mt);
         if (mw || ms) atomicAdd(&p.share[o], 2520ull * mw + ms);
     }
+    if (TYPES) {
+        __syncwarp();                                          // every lane's bin adds are done
+        for (int i = lane; i < 9 * P; i += 32) {
+            const uint32_t c = sm.bins[i];
+            if (c) { atomicAdd(&p.win_types[9 * p.maxp * s + i], (unsigned long long)c); sm.bins[i] = 0; }
+        }
+        __syncwarp();
+    }
 }
 
+template <int TYPES>
 __global__ void __launch_bounds__(kSeThreads, 1) showdown_equity_kernel(const ShowdownEquityParams p)
 {
     extern __shared__ __align__(128) uint8_t smem[];
@@ -241,10 +270,14 @@ __global__ void __launch_bounds__(kSeThreads, 1) showdown_equity_kernel(const Sh
         s_pair[i] = (uint16_t)((i - b * (b - 1) / 2) | b << 8);
     }
     for (int i = threadIdx.x; i < 6 * 64; i += blockDim.x) s_binom[i] = (uint32_t)plan_binom(i & 63, i >> 6);
+    uint32_t* s_bins = reinterpret_cast<uint32_t*>(extra + kSeExtraBytes);
+    if (TYPES)
+        for (int i = threadIdx.x; i < kSeWarps * 90; i += blockDim.x) s_bins[i] = 0;
     __syncthreads();
     SeSmem sm;
     sm.desc = s_desc; sm.pair = s_pair; sm.binom = s_binom;
     sm.deck = reinterpret_cast<uint32_t*>(extra + kSeDeckOff) + 64 * warp;
+    sm.bins = s_bins + 90 * warp;
 
     const unsigned long long* prefix = reinterpret_cast<const unsigned long long*>(p.workspace + kPlanWsPrefix);
     unsigned long long* counter = reinterpret_cast<unsigned long long*>(p.workspace + kPlanWsCounter);
@@ -276,16 +309,16 @@ __global__ void __launch_bounds__(kSeThreads, 1) showdown_equity_kernel(const Sh
             __syncwarp();
             const uint32_t r0 = (uint32_t)(g0 - a), r1 = (uint32_t)(e - a);
             switch (sh.players) {
-                case 1: se_segment<1>(p, st, sm, sh, s, r0, r1, lane); break;
-                case 2: se_segment<2>(p, st, sm, sh, s, r0, r1, lane); break;
-                case 3: se_segment<3>(p, st, sm, sh, s, r0, r1, lane); break;
-                case 4: se_segment<4>(p, st, sm, sh, s, r0, r1, lane); break;
-                case 5: se_segment<5>(p, st, sm, sh, s, r0, r1, lane); break;
-                case 6: se_segment<6>(p, st, sm, sh, s, r0, r1, lane); break;
-                case 7: se_segment<7>(p, st, sm, sh, s, r0, r1, lane); break;
-                case 8: se_segment<8>(p, st, sm, sh, s, r0, r1, lane); break;
-                case 9: se_segment<9>(p, st, sm, sh, s, r0, r1, lane); break;
-                case 10: se_segment<10>(p, st, sm, sh, s, r0, r1, lane); break;
+                case 1: se_segment<1, TYPES>(p, st, sm, sh, s, r0, r1, lane); break;
+                case 2: se_segment<2, TYPES>(p, st, sm, sh, s, r0, r1, lane); break;
+                case 3: se_segment<3, TYPES>(p, st, sm, sh, s, r0, r1, lane); break;
+                case 4: se_segment<4, TYPES>(p, st, sm, sh, s, r0, r1, lane); break;
+                case 5: se_segment<5, TYPES>(p, st, sm, sh, s, r0, r1, lane); break;
+                case 6: se_segment<6, TYPES>(p, st, sm, sh, s, r0, r1, lane); break;
+                case 7: se_segment<7, TYPES>(p, st, sm, sh, s, r0, r1, lane); break;
+                case 8: se_segment<8, TYPES>(p, st, sm, sh, s, r0, r1, lane); break;
+                case 9: se_segment<9, TYPES>(p, st, sm, sh, s, r0, r1, lane); break;
+                case 10: se_segment<10, TYPES>(p, st, sm, sh, s, r0, r1, lane); break;
                 default: break;
             }
             g0 = e;
@@ -298,10 +331,12 @@ cudaError_t launch_showdown_equity(const ShowdownEquityParams& p, cudaStream_t s
     const int prep_grid = (int)std::min<long long>((p.n + 255) / 256, 8ll * p.sm_count);
     se_prepare_kernel<<<prep_grid, 256, 0, s>>>(p);
     se_plan_kernel<<<1, kPlanThreads, 0, s>>>(p);
-    const size_t smem = 128 + (size_t)p.tables.value_bytes + p.tables.rowoff_bytes + p.tables.flush_bytes + kSeExtraBytes;
-    cudaError_t e = cudaFuncSetAttribute(showdown_equity_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    const size_t smem = 128 + (size_t)p.tables.value_bytes + p.tables.rowoff_bytes + p.tables.flush_bytes + kSeExtraBytes +
+                        (p.win_types ? kSeBinBytes : 0);
+    auto k = p.win_types ? showdown_equity_kernel<1> : showdown_equity_kernel<0>;
+    cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
-    showdown_equity_kernel<<<p.sm_count, kSeThreads, smem, s>>>(p);
+    k<<<p.sm_count, kSeThreads, smem, s>>>(p);
     return cudaGetLastError();
 }
 

@@ -174,13 +174,24 @@ def _dead_masks(dead, n, dev):
     return mask
 
 
-def showdown_equity_batch(holes, n_players, board, dead=None, deal_mode="uniform", device=None, validate=None):
+def _check_win_types(win_types):
+    if not isinstance(win_types, (bool, np.bool_)):
+        raise ValueError("win_types must be True or False, not %r" % (win_types,))
+    return bool(win_types)
+
+
+def showdown_equity_batch(holes, n_players, board, dead=None, deal_mode="uniform", device=None, validate=None,
+                          win_types=False):
     """Exact showdown equity of known hands: every completion of each spot's board, scored for every player.
     holes [N,maxp,2] (maxp 1..10), n_players [N], board [N,5] with 0xFF padding, dead [N,k] card ids removed from the deck
     (0xFF padding) or None.  deal_mode "uniform" enumerates every board completion from the unseen cards; "reference" leaves out
     the highest unseen id, which the reference's dealer never deals.  Returns a dict of int64 CUDA tensors: win, tie, share
-    [N,maxp] (share in units of 1/2520 pot per completion) and completions [N]; entries of players >= n_players are 0."""
+    [N,maxp] (share in units of 1/2520 pot per completion) and completions [N]; entries of players >= n_players are 0.
+    win_types=True adds win_types [N,maxp,9]: the completions in which each player holds the best rank, alone or tied, by the
+    hand type of that rank (indexed like HAND_TYPES; the bins of a player sum to its win + tie).  With every hand known,
+    {HAND_TYPES[t]: win_types[s,0,t] / completions[s]} is what run_montecarlo(...).winnerCardTypeList converges to."""
     from .equity import _DEAL
+    want_types = _check_win_types(win_types)
     torch = _torch()
     dev = _dev(device)
     flags = _want_check(holes, validate)
@@ -193,22 +204,28 @@ def showdown_equity_batch(holes, n_players, board, dead=None, deal_mode="uniform
     L = _lib.ensure_init(dev.index)
     out = {k: torch.empty((N, maxp), dtype=torch.int64, device=dev) for k in ("win", "tie", "share")}
     out["completions"] = torch.empty(N, dtype=torch.int64, device=dev)
+    if want_types:
+        out["win_types"] = torch.empty((N, maxp, 9), dtype=torch.int64, device=dev)
     ws = torch.empty(int(L.npk_showdown_equity_workspace_bytes(N)), dtype=torch.uint8, device=dev)
     with torch.cuda.device(dev):
-        _lib.check(L.npk_showdown_equity_batch(holes.data_ptr(), n_players.data_ptr(), board.data_ptr(),
-                                               masks.data_ptr() if masks is not None else None, N, maxp, _DEAL[deal_mode],
-                                               flags, out["win"].data_ptr(), out["tie"].data_ptr(), out["share"].data_ptr(),
-                                               out["completions"].data_ptr(), ws.data_ptr(),
-                                               torch.cuda.current_stream(dev).cuda_stream))
+        _lib.check(L.npk_showdown_equity_win_types_batch(holes.data_ptr(), n_players.data_ptr(), board.data_ptr(),
+                                                         masks.data_ptr() if masks is not None else None, N, maxp,
+                                                         _DEAL[deal_mode], flags, out["win"].data_ptr(), out["tie"].data_ptr(),
+                                                         out["share"].data_ptr(), out["completions"].data_ptr(),
+                                                         out["win_types"].data_ptr() if want_types else None, ws.data_ptr(),
+                                                         torch.cuda.current_stream(dev).cuda_stream))
     return out
 
 
-def showdown_equity(hands, table_cards=(), dead_cards=(), deal_mode="uniform"):
+def showdown_equity(hands, table_cards=(), dead_cards=(), deal_mode="uniform", win_types=False):
     """Exact equity of one spot whose hands are all known -- run_montecarlo with every entry of player_card_list known,
     without sampling, for every player.  hands: two card strings per player (1..10 players, e.g. [{'AS','KS'}, {'QH','QD'}]),
     table_cards: 0..5 card strings, dead_cards: cards removed from the deck (the reference's ghost cards).
     Returns dict(equity = split-pot equity per player, win, tie = completions won alone / tied for best, completions).
-    Invalid or repeated cards raise ValueError, like get_equity."""
+    win_types=True adds win_types: one list of nine per player, the completions it wins or ties by the hand type of its rank
+    (indexed like HAND_TYPES).  Player 0's bins divided by completions are what run_montecarlo(...).winnerCardTypeList
+    converges to.  Invalid or repeated cards raise ValueError, like get_equity."""
+    want_types = _check_win_types(win_types)
     holes = [card_ids(h) for h in hands]
     board, dead = card_ids(table_cards), card_ids(dead_cards)
     if not 1 <= len(holes) <= 10:
@@ -223,23 +240,32 @@ def showdown_equity(hands, table_cards=(), dead_cards=(), deal_mode="uniform"):
     try:
         out = showdown_equity_batch(np.array([holes], dtype=np.uint8), np.array([P], dtype=np.uint8),
                                     np.array([board + [NO_CARD] * (5 - len(board))], dtype=np.uint8),
-                                    np.array([dead or [NO_CARD]], dtype=np.uint8), deal_mode=deal_mode, validate=True)
+                                    np.array([dead or [NO_CARD]], dtype=np.uint8), deal_mode=deal_mode, validate=True,
+                                    win_types=want_types)
     except _lib.NpkError as exc:
         raise ValueError(str(exc)) from None
     win, tie, share = (out[k][0].tolist() for k in ("win", "tie", "share"))
     comp = int(out["completions"][0])
-    return {"equity": [x / (SHARE_UNIT * comp) for x in share], "win": win, "tie": tie, "completions": comp}
+    res = {"equity": [x / (SHARE_UNIT * comp) for x in share], "win": win, "tie": tie, "completions": comp}
+    if want_types:
+        res["win_types"] = out["win_types"][0].tolist()
+    return res
 
 
-def exact_equity_batch(holes, n_known, n_random, board, dead=None, deal_mode="reference", device=None, validate=None):
+def exact_equity_batch(holes, n_known, n_random, board, dead=None, deal_mode="reference", device=None, validate=None,
+                       win_types=False):
     """Exact equity against one or two unknown opponents, with known opponent hands and dead cards: every deal of the unknown
     hands and every completion of the board enumerated on the GPU.
     holes [N,maxk,2] (maxk 1..8): the hero, then the known opponents; n_known [N]: hands of `holes` in the spot, hero included;
     n_random [N]: unknown opponents (1 or 2); board [N,5] with 0xFF padding; dead [N,k] card ids removed from the deck (0xFF
     padding) or None.  deal_mode "uniform" counts every deal once; "reference" weights it by how often the reference's dealer
     makes it (include/npk.h, npk_exact_equity_batch).  Returns a dict of int64 CUDA tensors win, tie, lose [N] (hero strictly
-    best / tied for best / beaten); (win + tie) / (win + tie + lose) is the value run_montecarlo converges to."""
+    best / tied for best / beaten); (win + tie) / (win + tie + lose) is the value run_montecarlo converges to.
+    win_types=True adds win_types [N,9]: the part of win + tie (same weights) in which the hero's rank has each hand type, indexed
+    like HAND_TYPES (the nine bins sum to win + tie); {HAND_TYPES[t]: win_types[s,t] / (win + tie + lose)} is what
+    run_montecarlo(...).winnerCardTypeList converges to."""
     from .equity import _DEAL
+    want_types = _check_win_types(win_types)
     torch = _torch()
     dev = _dev(device)
     flags = _want_check(holes, validate)
@@ -252,20 +278,28 @@ def exact_equity_batch(holes, n_known, n_random, board, dead=None, deal_mode="re
     masks = _dead_masks(dead, N, dev) if dead is not None and N else None
     L = _lib.ensure_init(dev.index)
     out = {k: torch.empty(N, dtype=torch.int64, device=dev) for k in ("win", "tie", "lose")}
+    if want_types:
+        out["win_types"] = torch.empty((N, 9), dtype=torch.int64, device=dev)
     ws = torch.empty(int(L.npk_exact_equity_workspace_bytes(N)), dtype=torch.uint8, device=dev)
     with torch.cuda.device(dev):
-        _lib.check(L.npk_exact_equity_batch(holes.data_ptr(), n_known.data_ptr(), n_random.data_ptr(), board.data_ptr(),
-                                            masks.data_ptr() if masks is not None else None, N, maxk, _DEAL.get(deal_mode, -1),
-                                            flags, out["win"].data_ptr(), out["tie"].data_ptr(), out["lose"].data_ptr(),
-                                            ws.data_ptr(), torch.cuda.current_stream(dev).cuda_stream))
+        _lib.check(L.npk_exact_equity_win_types_batch(holes.data_ptr(), n_known.data_ptr(), n_random.data_ptr(),
+                                                      board.data_ptr(), masks.data_ptr() if masks is not None else None, N,
+                                                      maxk, _DEAL.get(deal_mode, -1), flags, out["win"].data_ptr(),
+                                                      out["tie"].data_ptr(), out["lose"].data_ptr(),
+                                                      out["win_types"].data_ptr() if want_types else None, ws.data_ptr(),
+                                                      torch.cuda.current_stream(dev).cuda_stream))
     return out
 
 
-def exact_equity_counts(player_cards, table_cards, players, known_opponents=(), ghost_cards='', deal_mode="reference"):
+def exact_equity_counts(player_cards, table_cards, players, known_opponents=(), ghost_cards='', deal_mode="reference",
+                        win_types=False):
     """The exact value run_montecarlo(player_card_list = [player_cards] + known_opponents, table_cards, players, ghost_cards)
     converges to, for one or two unknown opponents: players - 1 - len(known_opponents) must be 1 or 2.  Argument names and
     checks follow equity_counts_ranges; player_cards and every known opponent are two cards (no ranges).
-    Returns dict(equity = (win + tie) / (win + tie + lose), win, tie, lose)."""
+    Returns dict(equity = (win + tie) / (win + tie + lose), win, tie, lose).  win_types=True adds win_types: nine ints indexed
+    like HAND_TYPES, the part of win + tie in which the hero's hand has each type (they sum to win + tie);
+    {HAND_TYPES[t]: win_types[t] / (win + tie + lose)} is what run_montecarlo(...).winnerCardTypeList converges to."""
+    want_types = _check_win_types(win_types)
     players = int(players)
     if players < 1:
         raise IndexError("list index out of range")
@@ -298,11 +332,15 @@ def exact_equity_counts(player_cards, table_cards, players, known_opponents=(), 
     holes = np.array([[hole] + known], dtype=np.uint8)
     try:
         out = exact_equity_batch(holes, [1 + len(known)], [k], [board + [NO_CARD] * (5 - len(board))],
-                                 np.array([ghost or [NO_CARD]], dtype=np.uint8), deal_mode=deal_mode, validate=True)
+                                 np.array([ghost or [NO_CARD]], dtype=np.uint8), deal_mode=deal_mode, validate=True,
+                                 win_types=want_types)
     except _lib.NpkError as exc:
         raise ValueError(str(exc)) from None
     win, tie, lose = (int(out[x][0]) for x in ("win", "tie", "lose"))
-    return {"equity": (win + tie) / (win + tie + lose), "win": win, "tie": tie, "lose": lose}
+    res = {"equity": (win + tie) / (win + tie + lose), "win": win, "tie": tie, "lose": lose}
+    if want_types:
+        res["win_types"] = out["win_types"][0].tolist()
+    return res
 
 
 def host_tables():

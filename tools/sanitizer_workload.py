@@ -165,6 +165,24 @@ npk.exact_equity_batch(torch.randint(0, 256, (256, 8, 2), dtype=torch.uint8, dev
 torch.cuda.synchronize()
 print("ok exact equity", flush=True)
 
+# win-type histograms of both exact engines: the same spots and garbage bytes
+for mode in ("uniform", "reference"):
+    o = npk.exact_equity_batch(ee_h, ee_k, ee_r, ee_b, ee_d, deal_mode=mode, win_types=True)
+    assert (o["win_types"].sum(dim=1) == o["win"] + o["tie"]).all()
+    o = npk.showdown_equity_batch(se_h, se_n, se_b, se_d, deal_mode=mode, win_types=True)
+    assert (o["win_types"].sum(dim=2) == o["win"] + o["tie"]).all()
+npk.exact_equity_batch(torch.randint(0, 256, (256, 8, 2), dtype=torch.uint8, device="cuda"),
+                       torch.randint(0, 256, (256,), dtype=torch.uint8, device="cuda"),
+                       torch.randint(0, 4, (256,), dtype=torch.uint8, device="cuda"),
+                       torch.randint(0, 256, (256, 5), dtype=torch.uint8, device="cuda"),
+                       torch.randint(0, 256, (256, 3), dtype=torch.uint8, device="cuda"), win_types=True)
+npk.showdown_equity_batch(torch.randint(0, 256, (256, 10, 2), dtype=torch.uint8, device="cuda"),
+                          torch.randint(0, 256, (256,), dtype=torch.uint8, device="cuda"),
+                          torch.randint(0, 256, (256, 5), dtype=torch.uint8, device="cuda"),
+                          torch.randint(0, 256, (256, 3), dtype=torch.uint8, device="cuda"), win_types=True)
+torch.cuda.synchronize()
+print("ok exact win types", flush=True)
+
 # vectorised HoldemTable: self-play with both dealers, observation vector, showdowns
 tb = HoldemTables(96, n_players=6, seed=3, autoplay=[1] * 6)
 tb.enable_observations()
